@@ -65,6 +65,8 @@ def parse():
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-eager-gpu", action="store_true", help="skip the stock-PyTorch-on-B200 baseline")
     ap.add_argument("--windows", type=int, default=5, help="steady-state windows of 20 steps after the headline region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="one GPU: after the timed steps, write what the last one handed its "
+                    "caller (every model's loss and its parameters after the flush) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -614,6 +616,41 @@ def run_eager_gpu(dev, B, N, D, our_value):
                     "torch.optim.Adam(lr=1e-3, weight_decay=1e-5) over all rows; same workload (C2), fp32, TF32 off"}
 
 
+DUMP_ROWS = 1 << 16        # table rows sampled by --dump-outputs
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ms, losses, n_rows):
+    """--dump-outputs: the last timed step's loss of every model and, after the flush, its parameters under the reference's
+    state_dict keys, as float32 (integers as float64) .npy files.  Dense tensors are written whole; of the tables (n_rows
+    rows) the same fixed, seeded sample of rows, listed in table_rows.npy.  Two builds run with the same arguments can
+    then be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.random.default_rng(0).choice(n_rows, size=min(n_rows, DUMP_ROWS), replace=False)
+    rows.sort()
+    out = {"table_rows": rows.astype(np.float64)}
+    models = []
+    for m, _ in ms:                       # a co-located group holds LR, FM, DeepFM as its members, in that order
+        models.extend(m.members if hasattr(m, "members") else [m])
+    loss = torch.cat([l.reshape(-1) for l in losses]).cpu().numpy()
+    assert len(models) == loss.size == len(MODELS), (len(models), loss.size)
+    idx = None
+    for name, m, l in zip(MODELS, models, loss):
+        out[f"{name}.loss"] = np.float32(l)
+        for key, t in m.state_dict().items():
+            if t.dim() > 0 and t.shape[0] == n_rows:
+                if idx is None:
+                    idx = torch.as_tensor(rows, device=t.device)
+                t = t[idx]
+            a = t.cpu().numpy()
+            out[f"{name}.{key}"] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    torch.cuda.empty_cache()
+
+
 # ----------------------------------------------------------------------------------------------
 # B200 arm
 # ----------------------------------------------------------------------------------------------
@@ -627,6 +664,8 @@ def b200_arm(args):
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs runs on one GPU")
         dist.init_process_group("nccl", device_id=dev)
     B, N, D, K, W = args.batch, args.rows, args.dims, args.steps, args.warmup
     W = max(W, 3)
@@ -712,7 +751,7 @@ def b200_arm(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(K):
-        run_step(*batches[W + i])
+        losses = run_step(*batches[W + i])
     for m, _ in ms:
         m.flush()
     e1.record()
@@ -722,6 +761,8 @@ def b200_arm(args):
         launches += gstep.launches_per_step * K          # replayed launches are not seen by the host-side tally
     clk = clocks.stop()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ms, losses, N)
 
     def max_over_ranks(v):
         t = torch.tensor([v], device=dev, dtype=torch.float64)

@@ -227,3 +227,30 @@ def test_td3_action_masking_against_oracle():
     nxt = agent.to_next_state_c_actions(torch.as_tensor(d), torch.as_tensor(c), eps=torch.as_tensor(eps)).numpy()
     assert np.array_equal(cur, O.keep_top_d_actions(d, c))
     np.testing.assert_allclose(nxt, O.keep_top_d_actions(d, c, eps), rtol=1e-6, atol=1e-7)
+
+
+def test_bench_dump_outputs_layout(tmp_path):
+    """bench.py --dump-outputs: every model's loss and reference-keyed parameter lands in <name>.npy as float32/float64, the
+    N-row tables as the same seeded row sample (so two runs name and index the same values), within the 64 MB cap."""
+    import bench
+    N = 100_000
+    torch.manual_seed(0)
+    ms = [(TP.PortCTR(name, N, 15, 10), None) for name in bench.MODELS]
+    losses = [torch.tensor([0.5, 0.25, 0.125])]               # a co-located group returns its members' losses as one tensor
+    for out in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(str(out), ms, losses, N)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b"))
+    total = 0
+    for f in names:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), f
+        total += a.nbytes
+    assert total <= bench.DUMP_MAX_BYTES
+    rows = np.load(tmp_path / "a" / "table_rows.npy").astype(np.int64)
+    assert len(rows) == bench.DUMP_ROWS and np.all(np.diff(rows) > 0) and rows[-1] < N
+    for name, (m, _), loss in zip(bench.MODELS, ms, (0.5, 0.25, 0.125)):
+        assert np.load(tmp_path / "a" / f"{name}.loss.npy") == np.float32(loss)
+        for key, t in m.state_dict().items():
+            want = t.numpy()[rows] if t.shape[0] == N else t.numpy()
+            assert np.array_equal(np.load(tmp_path / "a" / f"{name}.{key}.npy"), want), (name, key)
