@@ -359,11 +359,14 @@ typedef struct rlctr_member {
     int64_t      rows_pitch;   /* 0 = fields*dim */
     /* gradient side (rlctr_group_rows_adam) */
     const float* dlogit;       /* [B] dL/dlogit of this member; NULL: it rides in the sums rows, column sums_pitch - RLCTR_GROUP_MAX + m
-                                * (one line per sample carries S and every member's dL/dlogit: what the row-sharded step all-gathers) */
+                                * (one line per sample carries S and every member's dL/dlogit: what the row-sharded step all-gathers).
+                                * Never read for a member without a first-order column and without RLCTR_FM_TERM (FNN, PNN, DCN:
+                                * its row gradient is `extra` alone) */
     const float* extra;        /* [B, fields*dim] dense-tail gradient on the latent columns, or NULL */
 } rlctr_member;
 /* One gather per (sample, field) for every member: logit / pctr / rows_out per member as rlctr_embed_fwd would produce them
- * from the member's stand-alone table; sums[b * sums_pitch + col] = column sums of the joint rows (optional: the backward's S;
+ * from the member's stand-alone table (a member with lin_col = -1, no bias and no RLCTR_FM_TERM has a table logit of 0: it
+ * usually asks for rows_out only); sums[b * sums_pitch + col] = column sums of the joint rows (optional: the backward's S;
  * sums_pitch = 0 means row_stride).  A row-sharded joint table (table->world > 1) is read through peers[] like rlctr_embed_fwd. */
 int rlctr_group_fwd(const int64_t* ids, const rlctr_table* table, const rlctr_member* members, int32_t n_members,
                     float* sums, int32_t sums_pitch, int64_t batch, int32_t fields, rlctr_stream_t stream);

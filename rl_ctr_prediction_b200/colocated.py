@@ -12,9 +12,13 @@ are laid side by side in one record
     [ exp_avg_sq                                        ] (pad)     exp_avg_sq block
 
 and one gather (rlctr_group_fwd), one catch-up (rlctr_rows_catchup) and one update (rlctr_group_rows_adam) serve all of
-them: 13 random line operations per (sample, field) and step instead of 23 for LR + FM + DeepFM.  Each member keeps the
-chunk alignment of its stand-alone row, so its logits and its updated parameters are bit-identical to the stand-alone
-model's (tests/test_gpu_colocated.py).
+them: 13 random line operations per (sample, field) and step instead of 23 for LR + FM + DeepFM.  Members may be any of the
+FM-row models of ``get_model`` (FFM's rows are wider than a line): LR, FM, DeepFM, WideAndDeep, FNN, InnerPNN, OuterPNN, DCN
+and AFM -- at D = 10 two vector members and LR fill one line (e.g. LR + FM + FNN, DeepFM + InnerPNN, FM + AFM).  A member with
+a dense tail computes its logit with its own ``_tail(z_table, rows)`` from the group's gather, so its tower, cross network or
+attention (and the dropout masks they draw from the member's own counter) are those of the stand-alone model.  Each member
+keeps the chunk alignment of its stand-alone row, so its logits and its updated parameters are bit-identical to the
+stand-alone model's (tests/test_gpu_colocated.py, tests/test_gpu_colocated_tails.py).
 
     lr, fm, dfm = (get_model(name, ...).to(dev) for name in ("LR", "FM", "DeepFM"))
     group = colocate([lr, fm, dfm])                       # re-homes the three tables into one; the members stay usable
@@ -33,6 +37,11 @@ import torch.nn as nn
 from . import _lib
 from . import p_model as Model
 from .tables import Geometry, round4, table_struct
+
+
+# the member kinds of one joint record: an FM-type row [w?, v_0 .. v_{D-1}] (or LR's scalar) and a logit the group step computes
+MEMBER_KINDS = (Model.LR, Model.FM, Model.DeepFM, Model.WideAndDeep, Model.FNN, Model.InnerPNN, Model.OuterPNN, Model.DCN,
+                Model.AFM)
 
 
 # 1: the group's catch-up works from the ids in batch order and the sort of the batch runs on a side stream (see train_step);
@@ -85,9 +94,9 @@ def _layout(members):
 
 
 class ColocatedCTR(Model._TableModel):
-    """``colocate(models)``: LR / FM-type drop-in models over one joint table.  The group owns the table, its lazy-exact
-    Adam state and the training step; the members keep ``forward`` (inference), ``state_dict`` / ``load_state_dict``
-    (reference keys) and their dense parameters."""
+    """``colocate(models)``: LR / FM-type drop-in models (``MEMBER_KINDS``) over one joint table.  The group owns the table,
+    its lazy-exact Adam state and the training step; the members keep ``forward`` (inference), ``state_dict`` /
+    ``load_state_dict`` (reference keys) and their dense parameters."""
 
     _kind = "group"
 
@@ -97,9 +106,10 @@ class ColocatedCTR(Model._TableModel):
         if not 1 <= len(models) <= _lib.RLCTR_GROUP_MAX:
             raise ValueError(f"a co-located group holds 1..{_lib.RLCTR_GROUP_MAX} models")
         for m in models:
-            # LR / FM: table only; DeepFM / W&D: logit = table part + tower(gathered rows) -- the forms the group step computes
-            if type(m) not in (Model.LR, Model.FM, Model.DeepFM, Model.WideAndDeep) or m.__dict__.get("_group") is not None:
-                raise _lib.RlctrError(f"{type(m).__name__} cannot join a co-located group (LR, FM, DeepFM, WideAndDeep; once)")
+            # LR / FM: table only; the others: logit = m._tail(table part or None, gathered rows)
+            if type(m) not in MEMBER_KINDS or m.__dict__.get("_group") is not None:
+                raise _lib.RlctrError(f"{type(m).__name__} cannot join a co-located group "
+                                      f"({', '.join(k.__name__ for k in MEMBER_KINDS)}; once)")
         n_rows = {m._geom.n_rows for m in models}
         devs = {m.table.device for m in models}
         if len(n_rows) != 1 or len(devs) != 1:
@@ -154,6 +164,9 @@ class ColocatedCTR(Model._TableModel):
 
     # ---- forward of every member from one gather ---------------------------------------------------------------------
     def _member_structs(self, B, F, dev, train, pctr=None):
+        """The members' views for rlctr_group_fwd.  logits[i]: the table part of member i's logit (bias + first order + FM
+        term), None for a member that has none (FNN, InnerPNN, OuterPNN, DCN: no linear column, no bias); rows[i]: the tower
+        input [B, pitch] of a member with a dense tail, else None."""
         arr = (_lib.Member * len(self.members))()
         logits, rows = [], []
         for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
@@ -162,14 +175,15 @@ class ColocatedCTR(Model._TableModel):
             s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
             bias = getattr(m, "bias", None)
             s.bias = _lib.ptr(bias.data) if bias is not None else None
-            tower = getattr(m, "mlp", None) is not None
-            z = torch.empty(B, dtype=torch.float32, device=dev) if (train or tower) else None
+            tail = hasattr(m, "_tail")
+            table_part = lin >= 0 or bias is not None or m._fm_term
+            z = torch.empty(B, dtype=torch.float32, device=dev) if table_part and (train or tail) else None
             logits.append(z)
             s.logit = _lib.ptr(z)
-            if pctr is not None and not tower:
+            if pctr is not None and not tail:
                 s.pctr, s.pctr_stride = pctr.data_ptr() + 4 * i, pctr.shape[1]
             r = None
-            if tower:
+            if tail:
                 pitch = round4(F * dim)                      # 16-byte aligned pitch: the tower's first GEMM fetches it by TMA
                 r = torch.empty(B, pitch, dtype=torch.float32, device=dev)
                 s.rows_out, s.rows_pitch = r.data_ptr(), pitch
@@ -190,9 +204,12 @@ class ColocatedCTR(Model._TableModel):
                   _lib.stream(), key="rlctr_group_fwd[infer]", meta=self._meta(B, F))
         for i, m in enumerate(self.members):
             if rows[i] is not None:
-                fd = F * self._cols[i][2]
-                out[:, i:i + 1] = torch.sigmoid(logits[i].view(B, 1) + m.mlp(rows[i][:, :fd]))
+                out[:, i:i + 1] = torch.sigmoid(m._tail(self._z(logits[i], B), rows[i][:, :F * self._cols[i][2]]))
         return out
+
+    @staticmethod
+    def _z(logit, B):
+        return logit.view(B, 1) if logit is not None else None
 
     # ---- the training step ---------------------------------------------------------------------------------------
     def train_step(self, x, y, optimizer):
@@ -252,10 +269,10 @@ class ColocatedCTR(Model._TableModel):
                                                  losses.data_ptr() + 4 * i, _lib.ptr(dl), _lib.ptr(dbias), _lib.ptr(ws), B, st),
                            "rlctr_bce_fwd_bwd")
                 extras.append(None)
-            else:                                            # dense tail: autograd over the tower only
+            else:                                            # dense tail: autograd over the member's tail only
                 fd = F * self._cols[i][2]
                 leaf = rows[i][:, :fd].detach().requires_grad_(True)
-                z = logits[i].view(B, 1) + m.mlp(leaf)
+                z = m._tail(self._z(logits[i], B), leaf)
                 zz = z.detach().reshape(-1).contiguous()
                 # (the head's own sum of dlogit is the bias gradient: the same block partition and tree as the stand-alone
                 # backward's rlctr_sigmoid_bwd sum -- the same bits, one launch less)

@@ -73,6 +73,8 @@ struct GroupCols {
                                              // sums_pitch - RLCTR_GROUP_MAX + m of the sample's sums row
     signed char member[32];                  // column -> member, -1: padding / stamp
     signed char role[32];                    // 0 none, 1 first-order weight, 2 latent column with the FM term, 3 latent column without
+    int dz_used;                             // bit m: a column of member m (role 1 or 2) uses its dL/dlogit.  A member whose row
+                                             // gradient is all dense tail (FNN, PNN, DCN: role 3 only) has no dL/dlogit load
 };
 struct GradView {
     GroupCols grp;
@@ -243,7 +245,8 @@ __device__ __forceinline__ float4 rowgrad_group(const GradView& g, const GroupLa
         const int m = gl.mem[k];
         if (m < 0) continue;
         const float* dzp = g.grp.dz[m];
-        const float dz = dzp ? __ldg(dzp + b) : __ldg(srow + g.grp.sums_pitch - RLCTR_GROUP_MAX + m);
+        const bool want_dz = gl.role[k] == 1 || gl.role[k] == 2;
+        const float dz = !want_dz ? 0.f : dzp ? __ldg(dzp + b) : __ldg(srow + g.grp.sums_pitch - RLCTR_GROUP_MAX + m);
         const float* ex = gl.role[k] >= 2 ? g.grp.extra[m] : nullptr;
         const float exv = ex ? __ldg(ex + (int64_t)erow * g.grp.dim[m] + (col0 + k - g.grp.emb_col[m])) : 0.f;
         f4set(r, k, group_col_grad(gl.role[k], dz, f4get(S, k), f4get(p, k), ex != nullptr, exv));
@@ -637,7 +640,7 @@ group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
 #pragma unroll
             for (int mm = 0; mm < RLCTR_GROUP_MAX; ++mm) {
                 dzv[mm] = 0.f;
-                if (mm < g.grp.n) dzv[mm] = g.grp.dz[mm] ? __ldg(g.grp.dz[mm] + b) : __ldg(srow + g.grp.sums_pitch - RLCTR_GROUP_MAX + mm);
+                if (mm < g.grp.n && ((g.grp.dz_used >> mm) & 1)) dzv[mm] = g.grp.dz[mm] ? __ldg(g.grp.dz[mm] + b) : __ldg(srow + g.grp.sums_pitch - RLCTR_GROUP_MAX + mm);
             }
 #pragma unroll
             for (int j = 0; j < CH; ++j) {
@@ -1598,7 +1601,9 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
     for (int m = 0; m < n_members; ++m) {
         const rlctr_member& mm = members[m];
         if (mm.dim < 0 || mm.emb_col < 0 || mm.emb_col + mm.dim > t.rs || mm.lin_col >= t.rs) return RLCTR_EINVAL;
-        if (!mm.dlogit && sums_pitch - RLCTR_GROUP_MAX < t.rs) return RLCTR_EINVAL;      // no room for dL/dlogit in the sums rows
+        const bool uses_dz = mm.lin_col >= 0 || ((mm.flags & RLCTR_FM_TERM) && mm.dim > 0);
+        if (uses_dz && !mm.dlogit && sums_pitch - RLCTR_GROUP_MAX < t.rs) return RLCTR_EINVAL;   // no room for dL/dlogit in the sums rows
+        if (uses_dz) g.grp.dz_used |= 1 << m;
         g.grp.dz[m] = mm.dlogit; g.grp.extra[m] = mm.extra; g.grp.emb_col[m] = mm.emb_col; g.grp.dim[m] = mm.dim;
         if (mm.lin_col >= 0) {
             if (g.grp.member[mm.lin_col] >= 0) return RLCTR_EINVAL;              // two members claim one column

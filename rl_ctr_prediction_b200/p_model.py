@@ -440,10 +440,14 @@ class DeepFM(FM):
         self.field_nums = int(field_nums)
         self.mlp = _tower(self.field_nums * self.latent_dims, device)
 
+    def _tail(self, z, rows):
+        """Logit [B, 1] from the table part z (bias + first order + FM term, [B, 1]) and the gathered rows [B, F*D]: the one
+        definition the stand-alone ``logit`` and a co-located group's step (colocated.py) share."""
+        return z + self.mlp(rows)
+
     def logit(self, x):
         """Pre-sigmoid output [B, 1] (graphs.eager_step feeds it to the fused sigmoid + BCE head)."""
-        z_fm, rows = self._run(x, True, False)
-        return z_fm + self.mlp(rows)
+        return self._tail(*self._run(x, True, False))
 
     def forward(self, x):
         return torch.sigmoid(self.logit(x))
@@ -499,9 +503,11 @@ class WideAndDeep(_TableModel):
         g = self._geom
         return [("linear.weight", g.lin_col, 1), ("embedding.weight", g.emb_col, g.dim)]
 
-    def logit(self, x):
-        z, rows = self._run(x, True, False)
+    def _tail(self, z, rows):
         return z + self.mlp(rows)
+
+    def logit(self, x):
+        return self._tail(*self._run(x, True, False))
 
     def forward(self, x):
         return torch.sigmoid(self.logit(x))
@@ -535,9 +541,12 @@ class FNN(_TableModel):
     def _tower_input(self, rows):
         return rows
 
-    def logit(self, x):
-        _, rows = self._run(x, True, False)
+    def _tail(self, z, rows):
+        """No first-order term and no bias: the logit is the tower's output alone and z is not read (None in a group)."""
         return self.mlp(self._tower_input(rows))
+
+    def logit(self, x):
+        return self._tail(*self._run(x, True, False))
 
     def forward(self, x):
         return torch.sigmoid(self.logit(x))
@@ -665,13 +674,16 @@ class DCN(_TableModel):
         g = self._geom
         return [("feature_embedding.weight", g.emb_col, g.dim)]
 
-    def logit(self, x):
-        _, rows = self._run(x, True, False)
+    def _tail(self, z, rows):
+        """No first-order term and no bias: z is not read (None in a group)."""
         W = torch.cat([m.weight for m in self.cross_net_w], dim=0)
         Bv = torch.stack(list(self.cross_net_b), dim=0)
         cn_x = _CrossNet.apply(rows, W, Bv)
         dn_x = self.DN(rows)
         return self.linear(torch.cat([cn_x, dn_x], dim=1))                              # :430-433
+
+    def logit(self, x):
+        return self._tail(*self._run(x, True, False))
 
     def forward(self, x):
         return torch.sigmoid(self.logit(x))                                             # :435
@@ -760,6 +772,10 @@ class AFM(_TableModel):
 
     def logit(self, x, masks=None):
         z, rows = self._run(x, True, False)
+        return self._tail(z, rows, masks)
+
+    def _tail(self, z, rows, masks=None):
+        """z: bias + first order [B, 1]; the attention term draws its two dropout masks from this model's counter."""
         packed = torch.cat([self.attention_net.weight.reshape(-1), self.attention_net.bias,
                             self.attention_softmax.weight.reshape(-1), self.attention_softmax.bias,
                             self.fc.weight.reshape(-1), self.fc.bias])
