@@ -327,6 +327,14 @@ int rlctr_sort_routed_pos(const uint32_t* keys, int64_t n_in, int64_t n_rows_loc
                           void* ws, size_t ws_bytes, rlctr_stream_t stream);
 int rlctr_push_rows_routed(const void* route_ws, int64_t n, int32_t world, int32_t rank, int64_t cap, const float* src,
                            int32_t width, void* const* peer_recv, rlctr_stream_t stream);
+/* The same push for up to RLCTR_GROUP_MAX sources in one pass over the bucket order (the dense-tail members of a row-sharded
+ * co-located group): source s is srcs[s] [n, widths[s]] (every width even, rows 8-byte aligned), and occurrence `slot` writes ONE
+ * interleaved row peer_recv[owner] + (rank * cap + bucket position) * pitch + off_s, off_s = sum_{t<s} widths[t],
+ * pitch = sum_s widths[s].  An owner's receive buffer is [world * cap, pitch]; member s of the update reads it with
+ * rlctr_member.extra = buffer + off_s, extra_pitch = pitch.  rlctr_push_rows_routed is this call with n_src = 1. */
+int rlctr_push_rows_routed_multi(const void* route_ws, int64_t n, int32_t world, int32_t rank, int64_t cap,
+                                 const float* const* srcs, const int32_t* widths, int32_t n_src, void* const* peer_recv,
+                                 rlctr_stream_t stream);
 int rlctr_rows_adam(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n,
                     const rlctr_rowgrad* grad, const rlctr_table* table, const rlctr_adam* opt,
                     void* ws, size_t ws_bytes, rlctr_stream_t stream);
@@ -363,6 +371,9 @@ typedef struct rlctr_member {
                                 * Never read for a member without a first-order column and without RLCTR_FM_TERM (FNN, PNN, DCN:
                                 * its row gradient is `extra` alone) */
     const float* extra;        /* [B, fields*dim] dense-tail gradient on the latent columns, or NULL */
+    int64_t      extra_pitch;  /* floats between consecutive occurrences' rows of `extra`; 0 = dim (the [B, fields*dim] layout).
+                                * The row-sharded group passes the interleaved receive rows of rlctr_push_rows_routed_multi:
+                                * extra = receive buffer + off_m, extra_pitch = the receive row's pitch */
 } rlctr_member;
 /* One gather per (sample, field) for every member: logit / pctr / rows_out per member as rlctr_embed_fwd would produce them
  * from the member's stand-alone table (a member with lin_col = -1, no bias and no RLCTR_FM_TERM has a table logit of 0: it
@@ -371,7 +382,7 @@ typedef struct rlctr_member {
 int rlctr_group_fwd(const int64_t* ids, const rlctr_table* table, const rlctr_member* members, int32_t n_members,
                     float* sums, int32_t sums_pitch, int64_t batch, int32_t fields, rlctr_stream_t stream);
 /* rlctr_rows_adam over the joint record: per column the gradient of the member that owns it
- * (first-order: dlogit_m[b]; latent: dlogit_m[b] * (sums[b, col] - row[col]) if RLCTR_FM_TERM, + extra_m[slot * dim + d]),
+ * (first-order: dlogit_m[b]; latent: dlogit_m[b] * (sums[b, col] - row[col]) if RLCTR_FM_TERM, + extra_m[slot * extra_pitch + d]),
  * reduced over the occurrences of an id in slot order, then ONE Adam step on the record.  b = slot / fields: for a row-sharded
  * table the slots are GLOBAL (src rank * n_per_rank + slot), `sums` is the all-gathered [world * B, sums_pitch] array, extra_m the
  * owner's receive buffer of rlctr_push_rows, and `world` sizes the grid for the owned ~1/world of the sorted view (the rest are

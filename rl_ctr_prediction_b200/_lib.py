@@ -62,7 +62,8 @@ class Member(C.Structure):
     """struct rlctr_member: one model's view of a co-located record"""
     _fields_ = [("lin_col", C.c_int32), ("emb_col", C.c_int32), ("dim", C.c_int32), ("flags", C.c_int32),
                 ("bias", C.c_void_p), ("logit", C.c_void_p), ("pctr", C.c_void_p), ("pctr_stride", C.c_int64),
-                ("rows_out", C.c_void_p), ("rows_pitch", C.c_int64), ("dlogit", C.c_void_p), ("extra", C.c_void_p)]
+                ("rows_out", C.c_void_p), ("rows_pitch", C.c_int64), ("dlogit", C.c_void_p), ("extra", C.c_void_p),
+                ("extra_pitch", C.c_int64)]
 
 
 RLCTR_GROUP_MAX = 4
@@ -115,6 +116,7 @@ SIGNATURES = {
     "rlctr_group_rows_adam": (C.c_int, [_P, _P, _I64, _TP, _AP, _MP, _I32, _P, _I32, _I32, _I32, _P, _P, _SZ, _P]),
     "rlctr_sort_routed_pos": (C.c_int, [_P, _I64, _I64, _P, _P, _P, _SZ, _P]),
     "rlctr_push_rows_routed": (C.c_int, [_P, _I64, _I32, _I32, _I64, _P, _I32, _P, _P]),
+    "rlctr_push_rows_routed_multi": (C.c_int, [_P, _I64, _I32, _I32, _I64, _P, _P, _I32, _P, _P]),
     "rlctr_rows_grad_dense": (C.c_int, [_P, _P, _I64, _GP, _TP, _P, _P, _SZ, _P]),
     "rlctr_lookup_stage_floats": (_I64, [_TP]),
     "rlctr_rows_lookup": (C.c_int, [_P, _P, _I64, _TP, _AP, _LP, _P, _SZ, _P]),

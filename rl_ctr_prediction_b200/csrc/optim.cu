@@ -67,6 +67,8 @@ struct GroupCols {
     const float* dz[RLCTR_GROUP_MAX];        // dL/dlogit of member m, [B]
     const float* extra[RLCTR_GROUP_MAX];     // dense-tail gradient on member m's latent columns, [B, fields * dim_m], or NULL
     int emb_col[RLCTR_GROUP_MAX], dim[RLCTR_GROUP_MAX];
+    int ex_pitch[RLCTR_GROUP_MAX];           // floats between consecutive occurrences' rows of extra[m] (dim, or the interleaved
+                                             // receive row of the routed multi-source push)
     const uint32_t* slot_of;                 // non-NULL (routed exchange): sorted_slots holds RECEIVE positions r; the global slot
                                              // (-> sample, for S and dL/dlogit) is slot_of[r], the dense-tail row is extra_m[r]
     int sums_pitch;                          // floats between the sums rows; dz[m] == NULL: dL/dlogit of member m rides in column
@@ -248,7 +250,7 @@ __device__ __forceinline__ float4 rowgrad_group(const GradView& g, const GroupLa
         const bool want_dz = gl.role[k] == 1 || gl.role[k] == 2;
         const float dz = !want_dz ? 0.f : dzp ? __ldg(dzp + b) : __ldg(srow + g.grp.sums_pitch - RLCTR_GROUP_MAX + m);
         const float* ex = gl.role[k] >= 2 ? g.grp.extra[m] : nullptr;
-        const float exv = ex ? __ldg(ex + (int64_t)erow * g.grp.dim[m] + (col0 + k - g.grp.emb_col[m])) : 0.f;
+        const float exv = ex ? __ldg(ex + (int64_t)erow * g.grp.ex_pitch[m] + (col0 + k - g.grp.emb_col[m])) : 0.f;
         f4set(r, k, group_col_grad(gl.role[k], dz, f4get(S, k), f4get(p, k), ex != nullptr, exv));
     }
     return r;
@@ -589,7 +591,7 @@ group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
     // per chunk of this lane: packed (member, role) of its four columns, and the dense-tail gradient of its vector member
     int desc[CH];                        // 4 x (role 2 bits | member 2 bits)
     const float* exb[CH];                // extra_m - emb_col_m + col0 of the chunk, or NULL
-    int exd[CH];                         // dim_m
+    int exd[CH];                         // extra_pitch_m
     bool live[CH];
 #pragma unroll
     for (int j = 0; j < CH; ++j) {
@@ -602,7 +604,7 @@ group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
             const int m = (live[j] && col < 32) ? (int)g.grp.member[col] : -1;
             const int role = m >= 0 ? (int)g.grp.role[col] : 0;
             desc[j] |= ((role & 3) | ((m & 3) << 2)) << (4 * k);
-            if (role >= 2 && g.grp.extra[m]) { exb[j] = g.grp.extra[m] + (col0 - g.grp.emb_col[m]); exd[j] = g.grp.dim[m]; }
+            if (role >= 2 && g.grp.extra[m]) { exb[j] = g.grp.extra[m] + (col0 - g.grp.emb_col[m]); exd[j] = g.grp.ex_pitch[m]; }
         }
     }
     const int sc5 = a.stamp_col >= 0 ? (a.stamp_col >> 2) : 0;         // chunk that holds the in-record stamp
@@ -1601,10 +1603,12 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
     for (int m = 0; m < n_members; ++m) {
         const rlctr_member& mm = members[m];
         if (mm.dim < 0 || mm.emb_col < 0 || mm.emb_col + mm.dim > t.rs || mm.lin_col >= t.rs) return RLCTR_EINVAL;
+        if (mm.extra_pitch != 0 && (mm.extra_pitch < mm.dim || mm.extra_pitch > INT32_MAX)) return RLCTR_EINVAL;
         const bool uses_dz = mm.lin_col >= 0 || ((mm.flags & RLCTR_FM_TERM) && mm.dim > 0);
         if (uses_dz && !mm.dlogit && sums_pitch - RLCTR_GROUP_MAX < t.rs) return RLCTR_EINVAL;   // no room for dL/dlogit in the sums rows
         if (uses_dz) g.grp.dz_used |= 1 << m;
         g.grp.dz[m] = mm.dlogit; g.grp.extra[m] = mm.extra; g.grp.emb_col[m] = mm.emb_col; g.grp.dim[m] = mm.dim;
+        g.grp.ex_pitch[m] = mm.extra_pitch ? (int)mm.extra_pitch : mm.dim;
         if (mm.lin_col >= 0) {
             if (g.grp.member[mm.lin_col] >= 0) return RLCTR_EINVAL;              // two members claim one column
             g.grp.member[mm.lin_col] = (signed char)m; g.grp.role[mm.lin_col] = 1;

@@ -254,13 +254,20 @@ namespace rlctr {
 __global__ void __launch_bounds__(256) iota_kernel(uint32_t* __restrict__ out, int64_t n) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) out[i] = (uint32_t)i;
 }
-// rows of `src` (width floats, even) in the bucket order rlctr_route_ids computed: row sslots[i] goes to owner skeys[i] at
-// recv[owner][(rank * cap + i - starts[owner]) * width]: consecutive threads write consecutive bytes of an owner's segment
+// rows of up to RLCTR_GROUP_MAX sources (src_s [n, width_s], widths even) in the bucket order rlctr_route_ids computed: occurrence
+// sslots[i] goes to owner skeys[i] as ONE interleaved row at recv[owner][(rank * cap + i - starts[owner]) * pitch], source s at float
+// offset off_s = sum_{t<s} width_t, pitch = sum_s width_s: consecutive threads write consecutive 8-byte pieces of an owner's segment
+struct PushSrcs {
+    const float* src[RLCTR_GROUP_MAX];
+    int width[RLCTR_GROUP_MAX];
+    int off[RLCTR_GROUP_MAX];
+    int n_src;
+};
 __global__ void __launch_bounds__(256)
 push_routed_kernel(const uint32_t* __restrict__ skeys, const uint32_t* __restrict__ sslots, const int64_t* __restrict__ starts,
-                   int64_t n, int world, int64_t seg0, int64_t cap, const float* __restrict__ src, int width,
+                   int64_t n, int world, int64_t seg0, int64_t cap, const __grid_constant__ PushSrcs ps, int pitch,
                    const __grid_constant__ ShardView sv) {
-    const int per = width >> 1;
+    const int per = pitch >> 1;
     const int64_t total = n * per;
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t i = t / per;
@@ -270,19 +277,35 @@ push_routed_kernel(const uint32_t* __restrict__ skeys, const uint32_t* __restric
         const int64_t pos = i - starts[o];
         if (pos >= cap) continue;                                   // overflow: flagged by rlctr_route_ids
         const uint32_t slot = __ldg(sslots + i);
-        const float2 v = __ldg(reinterpret_cast<const float2*>(src + (int64_t)slot * width) + j);
-        float* dst = const_cast<float*>(sv.peers[o]) + (seg0 + pos) * width;
+        int s = 0;                                                  // the source of piece j (n_src <= 4: a short scan)
+#pragma unroll
+        for (int q = 1; q < RLCTR_GROUP_MAX; ++q)
+            if (q < ps.n_src && 2 * j >= ps.off[q]) s = q;
+        const int c = 2 * j - ps.off[s];
+        const float2 v = __ldg(reinterpret_cast<const float2*>(ps.src[s] + (int64_t)slot * ps.width[s] + c));
+        float* dst = const_cast<float*>(sv.peers[o]) + (seg0 + pos) * pitch;
         reinterpret_cast<float2*>(dst)[j] = v;
     }
 }
 }  // namespace rlctr
 
-extern "C" int rlctr_push_rows_routed(const void* route_ws, int64_t n, int32_t world, int32_t rank, int64_t cap, const float* src,
-                                      int32_t width, void* const* peer_recv, rlctr_stream_t stream) {
-    if (!route_ws || !src || !peer_recv || n < 0 || width <= 0 || cap <= 0) return RLCTR_EINVAL;
+extern "C" int rlctr_push_rows_routed_multi(const void* route_ws, int64_t n, int32_t world, int32_t rank, int64_t cap,
+                                            const float* const* srcs, const int32_t* widths, int32_t n_src, void* const* peer_recv,
+                                            rlctr_stream_t stream) {
+    if (!route_ws || !srcs || !widths || !peer_recv || n < 0 || cap <= 0) return RLCTR_EINVAL;
+    if (n_src < 1 || n_src > RLCTR_GROUP_MAX) return RLCTR_EINVAL;
     if (world != 2 && world != 4 && world != 8) return RLCTR_EUNSUPPORTED;
-    if (rank < 0 || rank >= world || width % 2 != 0) return RLCTR_EINVAL;
-    if ((((uintptr_t)src) & 7u) != 0) return RLCTR_EALIGN;
+    if (rank < 0 || rank >= world) return RLCTR_EINVAL;
+    PushSrcs ps;
+    ps.n_src = n_src;
+    int pitch = 0;
+    for (int s = 0; s < RLCTR_GROUP_MAX; ++s) { ps.src[s] = nullptr; ps.width[s] = 0; ps.off[s] = 0; }
+    for (int s = 0; s < n_src; ++s) {
+        if (!srcs[s] || widths[s] <= 0 || widths[s] % 2 != 0) return RLCTR_EINVAL;
+        if ((((uintptr_t)srcs[s]) & 7u) != 0) return RLCTR_EALIGN;
+        ps.src[s] = srcs[s]; ps.width[s] = widths[s]; ps.off[s] = pitch;
+        pitch += widths[s];
+    }
     ShardView sv;
     sv.shift = 0; sv.mask = world - 1;
     for (int r = 0; r < RLCTR_MAX_WORLD; ++r) sv.peers[r] = nullptr;
@@ -297,11 +320,20 @@ extern "C" int rlctr_push_rows_routed(const void* route_ws, int64_t n, int32_t w
     const uint32_t* skeys = reinterpret_cast<const uint32_t*>(base + 2 * arr);
     const uint32_t* sslots = reinterpret_cast<const uint32_t*>(base + 3 * arr);
     const int64_t* starts = reinterpret_cast<const int64_t*>(base + 4 * arr);
-    int64_t blocks = (n * (width / 2) + 255) / 256;
+    int64_t blocks = (n * (pitch / 2) + 255) / 256;
     const int grid = (int)(blocks < RLCTR_SMS * 16 ? blocks : RLCTR_SMS * 16);
-    push_routed_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(skeys, sslots, starts, n, world, (int64_t)rank * cap, cap, src, width, sv);
+    push_routed_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(skeys, sslots, starts, n, world, (int64_t)rank * cap, cap, ps, pitch, sv);
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
+}
+
+// the one-source form: the same kernel, pitch = width (the same bytes in the same places as the multi call with n_src = 1)
+extern "C" int rlctr_push_rows_routed(const void* route_ws, int64_t n, int32_t world, int32_t rank, int64_t cap, const float* src,
+                                      int32_t width, void* const* peer_recv, rlctr_stream_t stream) {
+    if (!src) return RLCTR_EINVAL;
+    const float* srcs[1] = {src};
+    const int32_t widths[1] = {width};
+    return rlctr_push_rows_routed_multi(route_ws, n, world, rank, cap, srcs, widths, 1, peer_recv, stream);
 }
 
 extern "C" int rlctr_sort_routed_pos(const uint32_t* keys, int64_t n_in, int64_t n_rows_local, uint32_t* sorted_rows,

@@ -32,8 +32,13 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from . import _lib
+from . import colocated as _co
 from . import p_model as Model
 from .tables import Geometry, table_struct
+
+# the models with a dense tail (``_tail(z_table, rows)``) besides DeepFM, and the get_model names that differ from the class names
+TAIL_KINDS = ("WideAndDeep", "FNN", "InnerPNN", "OuterPNN", "DCN", "AFM")
+_ALIASES = {"W&D": "WideAndDeep", "IPNN": "InnerPNN", "OPNN": "OuterPNN"}
 
 
 def shard_rows(n_rows, world, rank):
@@ -168,9 +173,51 @@ def shared_sorted_view(x, n_rows, group):
     return view
 
 
+def _dense_member(kind, field_nums, latent_dims, device):
+    """The p_model module of ``kind`` as the dense part of a row-sharded model: its bias, tower, cross network or attention and the
+    ``_tail`` the stand-alone model runs, without an N-row table of its own (it is built over one row, which is dropped; the owner
+    re-homes ``table`` to its shard with :func:`_rehome`)."""
+    cls = getattr(Model, kind)
+    if kind == "LR":
+        m = cls(1, device=device)
+    elif kind == "FM":
+        m = cls(1, latent_dims, device=device)
+    else:
+        m = cls(1, field_nums, latent_dims, device=device)
+    del m.table
+    return m
+
+
+def _rehome(member, owner, geom):
+    """The member reads the owner's shard (not a parameter of the member: the owner lists it once) with geometry ``geom``;
+    flush / .to() go through the owner, and the member refuses to train on its own (p_model._TableModel._run)."""
+    member.__dict__["table"] = owner.table
+    member.__dict__["_group"] = owner
+    member._geom = geom
+    member._opt, member._stash = None, None
+
+
+def _copy_dense(dst, src):
+    """Every dense parameter of ``src`` (same class as ``dst``) into ``dst``, with what state_dict does not carry: the dropout
+    counters (``_rlctr_rng`` of every mlp.Tower and of AFM), AFM's ``dropout_p`` and the train / eval flags."""
+    sp = dict(src.named_parameters())
+    with torch.no_grad():
+        for name, p in dst.named_parameters():
+            p.data.copy_(sp[name].data)
+    for a, b in zip(dst.modules(), src.modules()):
+        a.training = b.training
+        st = getattr(b, "_rlctr_rng", None)
+        if st is not None:
+            a._rlctr_rng = st.clone()
+    if hasattr(src, "dropout_p"):
+        dst.dropout_p = src.dropout_p
+
+
 # ---------------------------------------------------------------------------------------------------
 class ShardedCTR(nn.Module):
-    """LR / FM / FFM / DeepFM with the table row-sharded over the process group.
+    """LR / FM / FFM / DeepFM, and the tail models WideAndDeep / FNN / InnerPNN / OuterPNN / DCN / AFM, with the table row-sharded
+    over the process group.  A tail model keeps its stand-alone row (16 floats, with or without the first-order column); its dense
+    part is the p_model module itself (``dense``: bias, tower, cross network or attention, and its ``_tail``).
 
     ``train_step(features, labels, optimizer)`` is the reference loop body (src/main/pretrain_main.py:96-102) for
     the local batch; ``forward(features)`` is the frozen scoring pass.  ``from_model`` shards an existing
@@ -179,7 +226,9 @@ class ShardedCTR(nn.Module):
 
     def __init__(self, kind, feature_nums, field_nums, latent_dims, group=None, device=None):
         super().__init__()
-        assert kind in ("LR", "FM", "FFM", "DeepFM")
+        kind = _ALIASES.get(kind, kind)
+        if kind not in ("LR", "FM", "FFM", "DeepFM") + TAIL_KINDS:
+            raise _lib.RlctrError(f"ShardedCTR: unknown model {kind!r} (LR, FM, FFM, DeepFM, {', '.join(TAIL_KINDS)})")
         self.kind, self.feature_nums, self.field_nums, self.latent_dims = kind, int(feature_nums), int(field_nums), int(latent_dims)
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
@@ -193,10 +242,11 @@ class ShardedCTR(nn.Module):
         elif kind == "FFM":
             g = Geometry.ffm(n_local, self.field_nums, self.latent_dims)
         else:
-            g = Geometry.fm(n_local, self.latent_dims)
+            g = Geometry.fm(n_local, self.latent_dims, with_linear=kind not in ("FNN", "InnerPNN", "OuterPNN", "DCN"))
         g = g.with_state()
         self._geom = g
-        self._kind = {"LR": "lr", "FM": "fm", "DeepFM": "fm", "FFM": "ffm"}[kind]
+        self._kind = {"LR": "lr", "FFM": "ffm"}.get(kind, "fm")
+        self._fm_term = kind in ("FM", "DeepFM")
         dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         self._pm = PeerMemory(n_alloc * g.row_pitch, torch.float32, dev, group)
         data = self._pm.local.view(n_alloc, g.row_pitch)
@@ -207,7 +257,13 @@ class ShardedCTR(nn.Module):
             data[:g.n_rows, used] = torch.randn(g.n_rows, len(used), device=dev)
         self.table = nn.Parameter(data)
         self.table._rlctr_owner = self
-        self.bias = nn.Parameter(torch.zeros(1, device=dev))
+        self.dense = None
+        if kind in TAIL_KINDS:
+            self.dense = _dense_member(kind, self.field_nums, self.latent_dims, dev)
+            _rehome(self.dense, self, g)
+            self.bias = getattr(self.dense, "bias", None)         # W&D, AFM: the member's own bias; FNN, PNN, DCN: none
+        else:
+            self.bias = nn.Parameter(torch.zeros(1, device=dev))
         self.mlp = Model._tower(self.field_nums * self.latent_dims, dev) if kind == "DeepFM" else None
         self._opt = None
         self._stash = None
@@ -260,6 +316,16 @@ class ShardedCTR(nn.Module):
     def barrier(self):
         self._pm.barrier()
 
+    @property
+    def _has_tail(self):
+        return self.mlp is not None or self.dense is not None
+
+    def _tail(self, z, rows):
+        """Logit [B, 1] from the table part z [B, 1] and the gathered rows [B, F*D]: the stand-alone model's ``_tail``."""
+        if self.dense is not None:
+            return self.dense._tail(z, rows)
+        return z + self.mlp(rows)                             # DeepFM
+
     @classmethod
     def from_model(cls, model, group=None):
         """Shard a single-GPU p_model instance (same parameters on every rank) over the group."""
@@ -269,7 +335,10 @@ class ShardedCTR(nn.Module):
         with torch.no_grad():
             shard = model.table.data[self.rank::self.world]
             self.table.data[:shard.shape[0]].copy_(shard)
-            self.bias.data.copy_(model.bias.data)
+            if self.dense is not None:
+                _copy_dense(self.dense, model)               # bias (W&D, AFM), towers, cross network, attention, dropout counters
+            else:
+                self.bias.data.copy_(model.bias.data)
             if self.mlp is not None:
                 self.mlp.load_state_dict(model.mlp.state_dict())
         self.barrier()
@@ -312,8 +381,8 @@ class ShardedCTR(nn.Module):
             return buf
         g = self._geom
         sizes = {"dlogit": (B + 3) // 4 * 4,
-                 "sums": B * g.row_stride if self._kind == "fm" else 0,
-                 "extra": B * F * g.dim if self.kind == "DeepFM" else 0,
+                 "sums": B * g.row_stride if self._fm_term else 0,
+                 "extra": B * F * g.dim if self._has_tail else 0,
                  "staged": B * F * g.row_stride if self._kind == "ffm" else 0}
         total = sum(sizes.values())
         pm = PeerMemory(total, torch.float32, self.table.device, self.group)
@@ -330,16 +399,16 @@ class ShardedCTR(nn.Module):
 
     def _exchange_buffers(self, B, F):
         """Receive side of the "push" exchange for batch size B: the all-gathered per-sample rows of every rank (plain local
-        tensors) and the symmetric buffer the sources write DeepFM's per-occurrence rows into."""
+        tensors) and the symmetric buffer the sources write the per-occurrence tail gradients into."""
         xb = self._xbuf.get(B)
         if xb is not None:
             return xb
         g, dev, G = self._geom, self.table.device, self.world
         bp = (B + 3) // 4 * 4
         xb = {"dlogit_all": torch.empty(G * bp, dtype=torch.float32, device=dev), "bp": bp, "sums_all": None, "recv": None}
-        if self._kind == "fm":
+        if self._fm_term:
             xb["sums_all"] = torch.empty(G * B * g.row_stride, dtype=torch.float32, device=dev)
-        if self.kind == "DeepFM":
+        if self._has_tail:
             pm = PeerMemory(G * B * F * g.dim, torch.float32, dev, self.group)
             pm.local.zero_()
             xb["recv"] = pm
@@ -363,13 +432,14 @@ class ShardedCTR(nn.Module):
                       None, 1, _lib.ptr(partners), B, F, self.latent_dims, _lib.stream(), key="rlctr_ffm_fwd[sharded]",
                       meta=self._meta(B, F))
         else:
-            sums = buf["sums"] if (train and self._kind == "fm") else None
+            sums = buf["sums"] if (train and self._fm_term) else None
             pitch = 0
-            if self.kind == "DeepFM":
+            if self._has_tail:
                 pitch = (F * g.dim + 3) // 4 * 4
                 trows = torch.empty(B, pitch, dtype=torch.float32, device=dev)
-            flags = _lib.RLCTR_FM_TERM if self.kind in ("FM", "DeepFM") else 0
-            _lib.call("rlctr_embed_fwd", lib.rlctr_embed_fwd, _lib.ptr(x), C.byref(t), _lib.ptr(self.bias.data), _lib.ptr(logit),
+            flags = _lib.RLCTR_FM_TERM if self._fm_term else 0
+            bias = self.bias.data if self.bias is not None else None
+            _lib.call("rlctr_embed_fwd", lib.rlctr_embed_fwd, _lib.ptr(x), C.byref(t), _lib.ptr(bias), _lib.ptr(logit),
                       None, 1, _lib.ptr(sums), _lib.ptr(trows), pitch, B, F, flags, _lib.stream(),
                       key=f"rlctr_embed_fwd[Sharded{self.kind}]",
                       meta=dict(self._meta(B, F), sums=sums is not None, rows=trows is not None, n_rows=self.feature_nums))
@@ -383,8 +453,8 @@ class ShardedCTR(nn.Module):
         self.flush()
         self.barrier()                                        # every shard is settled before anyone reads it
         logit, trows = self._interact(x, None, train=False)
-        if self.mlp is not None:
-            logit = logit + self.mlp(trows).reshape(-1)
+        if self._has_tail:
+            logit = self._tail(logit.view(-1, 1), trows).reshape(-1)
         self.barrier()                                        # nobody starts writing rows while a peer still reads
         return torch.sigmoid(logit).reshape(-1, 1)
 
@@ -409,31 +479,33 @@ class ShardedCTR(nn.Module):
         hook, self._after_gather = self._after_gather, None     # graphs.GraphedTrainStep: fork point of the captured step
         if hook is not None:
             hook()
-        tower_out = None
-        if self.mlp is not None:
+        z = None
+        if self._has_tail:
             trows.requires_grad_(True)
             with torch.enable_grad():
-                tower_out = self.mlp(trows).reshape(-1)
-            logit = logit + tower_out.detach()
+                z = self._tail(logit.view(B, 1), trows)
+            logit = z.detach().reshape(-1).contiguous()
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         dlogit = buf["dlogit"][:B]
-        dbias = torch.empty(1, dtype=torch.float32, device=dev)
+        dbias = torch.empty(1, dtype=torch.float32, device=dev) if self.bias is not None else None
         yi = y if y.dtype == torch.int64 else None
         yf = None if yi is not None else y.float()
         _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(logit), _lib.ptr(yi), _lib.ptr(yf), None, _lib.ptr(loss), _lib.ptr(dlogit),
                                          _lib.ptr(dbias), _lib.ptr(self._reduce_ws(dev)), B, st), "rlctr_bce_fwd_bwd")
         if self.world > 1:                                    # gradient of the GLOBAL mean loss
             dlogit.mul_(1.0 / self.world)
-            dbias.mul_(1.0 / self.world)
-        dz_in_sums = self.world > 1 and self._kind == "fm"
+            if dbias is not None:
+                dbias.mul_(1.0 / self.world)
+        dz_in_sums = self.world > 1 and self._fm_term
         if dz_in_sums:                                        # one aligned 64 B line per occurrence for the owners to pull
             buf["sums"].view(B, -1)[:, -1] = dlogit
         for p in self.parameters():
             p.grad = None
-        if tower_out is not None:
-            tower_out.backward(dlogit)
+        if z is not None:
+            z.backward(dlogit.view_as(z))
             buf["extra"].view(B, -1).copy_(trows.grad)
-        self.bias.grad = dbias
+        if self.bias is not None:
+            self.bias.grad = dbias
         if self.world > 1:
             dense = [p for p in self.parameters() if p is not self.table and p.grad is not None]
             flat = torch.cat([p.grad.reshape(-1) for p in dense])
@@ -497,43 +569,40 @@ def routed_view_pos(x, n_rows, group):
 
 
 # ---------------------------------------------------------------------------------------------------
-class _MemberGeom:
-    """Stand-in carrying the stand-alone geometry of a member kind for colocated._layout."""
-
-    def __init__(self, kind, n, d):
-        self._geom = Geometry.lr(n) if kind == "LR" else Geometry.fm(n, d)
-
-
 class ShardedGroup(nn.Module):
-    """Co-located records (colocated.py) over a row-sharded joint table: LR / FM / DeepFM trained on the same id stream share one
-    384-byte record per id, ``owner(id) = id mod G``.  Per step and rank: ONE routed sorted view (shared_sorted_view), one
-    catch-up of the owned records, one gather through the peer mapping (rlctr_group_fwd: one NVLink read per (sample, field)
-    for all members instead of one per member), one all_gather of the per-sample rows [B, 32] = column sums + every member's
-    dL/dlogit, one push of the tower-input gradients, one all_reduce of all dense gradients, two device barriers, one update
-    (rlctr_group_rows_adam).  The update equals the single-GPU group step on the concatenated global batch."""
+    """Co-located records (colocated.py) over a row-sharded joint table: the members ``colocate()`` accepts (LR, FM, DeepFM,
+    WideAndDeep, FNN, InnerPNN, OuterPNN, DCN, AFM) trained on the same id stream share one 384-byte record per id,
+    ``owner(id) = id mod G``.  Per step and rank: ONE routed sorted view (shared_sorted_view), one catch-up of the owned records, one
+    gather through the peer mapping (rlctr_group_fwd: one NVLink read per (sample, field) for all members instead of one per
+    member), one all_gather of the per-sample rows [B, 32] = column sums + the dL/dlogit of every member with a first-order or FM
+    column, ONE push of every dense-tail member's per-occurrence gradients (rlctr_push_rows_routed_multi: one interleaved row per
+    occurrence), one all_reduce of all dense gradients, two device barriers, one update (rlctr_group_rows_adam).  The update equals
+    the single-GPU group step on the concatenated global batch.  ``members[i]`` is the member's p_model module without a table of
+    its own: its bias, tower, cross network or attention, and the ``_tail`` the group step runs."""
 
     SUMS_PITCH = 32                    # one 128-byte line per sample: S (<= 28 floats) | dL/dlogit of members 0..3
 
     def __init__(self, kinds, feature_nums, field_nums, latent_dims, group=None, device=None):
         super().__init__()
-        from . import colocated as _co
-        kinds = tuple(kinds)
-        if not all(k in ("LR", "FM", "DeepFM") for k in kinds) or not 1 <= len(kinds) <= _lib.RLCTR_GROUP_MAX:
-            raise _lib.RlctrError("ShardedGroup members: LR, FM, DeepFM (up to four)")
+        kinds = tuple(_ALIASES.get(k, k) for k in kinds)
+        names = tuple(c.__name__ for c in _co.MEMBER_KINDS)
+        if not all(k in names for k in kinds) or not 1 <= len(kinds) <= _lib.RLCTR_GROUP_MAX:
+            raise _lib.RlctrError(f"ShardedGroup members: {', '.join(names)} (up to {_lib.RLCTR_GROUP_MAX}); got {', '.join(kinds)}")
         self.kinds, self.feature_nums, self.field_nums, self.latent_dims = kinds, int(feature_nums), int(field_nums), int(latent_dims)
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         if self.world not in (1, 2, 4, 8):
             raise _lib.RlctrError("row sharding supports 1, 2, 4 or 8 GPUs (owner = id & (G-1))")
+        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        members = [_dense_member(k, self.field_nums, self.latent_dims, dev) for k in kinds]
         n_local = max(shard_rows(self.feature_nums, self.world, self.rank), 1)
         n_alloc = max(shard_rows(self.feature_nums, self.world, 0), 1)
-        self._cols, used = _co._layout([_MemberGeom(k, n_local, self.latent_dims) for k in kinds])
+        self._cols, used = _co._layout(members)
         rs = (used + 1 + 3) // 4 * 4
         if rs > self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX:
             raise _lib.RlctrError("joint row too wide for the per-sample exchange row (28 floats)")
         self._geom = Geometry(n_local, rs, -1, 0, used, pitch=96, block=32, stamp_at=used)
-        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         self._pm = PeerMemory(n_alloc * 96, torch.float32, dev, group)
         data = self._pm.local.view(n_alloc, 96)
         data.zero_()
@@ -542,11 +611,21 @@ class ShardedGroup(nn.Module):
             data[:n_local, cols] = torch.randn(n_local, len(cols), device=dev)
         self.table = nn.Parameter(data)
         self.table._rlctr_owner = self
-        self.biases = nn.ParameterList([nn.Parameter(torch.zeros(1, device=dev)) for _ in kinds])
-        self.mlps = nn.ModuleList([Model._tower(self.field_nums * self.latent_dims, dev) if k == "DeepFM" else nn.Identity()
-                                   for k in kinds])
+        for m, (lin, emb, dim) in zip(members, self._cols):
+            _rehome(m, self, Geometry(n_local, rs, lin, emb, dim, pitch=96, block=32))
+        self.members = nn.ModuleList(members)
         self._opt, self._stash, self._ws, self._buf = None, None, {}, {}
         self.fork_ok = False
+
+    @property
+    def biases(self):
+        """The members' bias parameters (None for FNN, InnerPNN, OuterPNN, DCN)."""
+        return [getattr(m, "bias", None) for m in self.members]
+
+    @property
+    def mlps(self):
+        """The members' towers (``mlp``; nn.Identity for a member without one)."""
+        return [m.mlp if getattr(m, "mlp", None) is not None else nn.Identity() for m in self.members]
 
     # ---- protocol shared with optim.Adam / graphs ----------------------------------------------------------------------
     def _apply(self, fn, recurse=True):
@@ -568,6 +647,8 @@ class ShardedGroup(nn.Module):
 
     _reduce_ws = ShardedCTR._reduce_ws
     _rows_ws = Model._TableModel._rows_ws
+    _member_structs = _co.ColocatedCTR._member_structs
+    _z = staticmethod(_co.ColocatedCTR._z)
 
     def zero_grad(self, set_to_none=True):
         self._stash = None
@@ -578,20 +659,19 @@ class ShardedGroup(nn.Module):
 
     @classmethod
     def from_group(cls, cg, group=None):
-        """Shard a single-GPU colocated.ColocatedCTR (same parameters on every rank) over the process group."""
+        """Shard a single-GPU colocated.ColocatedCTR (same parameters on every rank) over the process group: the joint table, every
+        member's dense state and its dropout counters."""
         kinds = [type(m).__name__ for m in cg.members]
-        m0 = cg.members[-1]
-        self = cls(kinds, cg.feature_nums, getattr(m0, "field_nums", 15), max(getattr(m, "latent_dims", 1) for m in cg.members),
+        F = next((m.field_nums for m in cg.members if hasattr(m, "field_nums")), 15)
+        self = cls(kinds, cg.feature_nums, F, max(getattr(m, "latent_dims", 1) for m in cg.members),
                    group=group, device=cg.table.device)
         assert self._cols == cg._cols
         cg.flush()
         with torch.no_grad():
             shard = cg.table.data[self.rank::self.world]
             self.table.data[:shard.shape[0]].copy_(shard)
-            for i, m in enumerate(cg.members):
-                self.biases[i].data.copy_(m.bias.data)
-                if getattr(m, "mlp", None) is not None:
-                    self.mlps[i].load_state_dict(m.mlp.state_dict())
+        for dst, src in zip(self.members, cg.members):
+            _copy_dense(dst, src)
         self.barrier()
         return self
 
@@ -617,61 +697,56 @@ class ShardedGroup(nn.Module):
                 t.peers[r] = p
         return t
 
+    def _tail_sources(self):
+        """[(member, float offset in the interleaved receive row, width)] of the members with a dense tail, and the row's pitch:
+        each member's dim rounded up to even (the push moves 8-byte pieces)."""
+        out, off = [], 0
+        for i, m in enumerate(self.members):
+            if hasattr(m, "_tail"):
+                w = (self._cols[i][2] + 1) // 2 * 2
+                out.append((i, off, w))
+                off += w
+        return out, off
+
+    def _uses_dz(self, i):
+        """Member i reads its dL/dlogit in the update (a first-order column or the FM term); a tail-only member does not."""
+        lin, _, dim = self._cols[i]
+        return lin >= 0 or (self.members[i]._fm_term and dim > 0)
+
     def _exchange(self, B, F):
-        """Per batch size: this rank's per-sample exchange rows [B, 32], their all-gathered copy [G*B, 32], and per tower member
-        the symmetric receive buffer [G*n, D] the source ranks push their tower-input gradients into."""
+        """Per batch size: this rank's per-sample exchange rows [B, 32], their all-gathered copy [G*B, 32], and the ONE symmetric
+        receive buffer [G * cap, pitch] the source ranks push every dense-tail member's per-occurrence gradients into."""
         b = self._buf.get(B)
         if b is None:
-            dev, G, D = self.table.device, self.world, self.latent_dims
+            dev, G = self.table.device, self.world
             b = {"sums": torch.zeros(B, self.SUMS_PITCH, dtype=torch.float32, device=dev),
-                 "sums_all": torch.zeros(G * B, self.SUMS_PITCH, dtype=torch.float32, device=dev), "recv": {}}
-            for i, k in enumerate(self.kinds):
-                if k == "DeepFM" and G > 1:                   # dense per-source segments: [G * cap, D] (routed push)
-                    pm = PeerMemory(G * route_capacity(B * F, G) * D, torch.float32, dev, self.group)
-                    pm.local.zero_()
-                    b["recv"][i] = (pm, (C.c_void_p * 8)(*[int(p) for p in pm.ptrs]))
+                 "sums_all": torch.zeros(G * B, self.SUMS_PITCH, dtype=torch.float32, device=dev), "recv": None}
+            srcs, pitch = self._tail_sources()
+            if srcs and G > 1:                                # dense per-source segments of interleaved rows (routed push)
+                pm = PeerMemory(G * route_capacity(B * F, G) * pitch, torch.float32, dev, self.group)
+                pm.local.zero_()
+                b["recv"] = (pm, (C.c_void_p * 8)(*[int(p) for p in pm.ptrs]))
             self._buf[B] = b
         return b
 
-    def _members(self, B, F, dev):
-        arr = (_lib.Member * len(self.kinds))()
-        logits, rows = [], []
-        for i, (k, (lin, emb, dim)) in enumerate(zip(self.kinds, self._cols)):
-            s = arr[i]
-            s.lin_col, s.emb_col, s.dim = lin, emb, dim
-            s.flags = _lib.RLCTR_FM_TERM if k in ("FM", "DeepFM") else 0
-            s.bias = _lib.ptr(self.biases[i].data)
-            z = torch.empty(B, dtype=torch.float32, device=dev)
-            s.logit = _lib.ptr(z)
-            logits.append(z)
-            r = None
-            if k == "DeepFM":
-                pitch = (F * dim + 3) // 4 * 4
-                r = torch.empty(B, pitch, dtype=torch.float32, device=dev)
-                s.rows_out, s.rows_pitch = r.data_ptr(), pitch
-            rows.append(r)
-        return arr, logits, rows
-
     @torch.no_grad()
     def forward(self, x):
-        """pCTR of every member, float32 [B, M]."""
+        """pCTR of every member, float32 [B, M] (as colocated.ColocatedCTR.forward, the rows read through the peer mapping)."""
         lib = _lib.load()
         x = Model._check_ids(x)
         B, F = x.shape
         self.flush()
         self.barrier()
-        arr, logits, rows = self._members(B, F, x.device)
+        out = torch.empty(B, len(self.members), dtype=torch.float32, device=x.device)
+        arr, logits, rows = self._member_structs(B, F, x.device, False, pctr=out)
         t = self._global_struct()
-        _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, len(self.kinds), None, 0, B, F, _lib.stream(),
-                  key="rlctr_group_fwd[sharded infer]", meta=self._meta(B, F))
-        out = []
-        for i, k in enumerate(self.kinds):
-            z = logits[i]
+        _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, len(self.members), None, 0, B, F,
+                  _lib.stream(), key="rlctr_group_fwd[sharded infer]", meta=self._meta(B, F))
+        for i, m in enumerate(self.members):
             if rows[i] is not None:
-                z = z + self.mlps[i](rows[i][:, :F * self._cols[i][2]]).reshape(-1)
-            out.append(torch.sigmoid(z))
+                out[:, i:i + 1] = torch.sigmoid(m._tail(self._z(logits[i], B), rows[i][:, :F * self._cols[i][2]]))
         self.barrier()
-        return torch.stack(out, dim=1)
+        return out
 
     def train_step(self, features, labels, optimizer):
         """One step of every member on the local batch; returns the local mean BCE losses, float32 [M]."""
@@ -697,7 +772,7 @@ class ShardedGroup(nn.Module):
             _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(srows), n_all, C.byref(t), C.byref(a), st,
                       key="rlctr_rows_catchup[ShardedGroup]", meta=self._meta(n_all // F, F))
         self.barrier()                                        # B1: all owners caught their rows up | forward reads
-        arr, logits, rows = self._members(B, F, dev)
+        arr, logits, rows = self._member_structs(B, F, dev, True)
         t = self._global_struct()
         sums = buf["sums"]
         _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, M, _lib.ptr(sums), self.SUMS_PITCH, B, F, st,
@@ -706,26 +781,31 @@ class ShardedGroup(nn.Module):
         ws = self._reduce_ws(dev)
         for p in self.parameters():
             p.grad = None
-        extras = [None] * M
-        for i, k in enumerate(self.kinds):
+        extras, pitches = [None] * M, [0] * M
+        for i, m in enumerate(self.members):
             dl = torch.empty(B, dtype=torch.float32, device=dev)
-            dbias = torch.empty(1, dtype=torch.float32, device=dev)
-            z, tower_out, leaf = logits[i], None, None
-            if rows[i] is not None:
+            bias = getattr(m, "bias", None)
+            dbias = torch.empty(1, dtype=torch.float32, device=dev) if bias is not None else None
+            z = leaf = None
+            if rows[i] is None:                               # LR, FM: the table logit is the logit
+                zz = logits[i]
+            else:                                             # dense tail: the member's own _tail, autograd over it only
                 leaf = rows[i][:, :F * self._cols[i][2]].detach().requires_grad_(True)
-                with torch.enable_grad():
-                    tower_out = self.mlps[i](leaf).reshape(-1)
-                z = z + tower_out.detach()
-            _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(z), _lib.ptr(yi), _lib.ptr(yf), None, losses.data_ptr() + 4 * i, _lib.ptr(dl),
+                z = m._tail(self._z(logits[i], B), leaf)
+                zz = z.detach().reshape(-1).contiguous()
+            _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(zz), _lib.ptr(yi), _lib.ptr(yf), None, losses.data_ptr() + 4 * i, _lib.ptr(dl),
                                              _lib.ptr(dbias), _lib.ptr(ws), B, st), "rlctr_bce_fwd_bwd")
             if G > 1:                                         # gradient of the GLOBAL mean loss
                 dl.mul_(1.0 / G)
-                dbias.mul_(1.0 / G)
-            sums[:, self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX + i] = dl    # dL/dlogit rides in the sample's exchange row
-            if tower_out is not None:
-                tower_out.backward(dl)
+                if dbias is not None:
+                    dbias.mul_(1.0 / G)
+            if self._uses_dz(i):
+                sums[:, self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX + i] = dl    # dL/dlogit rides in the sample's exchange row
+            if z is not None:
+                z.backward(dl.view_as(z))
                 extras[i] = leaf.grad.contiguous()
-            self.biases[i].grad = dbias
+            if bias is not None:
+                bias.grad = dbias
         if G > 1:
             dense = [p for p in self.parameters() if p is not self.table and p.grad is not None]
             flat = torch.cat([p.grad.reshape(-1) for p in dense])
@@ -736,29 +816,41 @@ class ShardedGroup(nn.Module):
                 o += p.numel()
             dist.all_gather_into_tensor(buf["sums_all"], sums, group=self.group)
             sums_all = buf["sums_all"]
-            for i, (pm, ptrs) in buf["recv"].items():          # per-occurrence rows, in the routed bucket order: coalesced posted
-                n = B * F                                      # writes into dense per-source segments of the owners' memory
-                _lib.call("rlctr_push_rows_routed", lib.rlctr_push_rows_routed, _lib.ptr(view["route_ws"]), n, G, self.rank,
-                          view["cap"], _lib.ptr(extras[i]), self.latent_dims, ptrs, st, key="rlctr_push_rows",
-                          meta={"n": n, "width": self.latent_dims})
-                extras[i] = pm.local
+            if buf["recv"] is not None:                       # ONE push of every tail member's per-occurrence rows, in the routed
+                pm, ptrs = buf["recv"]                        # bucket order: interleaved rows, coalesced posted writes
+                n = B * F
+                tails, pitch = self._tail_sources()
+                keep = []
+                for i, off, w in tails:
+                    src = extras[i].view(n, -1)
+                    if src.shape[1] != w:                     # odd dim: a zero pad column (carried, never read by the update)
+                        src = torch.nn.functional.pad(src, (0, w - src.shape[1]))
+                    keep.append(src)
+                srcs = (C.c_void_p * len(keep))(*[s_.data_ptr() for s_ in keep])
+                widths = (C.c_int32 * len(keep))(*[w for _, _, w in tails])
+                _lib.call("rlctr_push_rows_routed_multi", lib.rlctr_push_rows_routed_multi, _lib.ptr(view["route_ws"]), n, G,
+                          self.rank, view["cap"], srcs, widths, len(keep), ptrs, st, key="rlctr_push_rows",
+                          meta={"n": n, "width": pitch, "sources": len(keep)})
+                for i, off, _ in tails:
+                    extras[i], pitches[i] = pm.local[off:], pitch
         else:
             sums_all = sums
         self.barrier()                                        # B2: every rank's gradient-side buffers are complete
         self._stash = {"sorted_ids": srows, "sorted_slots": sslots, "n": n_all, "fields": F, "sums": sums_all, "extra": extras,
-                       "slot_of": view["slot_of"] if view is not None else None}
+                       "extra_pitch": pitches, "slot_of": view["slot_of"] if view is not None else None}
         optimizer.step()
         return losses
 
     def _group_update(self, stash, opt_state, st):
         lib = _lib.load()
         arr = (_lib.Member * len(self.kinds))()
-        for i, (k, (lin, emb, dim)) in enumerate(zip(self.kinds, self._cols)):
+        for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
             s = arr[i]
             s.lin_col, s.emb_col, s.dim = lin, emb, dim
-            s.flags = _lib.RLCTR_FM_TERM if k in ("FM", "DeepFM") else 0
+            s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
             s.dlogit = None                                   # in the exchange rows
             s.extra = _lib.ptr(stash["extra"][i])
+            s.extra_pitch = stash["extra_pitch"][i]
         t, a = table_struct(self.table.data, self._geom), opt_state.struct()
         n, F = stash["n"], stash["fields"]
         ws_bytes = lib.rlctr_rows_ws_bytes(n)
