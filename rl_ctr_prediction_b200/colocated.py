@@ -30,6 +30,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+from dataclasses import dataclass
 
 import torch
 import torch.nn as nn
@@ -51,13 +52,63 @@ MEMBER_KINDS = (Model.LR, Model.FM, Model.DeepFM, Model.WideAndDeep, Model.FNN, 
 UNSORTED_CATCHUP = os.environ.get("RLCTR_GROUP_UNSORTED_CATCHUP", "0") != "0"
 
 
+@dataclass(slots=True)
 class GroupStash:
-    """What a group step leaves for the optimizer: the sorted view, the joint column sums and each member's gradient side."""
-    __slots__ = ("sorted_ids", "sorted_slots", "n", "fields", "sums", "dlogit", "extra")
+    """What a group step leaves for the optimizer: the sorted view, the joint column sums and each member's gradient side.  The
+    last four fields describe the row-sharded group's exchange (sharded.ShardedGroup); their defaults are the one-device group's."""
+    sorted_ids: torch.Tensor
+    sorted_slots: torch.Tensor
+    n: int
+    fields: int
+    sums: torch.Tensor
+    dlogit: list                       # per member: dL/dlogit [B], or None when it rides in the sums row
+    extra: list                        # per member: the tower-input gradient rows, or None
+    sums_pitch: int = 0                # floats between two samples' sums rows; 0 = the record's row_stride
+    world: int = 1
+    slot_of: torch.Tensor | None = None    # routed exchange: the global slot at every receive position
+    extra_pitch: list | None = None        # per member: floats between two rows of ``extra``; None = 0 for every member
 
-    def __init__(self, **kw):
-        for k in self.__slots__:
-            setattr(self, k, kw.get(k))
+
+def labels(y):
+    """(int64 labels, None) or (None, float32 labels): what rlctr_bce_fwd_bwd reads."""
+    y = y.reshape(-1).contiguous()
+    return (y, None) if y.dtype == torch.int64 else (None, y.float())
+
+
+def loss_head(m, logit, rows, y, loss, ws, dl=None, scale=1.0):
+    """Sigmoid + BCE of one model's logit and their gradient (rlctr_bce_fwd_bwd).  ``logit`` [B] is the table part (None for a
+    model without one); with tower rows [B, F*D] the logit is ``m._tail(logit, rows)``, run under autograd on a detached leaf.
+    ``scale`` multiplies dL/dlogit and the bias gradient before the tail's backward (1/G in a row-sharded step: the gradient of
+    the GLOBAL mean loss).  ``y``: :func:`labels`; the loss goes to the device address ``loss``, dL/dlogit to ``dl`` (allocated
+    when None), the bias gradient to ``m.bias.grad``.  Returns (dL/dlogit [B], the gradient of ``rows`` or None)."""
+    lib = _lib.load()
+    src = rows if rows is not None else logit
+    B, dev = src.shape[0], src.device
+    dl = torch.empty(B, dtype=torch.float32, device=dev) if dl is None else dl
+    bias = getattr(m, "bias", None)
+    dbias = torch.empty(1, dtype=torch.float32, device=dev) if bias is not None else None
+    z = leaf = None
+    if rows is None:
+        zz = logit
+    else:
+        leaf = rows.detach().requires_grad_(True)
+        z = m._tail(logit.view(B, 1) if logit is not None else None, leaf)
+        zz = z.detach().reshape(-1).contiguous()
+    # (the head's own sum of dlogit is the bias gradient: the same block partition and tree as the stand-alone backward's
+    # rlctr_sigmoid_bwd sum -- the same bits, one launch less)
+    _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(zz), _lib.ptr(y[0]), _lib.ptr(y[1]), None, loss, _lib.ptr(dl), _lib.ptr(dbias),
+                                     _lib.ptr(ws), B, _lib.stream()), "rlctr_bce_fwd_bwd")
+    if scale != 1.0:
+        dl.mul_(scale)
+        if dbias is not None:
+            dbias.mul_(scale)
+    grad = None
+    if z is not None:
+        z.backward(dl.view_as(z))
+        grad = leaf.grad.contiguous()
+    if bias is not None:
+        bias.grad = dbias
+    return dl, grad
 
 
 def _layout(members):
@@ -93,12 +144,97 @@ def _layout(members):
     return cols, used
 
 
-class ColocatedCTR(Model._TableModel):
+class _GroupStep:
+    """The parts of a group step that do not depend on where the joint table lives, shared by ColocatedCTR (one device) and
+    sharded.ShardedGroup (row-sharded).  The class provides ``members``, ``_cols``, ``_geom``, ``table``, ``_meta``,
+    ``_reduce_ws``, ``_rows_ws``, ``_global_struct()`` (the table as the gathers read it) and ``_UPDATE_KEY``."""
+
+    def _member_structs(self, B, F, dev, train, pctr=None):
+        """The members' views for rlctr_group_fwd.  logits[i]: the table part of member i's logit (bias + first order + FM
+        term), None for a member that has none (FNN, InnerPNN, OuterPNN, DCN: no linear column, no bias); rows[i]: the tower
+        input [B, pitch] of a member with a dense tail, else None."""
+        arr = (_lib.Member * len(self.members))()
+        logits, rows = [], []
+        for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
+            s = arr[i]
+            s.lin_col, s.emb_col, s.dim = lin, emb, dim
+            s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
+            bias = getattr(m, "bias", None)
+            s.bias = _lib.ptr(bias.data) if bias is not None else None
+            tail = hasattr(m, "_tail")
+            table_part = lin >= 0 or bias is not None or m._fm_term
+            z = torch.empty(B, dtype=torch.float32, device=dev) if table_part and (train or tail) else None
+            logits.append(z)
+            s.logit = _lib.ptr(z)
+            if pctr is not None and not tail:
+                s.pctr, s.pctr_stride = pctr.data_ptr() + 4 * i, pctr.shape[1]
+            r = None
+            if tail:
+                pitch = round4(F * dim)                      # 16-byte aligned pitch: the tower's first GEMM fetches it by TMA
+                r = torch.empty(B, pitch, dtype=torch.float32, device=dev)
+                s.rows_out, s.rows_pitch = r.data_ptr(), pitch
+            rows.append(r)
+        return arr, logits, rows
+
+    def _pctr(self, x, key):
+        """pCTR of every member on one gather: float32 [B, M] (column m = ``members[m](x)``)."""
+        lib = _lib.load()
+        B, F = x.shape
+        out = torch.empty(B, len(self.members), dtype=torch.float32, device=x.device)
+        arr, logits, rows = self._member_structs(B, F, x.device, False, pctr=out)
+        t = self._global_struct()
+        _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, len(self.members), None, 0, B, F,
+                  _lib.stream(), key=key, meta=self._meta(B, F))
+        for i, m in enumerate(self.members):
+            if rows[i] is not None:
+                z = logits[i].view(B, 1) if logits[i] is not None else None
+                out[:, i:i + 1] = torch.sigmoid(m._tail(z, rows[i][:, :F * self._cols[i][2]]))
+        return out
+
+    def _heads(self, F, logits, rows, y, scale=1.0):
+        """Every member's loss head (:func:`loss_head`) on the group's gather, the dense gradients set afresh.  Returns the losses
+        float32 [M], and dL/dlogit and the tower-input gradient (or None) per member."""
+        for p in self.parameters():
+            p.grad = None
+        losses = torch.empty(len(self.members), dtype=torch.float32, device=self.table.device)
+        ws = self._reduce_ws(self.table.device)
+        dlogits, extras = [], []
+        for i, m in enumerate(self.members):
+            r = rows[i][:, :F * self._cols[i][2]] if rows[i] is not None else None
+            dl, grad = loss_head(m, logits[i], r, y, losses.data_ptr() + 4 * i, ws, scale=scale)
+            dlogits.append(dl)
+            extras.append(grad)
+        return losses, dlogits, extras
+
+    def _group_update(self, stash, opt_state, st):
+        """optim.Adam.step() for the joint table: rlctr_group_rows_adam."""
+        lib = _lib.load()
+        M = len(self.members)
+        arr = (_lib.Member * M)()
+        pitches = stash.extra_pitch or [0] * M
+        for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
+            s = arr[i]
+            s.lin_col, s.emb_col, s.dim = lin, emb, dim
+            s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
+            s.dlogit = _lib.ptr(stash.dlogit[i])
+            s.extra = _lib.ptr(stash.extra[i])
+            s.extra_pitch = pitches[i]
+        t, a = table_struct(self.table.data, self._geom), opt_state.struct()
+        ws_bytes = lib.rlctr_rows_ws_bytes(stash.n)
+        ws = self._rows_ws(ws_bytes)
+        _lib.call("rlctr_group_rows_adam", lib.rlctr_group_rows_adam, _lib.ptr(stash.sorted_ids), _lib.ptr(stash.sorted_slots),
+                  stash.n, C.byref(t), C.byref(a), arr, M, _lib.ptr(stash.sums), stash.sums_pitch, stash.fields, stash.world,
+                  _lib.ptr(stash.slot_of), _lib.ptr(ws), ws_bytes, st, key=self._UPDATE_KEY,
+                  meta=self._meta(stash.n // stash.fields, stash.fields))
+
+
+class ColocatedCTR(_GroupStep, Model._TableModel):
     """``colocate(models)``: LR / FM-type drop-in models (``MEMBER_KINDS``) over one joint table.  The group owns the table,
     its lazy-exact Adam state and the training step; the members keep ``forward`` (inference), ``state_dict`` /
     ``load_state_dict`` (reference keys) and their dense parameters."""
 
     _kind = "group"
+    _UPDATE_KEY = "rlctr_group_rows_adam"
 
     def __init__(self, models):
         super().__init__()
@@ -162,54 +298,16 @@ class ColocatedCTR(Model._TableModel):
         return {"model": "+".join(type(m).__name__ for m in self.members), "B": B, "F": F, "rs": g.row_stride, "dim": g.dim,
                 "n_rows": g.n_rows, "lin": False, "members": [(type(m).__name__, c[2]) for m, c in zip(self.members, self._cols)]}
 
-    # ---- forward of every member from one gather ---------------------------------------------------------------------
-    def _member_structs(self, B, F, dev, train, pctr=None):
-        """The members' views for rlctr_group_fwd.  logits[i]: the table part of member i's logit (bias + first order + FM
-        term), None for a member that has none (FNN, InnerPNN, OuterPNN, DCN: no linear column, no bias); rows[i]: the tower
-        input [B, pitch] of a member with a dense tail, else None."""
-        arr = (_lib.Member * len(self.members))()
-        logits, rows = [], []
-        for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
-            s = arr[i]
-            s.lin_col, s.emb_col, s.dim = lin, emb, dim
-            s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
-            bias = getattr(m, "bias", None)
-            s.bias = _lib.ptr(bias.data) if bias is not None else None
-            tail = hasattr(m, "_tail")
-            table_part = lin >= 0 or bias is not None or m._fm_term
-            z = torch.empty(B, dtype=torch.float32, device=dev) if table_part and (train or tail) else None
-            logits.append(z)
-            s.logit = _lib.ptr(z)
-            if pctr is not None and not tail:
-                s.pctr, s.pctr_stride = pctr.data_ptr() + 4 * i, pctr.shape[1]
-            r = None
-            if tail:
-                pitch = round4(F * dim)                      # 16-byte aligned pitch: the tower's first GEMM fetches it by TMA
-                r = torch.empty(B, pitch, dtype=torch.float32, device=dev)
-                s.rows_out, s.rows_pitch = r.data_ptr(), pitch
-            rows.append(r)
-        return arr, logits, rows
+    def _global_struct(self):
+        """The joint table as the gathers read it (one device: the table itself)."""
+        return table_struct(self.table.data, self._geom)
 
     @torch.no_grad()
     def forward(self, x):
         """pCTR of every member on one gather: float32 [B, M] (column m = ``members[m](x)``)."""
-        lib = _lib.load()
         x = Model._check_ids(x)
-        B, F = x.shape
         self.flush()
-        out = torch.empty(B, len(self.members), dtype=torch.float32, device=x.device)
-        arr, logits, rows = self._member_structs(B, F, x.device, False, pctr=out)
-        t = table_struct(self.table.data, self._geom)
-        _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, len(self.members), None, 0, B, F,
-                  _lib.stream(), key="rlctr_group_fwd[infer]", meta=self._meta(B, F))
-        for i, m in enumerate(self.members):
-            if rows[i] is not None:
-                out[:, i:i + 1] = torch.sigmoid(m._tail(self._z(logits[i], B), rows[i][:, :F * self._cols[i][2]]))
-        return out
-
-    @staticmethod
-    def _z(logit, B):
-        return logit.view(B, 1) if logit is not None else None
+        return self._pctr(x, "rlctr_group_fwd[infer]")
 
     # ---- the training step ---------------------------------------------------------------------------------------
     def train_step(self, x, y, optimizer):
@@ -223,9 +321,7 @@ class ColocatedCTR(Model._TableModel):
         x = Model._check_ids(x)
         B, F = x.shape
         dev, st, g = x.device, _lib.stream(), self._geom
-        yy = y.reshape(-1).contiguous()
-        yi = yy if yy.dtype == torch.int64 else None
-        yf = None if yi is not None else yy.float()
+        y = labels(y)
         t = table_struct(self.table.data, g)
         # The sorted view is needed by the scatter at the END of the step only: with the catch-up working from the ids in batch
         # order (rlctr_rows_catchup_ids: a claim bit per row tells the occurrences of an id apart) the sort runs on its own
@@ -257,56 +353,12 @@ class ColocatedCTR(Model._TableModel):
         sums = torch.empty(B, g.row_stride, dtype=torch.float32, device=dev)
         _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, M, _lib.ptr(sums), 0, B, F, st,
                   key="rlctr_group_fwd[train]", meta=self._meta(B, F))
-        losses = torch.empty(M, dtype=torch.float32, device=dev)
-        dlogits, extras = [], []
-        ws = self._reduce_ws(dev)
-        for i, m in enumerate(self.members):
-            dl = torch.empty(B, dtype=torch.float32, device=dev)
-            dbias = torch.empty(1, dtype=torch.float32, device=dev)
-            bias = getattr(m, "bias", None)
-            if rows[i] is None:                              # LR, FM: the loss head and its gradient in one call
-                _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(logits[i]), _lib.ptr(yi), _lib.ptr(yf), None,
-                                                 losses.data_ptr() + 4 * i, _lib.ptr(dl), _lib.ptr(dbias), _lib.ptr(ws), B, st),
-                           "rlctr_bce_fwd_bwd")
-                extras.append(None)
-            else:                                            # dense tail: autograd over the member's tail only
-                fd = F * self._cols[i][2]
-                leaf = rows[i][:, :fd].detach().requires_grad_(True)
-                z = m._tail(self._z(logits[i], B), leaf)
-                zz = z.detach().reshape(-1).contiguous()
-                # (the head's own sum of dlogit is the bias gradient: the same block partition and tree as the stand-alone
-                # backward's rlctr_sigmoid_bwd sum -- the same bits, one launch less)
-                _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(zz), _lib.ptr(yi), _lib.ptr(yf), None, losses.data_ptr() + 4 * i,
-                                                 _lib.ptr(dl), _lib.ptr(dbias) if bias is not None else None, _lib.ptr(ws), B, st),
-                           "rlctr_bce_fwd_bwd")
-                m.zero_grad()
-                z.backward(dl.view_as(z))
-                extras.append(leaf.grad.contiguous())
-            if bias is not None:
-                bias.grad = dbias
-            dlogits.append(dl)
+        losses, dlogits, extras = self._heads(F, logits, rows, y)
         self._stash = GroupStash(sorted_ids=sid, sorted_slots=sslot, n=B * F, fields=F, sums=sums, dlogit=dlogits, extra=extras)
         if side is not None:
             torch.cuda.current_stream(dev).wait_stream(side)     # join: the scatter reads the sorted view
         optimizer.step()
         return losses
-
-    def _group_update(self, stash, opt_state, st):
-        """optim.Adam.step() for the joint table: rlctr_group_rows_adam."""
-        lib = _lib.load()
-        arr = (_lib.Member * len(self.members))()
-        for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
-            s = arr[i]
-            s.lin_col, s.emb_col, s.dim = lin, emb, dim
-            s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
-            s.dlogit = _lib.ptr(stash.dlogit[i])
-            s.extra = _lib.ptr(stash.extra[i])
-        t, a = table_struct(self.table.data, self._geom), opt_state.struct()
-        ws_bytes = lib.rlctr_rows_ws_bytes(stash.n)
-        ws = self._rows_ws(ws_bytes)
-        _lib.call("rlctr_group_rows_adam", lib.rlctr_group_rows_adam, _lib.ptr(stash.sorted_ids), _lib.ptr(stash.sorted_slots),
-                  stash.n, C.byref(t), C.byref(a), arr, len(self.members), _lib.ptr(stash.sums), 0, stash.fields, 1, None,
-                  _lib.ptr(ws), ws_bytes, st, key="rlctr_group_rows_adam", meta=self._meta(stash.n // stash.fields, stash.fields))
 
 
 def colocate(models) -> ColocatedCTR:

@@ -5,22 +5,24 @@ over NVLink/NVSwitch).  Samples are data-parallel; every table is row-sharded: `
 ``local_row(id) = id div G`` (modulo spreads the Zipf heads of a dictionary-ranked vocabulary); optimizer state
 is sharded with the rows.  Dense parameters (bias, tower) are replicated and their gradients all-reduced (NCCL).
 
-The lookup and the gradient exchange are NOT collectives: every shard (and every rank's small gradient-side
-buffers) lives in symmetric memory -- peer-mapped over NVLink -- and the kernels address it directly:
+Every shard (and every rank's small gradient-side buffers) lives in symmetric memory -- peer-mapped over NVLink -- and
+the kernels address it directly:
 
     forward   rlctr_embed_fwd / rlctr_ffm_fwd read row ``id`` at ``peers[id % G] + (id / G) * pitch``: the gather
               IS the exchange (64 B NVLink reads; measured 529 GB/s for random rows, profiles/r1_symm_probe.md);
-    backward  every rank leaves dlogit / column sums / tower-input gradients in its symmetric buffers; the OWNER of a
-              row pulls them (``rlctr_rowgrad.peer_*``) inside the sort / segment-reduce / fused-Adam kernel and
-              recomputes the row gradient exactly as the single-GPU kernel does.
+    backward  the per-sample rows (dlogit, column sums) are replicated with one ``all_gather``; the source rank PUSHES the
+              per-occurrence rows (tower-input gradients) into the owner's receive buffer (posted NVLink writes).  The owner's
+              sort / segment-reduce / fused-Adam kernel reads them through ``rlctr_rowgrad.peer_*`` -- local memory, except
+              FFM's partner rows, which it reads on the source rank through the peer mapping -- and recomputes the row
+              gradient exactly as the single-GPU kernel does.
 
-What does travel as a collective is the id list: one fixed-size ``all_gather`` of the batch's ids per step (4 B per
-gathered row, shared by every model fed with that batch).  Each rank keeps the ids it owns (sentinel keys for the
-rest), sorts them once (``rlctr_sort_ids_sharded``) and uses that view for the lazy-Adam catch-up and for the
-update.  Two device-side barriers per model step order the phases (catch-up | forward reads ... backward | owner
-update); nothing synchronises with the host and no count ever leaves the device, so the sharded step is as
-graph-capturable as the single-GPU one.  The owner walks occurrences in (source rank, slot) order: a sharded step
-is bit-identical from run to run and equal to the single-GPU step on the concatenated batch.
+The ids reach their owners the same way: every rank writes the (local row, global slot) pairs of the ids a peer owns into
+that peer's receive buffer and each owner sorts what it received (``shared_sorted_view``; ``RLCTR_SHARD_ROUTE=0``: one
+``all_gather`` of the ids and ``rlctr_sort_ids_sharded``).  That sorted view serves the lazy-Adam catch-up and the update.
+Two device-side barriers per model step order the phases (catch-up | forward reads ... backward | owner update); nothing
+synchronises with the host and no count ever leaves the device, so the sharded step is as graph-capturable as the
+single-GPU one.  The owner walks occurrences in (source rank, slot) order: a sharded step is bit-identical from run to
+run and equal to the single-GPU step on the concatenated batch.
 """
 from __future__ import annotations
 
@@ -109,12 +111,39 @@ def _route_buffers(n, world, dev, group):
 
 
 def check_route_overflow():
-    """Host-side check of the routing overflow flags (one device -> host read each; called from ShardedCTR.flush)."""
+    """Host-side check of the routing overflow flags (one device -> host read each; called from flush)."""
     for (n, world, _), rb in _ROUTE.items():
         if int(rb["overflow"].item()) != 0:
             raise _lib.RlctrError(f"owner routing overflow: some rank sent more than {rb['cap']} of its {n} ids to one owner "
                                   f"(skewed ids); the steps since the last check are incomplete.  Rerun with a larger "
-                                  f"RLCTR_ROUTE_CAP (now {os.environ.get('RLCTR_ROUTE_CAP', '1.5')}) or RLCTR_SHARD_ROUTE=0")
+                                  f"RLCTR_ROUTE_CAP (now {os.environ.get('RLCTR_ROUTE_CAP', '1.5')}); ShardedCTR models can "
+                                  f"also run without routing (RLCTR_SHARD_ROUTE=0), ShardedGroup always routes")
+
+
+def _route(x, n_rows, group):
+    """Owner routing of the batch's ids: every rank writes the (local row, global slot) pairs of the ids a peer owns straight
+    into that peer's receive buffer (rlctr_route_ids: posted NVLink writes, a fixed capacity per source), then one device
+    barrier.  Returns what the owner's sort of its G * cap received pairs needs: the received ``keys`` (local rows) and
+    ``slot_of`` (global slots), ``n_all``, ``n_local``, the sort's outputs ``rows`` and ``out`` (int32 [n_all]) and its
+    workspace ``ws`` / ``ws_bytes``; and ``cap`` and ``route_ws`` (the bucket order of this rank's ids, which the routed
+    gradient push reuses)."""
+    lib = _lib.load()
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    dev, n = x.device, x.numel()
+    rb = _route_buffers(n, world, dev, group)
+    cap = rb["cap"]
+    ws_bytes = lib.rlctr_route_ws_bytes(n, world)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    _lib.call("rlctr_route_ids", lib.rlctr_route_ids, _lib.ptr(x), n, world, rank, n_rows, cap, rb["kp"], rb["vp"],
+              _lib.ptr(rb["overflow"]), _lib.ptr(ws), ws_bytes, _lib.stream(), meta={"n": n, "world": world, "cap": cap})
+    rb["keys"].barrier()                                         # every source's segment of my receive buffer is complete
+    n_all = world * cap
+    r = {"keys": rb["keys"].local, "slot_of": rb["vals"].local, "cap": cap, "route_ws": ws, "n_all": n_all,
+         "n_local": max(shard_rows(n_rows, world, rank), 1),
+         "rows": torch.empty(n_all, dtype=torch.int32, device=dev), "out": torch.empty(n_all, dtype=torch.int32, device=dev)}
+    r["ws_bytes"] = lib.rlctr_sort_ws_bytes(n_all, r["n_local"])
+    r["ws"] = torch.empty(r["ws_bytes"], dtype=torch.uint8, device=dev)
+    return r
 
 
 def shared_sorted_view(x, n_rows, group):
@@ -136,41 +165,38 @@ def shared_sorted_view(x, n_rows, group):
     n = x.numel()
     st = _lib.stream()
     if world > 1 and os.environ.get("RLCTR_SHARD_ROUTE", "1") == "1":
-        rb = _route_buffers(n, world, dev, group)
-        cap = rb["cap"]
-        ws_bytes = lib.rlctr_route_ws_bytes(n, world)
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        _lib.call("rlctr_route_ids", lib.rlctr_route_ids, _lib.ptr(x), n, world, rank, n_rows, cap, rb["kp"], rb["vp"],
-                  _lib.ptr(rb["overflow"]), _lib.ptr(ws), ws_bytes, st, meta={"n": n, "world": world, "cap": cap})
-        rb["keys"].barrier()                                     # every source's segment of my receive buffer is complete
-        n_all = world * cap
+        r = _route(x, n_rows, group)
+        _lib.call("rlctr_sort_routed", lib.rlctr_sort_routed, _lib.ptr(r["keys"]), _lib.ptr(r["slot_of"]), r["n_all"], r["n_local"],
+                  _lib.ptr(r["rows"]), _lib.ptr(r["out"]), _lib.ptr(r["ws"]), r["ws_bytes"], st, key="rlctr_sort_ids",
+                  meta={"n": r["n_all"]})
+        view = (r["rows"], r["out"], r["n_all"])
+    else:
+        ids32 = x.reshape(-1).clamp(-1, n_rows).to(torch.int32)          # out-of-range ids stay out of range in 32 bits
+        if world > 1:
+            all32 = torch.empty(world * n, dtype=torch.int32, device=dev)
+            dist.all_gather_into_tensor(all32, ids32, group=group)
+        else:
+            all32 = ids32
+        n_all = world * n
         srows = torch.empty(n_all, dtype=torch.int32, device=dev)
         sslots = torch.empty(n_all, dtype=torch.int32, device=dev)
-        n_local = shard_rows(n_rows, world, rank)
-        ws2_bytes = lib.rlctr_sort_ws_bytes(n_all, max(n_local, 1))
-        ws2 = torch.empty(ws2_bytes, dtype=torch.uint8, device=dev)
-        _lib.call("rlctr_sort_routed", lib.rlctr_sort_routed, _lib.ptr(rb["keys"].local), _lib.ptr(rb["vals"].local), n_all,
-                  max(n_local, 1), _lib.ptr(srows), _lib.ptr(sslots), _lib.ptr(ws2), ws2_bytes, st, key="rlctr_sort_ids",
-                  meta={"n": n_all})
+        ws_bytes = lib.rlctr_sort_ws_bytes(n_all, n_rows)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        _lib.call("rlctr_sort_ids_sharded", lib.rlctr_sort_ids_sharded, _lib.ptr(all32), n_all, world, rank, n_rows,
+                  _lib.ptr(srows), _lib.ptr(sslots), _lib.ptr(ws), ws_bytes, st, key="rlctr_sort_ids", meta={"n": n_all})
         view = (srows, sslots, n_all)
-        _VIEW_CACHE.update(key=key, x=x, view=view)
-        return view
-    ids32 = x.reshape(-1).clamp(-1, n_rows).to(torch.int32)          # out-of-range ids stay out of range in 32 bits
-    if world > 1:
-        all32 = torch.empty(world * n, dtype=torch.int32, device=dev)
-        dist.all_gather_into_tensor(all32, ids32, group=group)
-    else:
-        all32 = ids32
-    n_all = world * n
-    srows = torch.empty(n_all, dtype=torch.int32, device=dev)
-    sslots = torch.empty(n_all, dtype=torch.int32, device=dev)
-    ws_bytes = lib.rlctr_sort_ws_bytes(n_all, n_rows)
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-    _lib.call("rlctr_sort_ids_sharded", lib.rlctr_sort_ids_sharded, _lib.ptr(all32), n_all, world, rank, n_rows, _lib.ptr(srows),
-              _lib.ptr(sslots), _lib.ptr(ws), ws_bytes, st, key="rlctr_sort_ids", meta={"n": n_all})
-    view = (srows, sslots, n_all)
     _VIEW_CACHE.update(key=key, x=x, view=view)
     return view
+
+
+def routed_view_pos(x, n_rows, group):
+    """The routed sorted view with RECEIVE POSITIONS as values (rlctr_sort_routed_pos), plus what the routed gradient push needs:
+    {"rows", "pos", "n_all", "cap", "route_ws" (bucket order of this rank's ids), "slot_of" (global slot at every receive position)}."""
+    lib = _lib.load()
+    r = _route(x, n_rows, group)
+    _lib.call("rlctr_sort_routed_pos", lib.rlctr_sort_routed_pos, _lib.ptr(r["keys"]), r["n_all"], r["n_local"], _lib.ptr(r["rows"]),
+              _lib.ptr(r["out"]), _lib.ptr(r["ws"]), r["ws_bytes"], _lib.stream(), key="rlctr_sort_ids", meta={"n": r["n_all"]})
+    return dict(r, pos=r["out"])
 
 
 def _dense_member(kind, field_nums, latent_dims, device):
@@ -214,138 +240,69 @@ def _copy_dense(dst, src):
 
 
 # ---------------------------------------------------------------------------------------------------
-class ShardedCTR(nn.Module):
-    """LR / FM / FFM / DeepFM, and the tail models WideAndDeep / FNN / InnerPNN / OuterPNN / DCN / AFM, with the table row-sharded
-    over the process group.  A tail model keeps its stand-alone row (16 floats, with or without the first-order column); its dense
-    part is the p_model module itself (``dense``: bias, tower, cross network or attention, and its ``_tail``).
+class _ShardedTable(nn.Module):
+    """What ShardedCTR and ShardedGroup share: the process group, this rank's shard of the table in symmetric memory (the
+    ``table`` Parameter, which optim.Adam hands back to this module), the device barrier, the table structs the kernels see, the
+    lazy-Adam catch-up of the owned rows and the all-reduce of the dense gradients.  Every rank must call the same methods in the
+    same order (they contain device barriers)."""
 
-    ``train_step(features, labels, optimizer)`` is the reference loop body (src/main/pretrain_main.py:96-102) for
-    the local batch; ``forward(features)`` is the frozen scoring pass.  ``from_model`` shards an existing
-    single-GPU model (for the 1-vs-G equivalence check); ``gather_table`` rebuilds the full fused table on every
-    rank.  Every rank must call the same methods in the same order (they contain device barriers)."""
-
-    def __init__(self, kind, feature_nums, field_nums, latent_dims, group=None, device=None):
+    def __init__(self, feature_nums, group, device):
         super().__init__()
-        kind = _ALIASES.get(kind, kind)
-        if kind not in ("LR", "FM", "FFM", "DeepFM") + TAIL_KINDS:
-            raise _lib.RlctrError(f"ShardedCTR: unknown model {kind!r} (LR, FM, FFM, DeepFM, {', '.join(TAIL_KINDS)})")
-        self.kind, self.feature_nums, self.field_nums, self.latent_dims = kind, int(feature_nums), int(field_nums), int(latent_dims)
-        self.group = group
+        self.feature_nums, self.group = int(feature_nums), group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         if self.world not in (1, 2, 4, 8):
             raise _lib.RlctrError("row sharding supports 1, 2, 4 or 8 GPUs (owner = id & (G-1))")
-        n_local = max(shard_rows(self.feature_nums, self.world, self.rank), 1)
-        n_alloc = max(shard_rows(self.feature_nums, self.world, 0), 1)           # same allocation size on every rank
-        if kind == "LR":
-            g = Geometry.lr(n_local)
-        elif kind == "FFM":
-            g = Geometry.ffm(n_local, self.field_nums, self.latent_dims)
-        else:
-            g = Geometry.fm(n_local, self.latent_dims, with_linear=kind not in ("FNN", "InnerPNN", "OuterPNN", "DCN"))
-        g = g.with_state()
-        self._geom = g
-        self._kind = {"LR": "lr", "FFM": "ffm"}.get(kind, "fm")
-        self._fm_term = kind in ("FM", "DeepFM")
-        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        self._pm = PeerMemory(n_alloc * g.row_pitch, torch.float32, dev, group)
-        data = self._pm.local.view(n_alloc, g.row_pitch)
-        data.zero_()
-        used = [g.lin_col] if g.lin_col >= 0 else []
-        used += list(range(g.emb_col, g.emb_col + g.dim))
-        if used:
-            data[:g.n_rows, used] = torch.randn(g.n_rows, len(used), device=dev)
-        self.table = nn.Parameter(data)
-        self.table._rlctr_owner = self
-        self.dense = None
-        if kind in TAIL_KINDS:
-            self.dense = _dense_member(kind, self.field_nums, self.latent_dims, dev)
-            _rehome(self.dense, self, g)
-            self.bias = getattr(self.dense, "bias", None)         # W&D, AFM: the member's own bias; FNN, PNN, DCN: none
-        else:
-            self.bias = nn.Parameter(torch.zeros(1, device=dev))
-        self.mlp = Model._tower(self.field_nums * self.latent_dims, dev) if kind == "DeepFM" else None
-        self._opt = None
-        self._stash = None
-        self._ws = {}
-        self._gbuf = {}
-        self._xbuf = {}
-        # how the owners get the gradient side of remote samples: "push" = replicate the per-sample rows (dlogit / column sums)
-        # with one all_gather and let the source ranks WRITE the per-occurrence rows (DeepFM's tower-input gradients) into the
-        # owners' memory, so that the update kernel reads local memory only; "pull" = the owners read everything through the peer
-        # mapping inside the update kernel (2-3 us NVLink round trips on its dependent path; kept for comparison and for FFM's
-        # 600-byte partner rows)
-        self.exchange = os.environ.get("RLCTR_SHARD_EXCHANGE", "push")
+        self._n_local = max(shard_rows(self.feature_nums, self.world, self.rank), 1)
+        self._dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        self._opt, self._stash, self._ws = None, None, {}
         # True when `group` is used by this model alone: its step may then run as a parallel branch of a captured graph
         # (graphs.GraphedTrainStep), overlapping its NVLink-bound gathers with another model's GEMMs
         self.fork_ok = False
-        self._after_gather = None
 
-    # ---- protocol shared with optim.Adam --------------------------------------------------------
+    def _alloc_table(self, col_groups):
+        """The shard [n_alloc, row_pitch] (the same allocation on every rank) as the ``table`` Parameter: zeros, and N(0, 1) in
+        every list of columns of ``col_groups`` (one draw per list) over the owned rows."""
+        n_alloc, pitch = max(shard_rows(self.feature_nums, self.world, 0), 1), self._geom.row_pitch
+        self._pm = PeerMemory(n_alloc * pitch, torch.float32, self._dev, self.group)
+        data = self._pm.local.view(n_alloc, pitch)
+        data.zero_()
+        for cols in col_groups:
+            data[:self._n_local, cols] = torch.randn(self._n_local, len(cols), device=self._dev)
+        self.table = nn.Parameter(data)
+        self.table._rlctr_owner = self
+
+    def _copy_shard(self, full):
+        """This rank's rows (ids rank, rank + G, ...) of a single-GPU table [N, row_pitch] into the shard."""
+        with torch.no_grad():
+            shard = full[self.rank::self.world]
+            self.table.data[:shard.shape[0]].copy_(shard)
+
+    # ---- protocol shared with optim.Adam / graphs ----------------------------------------------------------------------
     def _apply(self, fn, recurse=True):
-        # the shard lives in symmetric memory: .to()/.cuda() must not move it
-        saved = self._parameters.pop("table")
+        saved = self._parameters.pop("table")            # the shard lives in symmetric memory: .to()/.cuda() must not move it
         out = super()._apply(fn, recurse)
         self._parameters["table"] = saved
         self.table._rlctr_owner = self
         return out
-
-    def _meta(self, B, F):
-        g = self._geom
-        return {"model": "Sharded" + self.kind, "B": B, "F": max(F, 1), "rs": g.row_stride, "dim": g.dim, "n_rows": g.n_rows,
-                "lin": g.lin_col >= 0}
 
     def flush(self):
         if self._opt is not None:
             self._opt.flush(self.table.data)
         check_route_overflow()
 
-    def _reduce_ws(self, dev):
-        ws = self._ws.get("reduce")
-        if ws is None:
-            ws = torch.zeros(_lib.RLCTR_REDUCE_WS_BYTES, dtype=torch.uint8, device=dev)
-            self._ws["reduce"] = ws
-        return ws
-
     def zero_grad(self, set_to_none=True):
         self._stash = None
         return super().zero_grad(set_to_none)
 
-    _rows_ws = Model._TableModel._rows_ws
-
     def barrier(self):
         self._pm.barrier()
 
-    @property
-    def _has_tail(self):
-        return self.mlp is not None or self.dense is not None
-
-    def _tail(self, z, rows):
-        """Logit [B, 1] from the table part z [B, 1] and the gathered rows [B, F*D]: the stand-alone model's ``_tail``."""
-        if self.dense is not None:
-            return self.dense._tail(z, rows)
-        return z + self.mlp(rows)                             # DeepFM
-
-    @classmethod
-    def from_model(cls, model, group=None):
-        """Shard a single-GPU p_model instance (same parameters on every rank) over the group."""
-        kind = type(model).__name__
-        self = cls(kind, model.feature_nums, getattr(model, "field_nums", 15), getattr(model, "latent_dims", 1),
-                   group=group, device=model.table.device)
-        with torch.no_grad():
-            shard = model.table.data[self.rank::self.world]
-            self.table.data[:shard.shape[0]].copy_(shard)
-            if self.dense is not None:
-                _copy_dense(self.dense, model)               # bias (W&D, AFM), towers, cross network, attention, dropout counters
-            else:
-                self.bias.data.copy_(model.bias.data)
-            if self.mlp is not None:
-                self.mlp.load_state_dict(model.mlp.state_dict())
-        self.barrier()
-        return self
+    _reduce_ws = Model._TableModel._reduce_ws
+    _rows_ws = Model._TableModel._rows_ws
 
     def gather_table(self):
-        """The full fused table [N, row_pitch], rebuilt on every rank (tests / checkpointing)."""
+        """The full table [N, row_pitch], rebuilt on every rank (tests / checkpointing)."""
         self.flush()
         mine = self.table.data.contiguous()
         if self.world == 1:
@@ -354,11 +311,9 @@ class ShardedCTR(nn.Module):
         dist.all_gather(parts, mine, group=self.group)
         full = torch.empty(self.feature_nums, self._geom.row_pitch, dtype=torch.float32, device=mine.device)
         for r in range(self.world):
-            cnt = shard_rows(self.feature_nums, self.world, r)
-            full[r::self.world] = parts[r][:cnt]
+            full[r::self.world] = parts[r][:shard_rows(self.feature_nums, self.world, r)]
         return full
 
-    # ---- table structs ----------------------------------------------------------------------------
     def _local_struct(self):
         """The shard as the optimizer kernels see it: n_local rows, local row ids."""
         return table_struct(self.table.data, self._geom)
@@ -373,9 +328,105 @@ class ShardedCTR(nn.Module):
                 t.peers[r] = p
         return t
 
+    # ---- pieces of the step -------------------------------------------------------------------------------------------
+    def _catchup(self, srows, n_all, F, key):
+        """Lazy Adam: bring the owned rows of the sorted view up to date before any rank reads them."""
+        opt = self._opt
+        if opt is not None and opt.lazy and opt.dirty:
+            lib = _lib.load()
+            t, a = self._local_struct(), opt.struct()
+            _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(srows), n_all, C.byref(t), C.byref(a), _lib.stream(),
+                      key=key, meta=self._meta(n_all // F, F))
+
+    def _allreduce_dense(self):
+        """Sum every dense gradient over the ranks: one all_reduce of them all, flattened."""
+        dense = [p for p in self.parameters() if p is not self.table and p.grad is not None]
+        flat = torch.cat([p.grad.reshape(-1) for p in dense])
+        dist.all_reduce(flat, group=self.group)
+        o = 0
+        for p in dense:
+            p.grad = flat[o:o + p.numel()].view_as(p).clone()
+            o += p.numel()
+
+
+class ShardedCTR(_ShardedTable):
+    """LR / FM / FFM / DeepFM, and the tail models WideAndDeep / FNN / InnerPNN / OuterPNN / DCN / AFM, with the table row-sharded
+    over the process group.  A tail model keeps its stand-alone row (16 floats, with or without the first-order column); its dense
+    part is the p_model module itself (``dense``: bias, tower, cross network or attention, and its ``_tail``).
+
+    ``train_step(features, labels, optimizer)`` is the reference loop body (src/main/pretrain_main.py:96-102) for
+    the local batch; ``forward(features)`` is the frozen scoring pass.  ``from_model`` shards an existing
+    single-GPU model (for the 1-vs-G equivalence check); ``gather_table`` rebuilds the full fused table on every
+    rank.  Every rank must call the same methods in the same order (they contain device barriers).
+
+    The owners get the gradient side of remote samples by PUSH: the per-sample rows (dlogit, or the sums rows that carry it)
+    are replicated with one all_gather, and the source ranks WRITE the per-occurrence rows (the tower-input gradients) into the
+    owners' memory, so the update reads local memory only -- but for FFM's 600-byte partner rows, which it reads on the source
+    rank through the peer mapping."""
+
+    def __init__(self, kind, feature_nums, field_nums, latent_dims, group=None, device=None):
+        kind = _ALIASES.get(kind, kind)
+        if kind not in ("LR", "FM", "FFM", "DeepFM") + TAIL_KINDS:
+            raise _lib.RlctrError(f"ShardedCTR: unknown model {kind!r} (LR, FM, FFM, DeepFM, {', '.join(TAIL_KINDS)})")
+        super().__init__(feature_nums, group, device)
+        self.kind, self.field_nums, self.latent_dims = kind, int(field_nums), int(latent_dims)
+        if kind == "LR":
+            g = Geometry.lr(self._n_local)
+        elif kind == "FFM":
+            g = Geometry.ffm(self._n_local, self.field_nums, self.latent_dims)
+        else:
+            g = Geometry.fm(self._n_local, self.latent_dims, with_linear=kind not in ("FNN", "InnerPNN", "OuterPNN", "DCN"))
+        self._geom = g = g.with_state()
+        self._kind = {"LR": "lr", "FFM": "ffm"}.get(kind, "fm")
+        self._fm_term = kind in ("FM", "DeepFM")
+        self._alloc_table([([g.lin_col] if g.lin_col >= 0 else []) + list(range(g.emb_col, g.emb_col + g.dim))])
+        self.dense = None
+        if kind in TAIL_KINDS:
+            self.dense = _dense_member(kind, self.field_nums, self.latent_dims, self._dev)
+            _rehome(self.dense, self, g)
+            self.bias = getattr(self.dense, "bias", None)         # W&D, AFM: the member's own bias; FNN, PNN, DCN: none
+        else:
+            self.bias = nn.Parameter(torch.zeros(1, device=self._dev))
+        self.mlp = Model._tower(self.field_nums * self.latent_dims, self._dev) if kind == "DeepFM" else None
+        self._gbuf, self._xbuf = {}, {}
+        self._after_gather = None
+
+    def _meta(self, B, F):
+        g = self._geom
+        return {"model": "Sharded" + self.kind, "B": B, "F": max(F, 1), "rs": g.row_stride, "dim": g.dim, "n_rows": g.n_rows,
+                "lin": g.lin_col >= 0}
+
+    @property
+    def _has_tail(self):
+        return self.mlp is not None or self.dense is not None
+
+    def _tail(self, z, rows):
+        """Logit [B, 1] from the table part z [B, 1] and the gathered rows [B, F*D]: the stand-alone model's ``_tail``."""
+        if self.dense is not None:
+            return self.dense._tail(z, rows)
+        return z + self.mlp(rows)                             # DeepFM
+
+    @classmethod
+    def from_model(cls, model, group=None):
+        """Shard a single-GPU p_model instance (same parameters on every rank) over the group: its table, its dense parameters,
+        and the dropout counters and train / eval flags of its tower, cross network or attention."""
+        kind = type(model).__name__
+        self = cls(kind, model.feature_nums, getattr(model, "field_nums", 15), getattr(model, "latent_dims", 1),
+                   group=group, device=model.table.device)
+        self._copy_shard(model.table.data)
+        if self.dense is not None:
+            _copy_dense(self.dense, model)                   # bias (W&D, AFM), towers, cross network, attention
+        else:
+            with torch.no_grad():
+                self.bias.data.copy_(model.bias.data)
+            if self.mlp is not None:
+                _copy_dense(self.mlp, model.mlp)             # DeepFM's tower
+        self.barrier()
+        return self
+
     def _grad_buffers(self, B, F):
-        """dlogit [B] | sums [B, rs] | extra [B, F*D] | staged [B*F, rs] in ONE symmetric allocation per batch size:
-        what the owners of this rank's rows pull after the backward."""
+        """dlogit [B] | sums [B, rs] | extra [B, F*D] | staged [B*F, rs] in ONE symmetric allocation per batch size: this rank's
+        gradient side of the step (the owners read the staged FFM partner rows in place, through ``staged_ptrs``)."""
         buf = self._gbuf.get(B)
         if buf is not None:
             return buf
@@ -398,8 +449,8 @@ class ShardedCTR(nn.Module):
         return buf
 
     def _exchange_buffers(self, B, F):
-        """Receive side of the "push" exchange for batch size B: the all-gathered per-sample rows of every rank (plain local
-        tensors) and the symmetric buffer the sources write the per-occurrence tail gradients into."""
+        """Receive side of the push for batch size B: the all-gathered per-sample rows of every rank (plain local tensors) and
+        the symmetric buffer the sources write the per-occurrence tail gradients into."""
         xb = self._xbuf.get(B)
         if xb is not None:
             return xb
@@ -464,77 +515,42 @@ class ShardedCTR(nn.Module):
         lib = _lib.load()
         x = Model._check_ids(features)
         B, F = x.shape
-        dev = x.device
-        st = _lib.stream()
-        y = labels.reshape(-1).contiguous()
+        G, st = self.world, _lib.stream()
+        y = _co.labels(labels)
         buf = self._grad_buffers(B, F)
         srows, sslots, n_all = shared_sorted_view(x, self.feature_nums, self.group)
-        opt = self._opt
-        if opt is not None and opt.lazy and opt.dirty:
-            t, a = self._local_struct(), opt.struct()
-            _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(srows), n_all, C.byref(t), C.byref(a), st,
-                      key=f"rlctr_rows_catchup[Sharded{self.kind}]", meta=self._meta(n_all // F, F))
+        self._catchup(srows, n_all, F, f"rlctr_rows_catchup[Sharded{self.kind}]")
         self.barrier()                                        # B1: all owners caught their rows up | forward reads
         logit, trows = self._interact(x, buf, train=True)
         hook, self._after_gather = self._after_gather, None     # graphs.GraphedTrainStep: fork point of the captured step
         if hook is not None:
             hook()
-        z = None
-        if self._has_tail:
-            trows.requires_grad_(True)
-            with torch.enable_grad():
-                z = self._tail(logit.view(B, 1), trows)
-            logit = z.detach().reshape(-1).contiguous()
-        loss = torch.empty(1, dtype=torch.float32, device=dev)
-        dlogit = buf["dlogit"][:B]
-        dbias = torch.empty(1, dtype=torch.float32, device=dev) if self.bias is not None else None
-        yi = y if y.dtype == torch.int64 else None
-        yf = None if yi is not None else y.float()
-        _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(logit), _lib.ptr(yi), _lib.ptr(yf), None, _lib.ptr(loss), _lib.ptr(dlogit),
-                                         _lib.ptr(dbias), _lib.ptr(self._reduce_ws(dev)), B, st), "rlctr_bce_fwd_bwd")
-        if self.world > 1:                                    # gradient of the GLOBAL mean loss
-            dlogit.mul_(1.0 / self.world)
-            if dbias is not None:
-                dbias.mul_(1.0 / self.world)
-        dz_in_sums = self.world > 1 and self._fm_term
-        if dz_in_sums:                                        # one aligned 64 B line per occurrence for the owners to pull
-            buf["sums"].view(B, -1)[:, -1] = dlogit
+        loss = torch.empty(1, dtype=torch.float32, device=x.device)
         for p in self.parameters():
             p.grad = None
-        if z is not None:
-            z.backward(dlogit.view_as(z))
-            buf["extra"].view(B, -1).copy_(trows.grad)
-        if self.bias is not None:
-            self.bias.grad = dbias
-        if self.world > 1:
-            dense = [p for p in self.parameters() if p is not self.table and p.grad is not None]
-            flat = torch.cat([p.grad.reshape(-1) for p in dense])
-            dist.all_reduce(flat, group=self.group)
-            o = 0
-            for p in dense:
-                p.grad = flat[o:o + p.numel()].view_as(p).clone()
-                o += p.numel()
+        dlogit, grad = _co.loss_head(self, logit, trows, y, loss.data_ptr(), self._reduce_ws(x.device), dl=buf["dlogit"][:B],
+                                     scale=1.0 / G)
+        if grad is not None:
+            buf["extra"].view(B, -1).copy_(grad)
+        dz_in_sums = G > 1 and self._fm_term
+        if dz_in_sums:                                        # one aligned 64 B line per occurrence for the owners to read
+            buf["sums"].view(B, -1)[:, -1] = dlogit
         peer = None
-        if self.world > 1:
-            peer = {"world": self.world, "n_per_rank": B * F, "staged": buf["staged_ptrs"], "dlogit": buf["dlogit_ptrs"],
-                    "sums": buf["sums_ptrs"], "extra": buf["extra_ptrs"]}
-            if self.exchange == "push":
-                xb = self._exchange_buffers(B, F)
-                g = self._geom
-                if dz_in_sums:                                # dlogit rides in the sums rows: one all_gather serves both
-                    dist.all_gather_into_tensor(xb["sums_all"], buf["sums"], group=self.group)
-                    per = 4 * B * g.row_stride
-                    peer["sums"] = [xb["sums_all"].data_ptr() + r * per for r in range(self.world)]
-                    peer["dlogit"] = [xb["dlogit_all"].data_ptr() + r * 4 * xb["bp"] for r in range(self.world)]   # not read
-                else:
-                    dist.all_gather_into_tensor(xb["dlogit_all"], buf["dlogit"], group=self.group)
-                    peer["dlogit"] = [xb["dlogit_all"].data_ptr() + r * 4 * xb["bp"] for r in range(self.world)]
-                if xb["recv"] is not None:                    # per-occurrence rows: posted writes into the owners' memory
-                    n = B * F
-                    _lib.call("rlctr_push_rows", lib.rlctr_push_rows, _lib.ptr(x), n, self.world, self.rank, self.feature_nums,
-                              _lib.ptr(buf["extra"]), g.dim, xb["recv_ptrs"], st, meta={"n": n, "width": g.dim})
-                    mine = xb["recv"].local.data_ptr()
-                    peer["extra"] = [mine + r * 4 * n * g.dim for r in range(self.world)]
+        if G > 1:
+            self._allreduce_dense()
+            xb, g = self._exchange_buffers(B, F), self._geom
+            peer = {"world": G, "n_per_rank": B * F, "staged": buf["staged_ptrs"], "sums": None, "extra": None,
+                    "dlogit": [xb["dlogit_all"].data_ptr() + r * 4 * xb["bp"] for r in range(G)]}    # not read with dz_in_sums
+            if dz_in_sums:                                    # dlogit rides in the sums rows: one all_gather serves both
+                dist.all_gather_into_tensor(xb["sums_all"], buf["sums"], group=self.group)
+                peer["sums"] = [xb["sums_all"].data_ptr() + r * 4 * B * g.row_stride for r in range(G)]
+            else:
+                dist.all_gather_into_tensor(xb["dlogit_all"], buf["dlogit"], group=self.group)
+            if xb["recv"] is not None:                        # per-occurrence rows: posted writes into the owners' memory
+                n = B * F
+                _lib.call("rlctr_push_rows", lib.rlctr_push_rows, _lib.ptr(x), n, G, self.rank, self.feature_nums,
+                          _lib.ptr(buf["extra"]), g.dim, xb["recv_ptrs"], st, meta={"n": n, "width": g.dim})
+                peer["extra"] = [xb["recv"].local.data_ptr() + r * 4 * n * g.dim for r in range(G)]
         self.barrier()                                        # B2: every rank's gradient-side buffers are complete
         self._stash = Model.RowsStash(sorted_ids=srows, sorted_slots=sslots, n=n_all, dlogit=dlogit, sums=buf["sums"],
                                       extra=buf["extra"], staged=buf["staged"], fields=F,
@@ -544,32 +560,8 @@ class ShardedCTR(nn.Module):
         return loss.reshape(())
 
 
-def routed_view_pos(x, n_rows, group):
-    """The routed sorted view with RECEIVE POSITIONS as values (rlctr_sort_routed_pos), plus what the routed gradient push needs:
-    {"rows", "pos", "n_all", "cap", "route_ws" (bucket order of this rank's ids), "slot_of" (global slot at every receive position)}."""
-    lib = _lib.load()
-    world, rank = dist.get_world_size(group), dist.get_rank(group)
-    dev, n, st = x.device, x.numel(), _lib.stream()
-    rb = _route_buffers(n, world, dev, group)
-    cap = rb["cap"]
-    ws_bytes = lib.rlctr_route_ws_bytes(n, world)
-    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-    _lib.call("rlctr_route_ids", lib.rlctr_route_ids, _lib.ptr(x), n, world, rank, n_rows, cap, rb["kp"], rb["vp"],
-              _lib.ptr(rb["overflow"]), _lib.ptr(ws), ws_bytes, st, meta={"n": n, "world": world, "cap": cap})
-    rb["keys"].barrier()                                         # every source's segment of my receive buffer is complete
-    n_all = world * cap
-    srows = torch.empty(n_all, dtype=torch.int32, device=dev)
-    spos = torch.empty(n_all, dtype=torch.int32, device=dev)
-    n_local = max(shard_rows(n_rows, world, rank), 1)
-    ws2_bytes = lib.rlctr_sort_ws_bytes(n_all, n_local)
-    ws2 = torch.empty(ws2_bytes, dtype=torch.uint8, device=dev)
-    _lib.call("rlctr_sort_routed_pos", lib.rlctr_sort_routed_pos, _lib.ptr(rb["keys"].local), n_all, n_local, _lib.ptr(srows),
-              _lib.ptr(spos), _lib.ptr(ws2), ws2_bytes, st, key="rlctr_sort_ids", meta={"n": n_all})
-    return {"rows": srows, "pos": spos, "n_all": n_all, "cap": cap, "route_ws": ws, "slot_of": rb["vals"].local}
-
-
 # ---------------------------------------------------------------------------------------------------
-class ShardedGroup(nn.Module):
+class ShardedGroup(_co._GroupStep, _ShardedTable):
     """Co-located records (colocated.py) over a row-sharded joint table: the members ``colocate()`` accepts (LR, FM, DeepFM,
     WideAndDeep, FNN, InnerPNN, OuterPNN, DCN, AFM) trained on the same id stream share one 384-byte record per id,
     ``owner(id) = id mod G``.  Per step and rank: ONE routed sorted view (shared_sorted_view), one catch-up of the owned records, one
@@ -581,41 +573,26 @@ class ShardedGroup(nn.Module):
     its own: its bias, tower, cross network or attention, and the ``_tail`` the group step runs."""
 
     SUMS_PITCH = 32                    # one 128-byte line per sample: S (<= 28 floats) | dL/dlogit of members 0..3
+    _UPDATE_KEY = "rlctr_group_rows_adam[ShardedGroup]"
 
     def __init__(self, kinds, feature_nums, field_nums, latent_dims, group=None, device=None):
-        super().__init__()
         kinds = tuple(_ALIASES.get(k, k) for k in kinds)
         names = tuple(c.__name__ for c in _co.MEMBER_KINDS)
         if not all(k in names for k in kinds) or not 1 <= len(kinds) <= _lib.RLCTR_GROUP_MAX:
             raise _lib.RlctrError(f"ShardedGroup members: {', '.join(names)} (up to {_lib.RLCTR_GROUP_MAX}); got {', '.join(kinds)}")
-        self.kinds, self.feature_nums, self.field_nums, self.latent_dims = kinds, int(feature_nums), int(field_nums), int(latent_dims)
-        self.group = group
-        self.world = dist.get_world_size(group) if dist.is_initialized() else 1
-        self.rank = dist.get_rank(group) if dist.is_initialized() else 0
-        if self.world not in (1, 2, 4, 8):
-            raise _lib.RlctrError("row sharding supports 1, 2, 4 or 8 GPUs (owner = id & (G-1))")
-        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-        members = [_dense_member(k, self.field_nums, self.latent_dims, dev) for k in kinds]
-        n_local = max(shard_rows(self.feature_nums, self.world, self.rank), 1)
-        n_alloc = max(shard_rows(self.feature_nums, self.world, 0), 1)
+        super().__init__(feature_nums, group, device)
+        self.kinds, self.field_nums, self.latent_dims = kinds, int(field_nums), int(latent_dims)
+        members = [_dense_member(k, self.field_nums, self.latent_dims, self._dev) for k in kinds]
         self._cols, used = _co._layout(members)
         rs = (used + 1 + 3) // 4 * 4
         if rs > self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX:
             raise _lib.RlctrError("joint row too wide for the per-sample exchange row (28 floats)")
-        self._geom = Geometry(n_local, rs, -1, 0, used, pitch=96, block=32, stamp_at=used)
-        self._pm = PeerMemory(n_alloc * 96, torch.float32, dev, group)
-        data = self._pm.local.view(n_alloc, 96)
-        data.zero_()
-        for lin, emb, dim in self._cols:
-            cols = ([lin] if lin >= 0 else []) + list(range(emb, emb + dim))
-            data[:n_local, cols] = torch.randn(n_local, len(cols), device=dev)
-        self.table = nn.Parameter(data)
-        self.table._rlctr_owner = self
+        self._geom = Geometry(self._n_local, rs, -1, 0, used, pitch=96, block=32, stamp_at=used)
+        self._alloc_table([([lin] if lin >= 0 else []) + list(range(emb, emb + dim)) for lin, emb, dim in self._cols])
         for m, (lin, emb, dim) in zip(members, self._cols):
-            _rehome(m, self, Geometry(n_local, rs, lin, emb, dim, pitch=96, block=32))
+            _rehome(m, self, Geometry(self._n_local, rs, lin, emb, dim, pitch=96, block=32))
         self.members = nn.ModuleList(members)
-        self._opt, self._stash, self._ws, self._buf = None, None, {}, {}
-        self.fork_ok = False
+        self._buf = {}
 
     @property
     def biases(self):
@@ -627,35 +604,10 @@ class ShardedGroup(nn.Module):
         """The members' towers (``mlp``; nn.Identity for a member without one)."""
         return [m.mlp if getattr(m, "mlp", None) is not None else nn.Identity() for m in self.members]
 
-    # ---- protocol shared with optim.Adam / graphs ----------------------------------------------------------------------
-    def _apply(self, fn, recurse=True):
-        saved = self._parameters.pop("table")            # the shard lives in symmetric memory: .to() must not move it
-        out = super()._apply(fn, recurse)
-        self._parameters["table"] = saved
-        self.table._rlctr_owner = self
-        return out
-
     def _meta(self, B, F):
         g = self._geom
         return {"model": "Sharded" + "+".join(self.kinds), "B": B, "F": max(F, 1), "rs": g.row_stride, "dim": g.dim,
                 "n_rows": g.n_rows, "lin": False, "members": [(k, c[2]) for k, c in zip(self.kinds, self._cols)]}
-
-    def flush(self):
-        if self._opt is not None:
-            self._opt.flush(self.table.data)
-        check_route_overflow()
-
-    _reduce_ws = ShardedCTR._reduce_ws
-    _rows_ws = Model._TableModel._rows_ws
-    _member_structs = _co.ColocatedCTR._member_structs
-    _z = staticmethod(_co.ColocatedCTR._z)
-
-    def zero_grad(self, set_to_none=True):
-        self._stash = None
-        return super().zero_grad(set_to_none)
-
-    def barrier(self):
-        self._pm.barrier()
 
     @classmethod
     def from_group(cls, cg, group=None):
@@ -667,35 +619,11 @@ class ShardedGroup(nn.Module):
                    group=group, device=cg.table.device)
         assert self._cols == cg._cols
         cg.flush()
-        with torch.no_grad():
-            shard = cg.table.data[self.rank::self.world]
-            self.table.data[:shard.shape[0]].copy_(shard)
+        self._copy_shard(cg.table.data)
         for dst, src in zip(self.members, cg.members):
             _copy_dense(dst, src)
         self.barrier()
         return self
-
-    def gather_table(self):
-        """The full joint table [N, 96], rebuilt on every rank (tests / checkpointing)."""
-        self.flush()
-        mine = self.table.data.contiguous()
-        if self.world == 1:
-            return mine[:self.feature_nums].clone()
-        parts = [torch.empty_like(mine) for _ in range(self.world)]
-        dist.all_gather(parts, mine, group=self.group)
-        full = torch.empty(self.feature_nums, 96, dtype=torch.float32, device=mine.device)
-        for r in range(self.world):
-            full[r::self.world] = parts[r][:shard_rows(self.feature_nums, self.world, r)]
-        return full
-
-    def _global_struct(self):
-        g = self._geom
-        t = _lib.Table(self.table.data.data_ptr(), self.feature_nums, g.row_stride, g.lin_col, g.emb_col, g.dim, g.row_pitch)
-        if self.world > 1:
-            t.world = self.world
-            for r, p in enumerate(self._pm.ptrs):
-                t.peers[r] = p
-        return t
 
     def _tail_sources(self):
         """[(member, float offset in the interleaved receive row, width)] of the members with a dense tail, and the row's pitch:
@@ -732,34 +660,22 @@ class ShardedGroup(nn.Module):
     @torch.no_grad()
     def forward(self, x):
         """pCTR of every member, float32 [B, M] (as colocated.ColocatedCTR.forward, the rows read through the peer mapping)."""
-        lib = _lib.load()
         x = Model._check_ids(x)
-        B, F = x.shape
         self.flush()
-        self.barrier()
-        out = torch.empty(B, len(self.members), dtype=torch.float32, device=x.device)
-        arr, logits, rows = self._member_structs(B, F, x.device, False, pctr=out)
-        t = self._global_struct()
-        _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, len(self.members), None, 0, B, F,
-                  _lib.stream(), key="rlctr_group_fwd[sharded infer]", meta=self._meta(B, F))
-        for i, m in enumerate(self.members):
-            if rows[i] is not None:
-                out[:, i:i + 1] = torch.sigmoid(m._tail(self._z(logits[i], B), rows[i][:, :F * self._cols[i][2]]))
-        self.barrier()
+        self.barrier()                                        # every shard is settled before anyone reads it
+        out = self._pctr(x, "rlctr_group_fwd[sharded infer]")
+        self.barrier()                                        # nobody starts writing rows while a peer still reads
         return out
 
     def train_step(self, features, labels, optimizer):
         """One step of every member on the local batch; returns the local mean BCE losses, float32 [M]."""
         lib = _lib.load()
-        opt = self._opt
-        if opt is None:
+        if self._opt is None:
             raise _lib.RlctrError("build rl_ctr_prediction_b200.optim.Adam(group.parameters(), ...) before training the group")
         x = Model._check_ids(features)
         B, F = x.shape
-        dev, st, G, M = x.device, _lib.stream(), self.world, len(self.kinds)
-        y = labels.reshape(-1).contiguous()
-        yi = y if y.dtype == torch.int64 else None
-        yf = None if yi is not None else y.float()
+        st, G, M = _lib.stream(), self.world, len(self.members)
+        y = _co.labels(labels)
         buf = self._exchange(B, F)
         view = None
         if G > 1:                                             # routed exchange: positions in the owner's receive buffers
@@ -767,55 +683,22 @@ class ShardedGroup(nn.Module):
             srows, sslots, n_all = view["rows"], view["pos"], view["n_all"]
         else:
             srows, sslots, n_all = shared_sorted_view(x, self.feature_nums, self.group)
-        if opt.lazy and opt.dirty:
-            t, a = table_struct(self.table.data, self._geom), opt.struct()
-            _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(srows), n_all, C.byref(t), C.byref(a), st,
-                      key="rlctr_rows_catchup[ShardedGroup]", meta=self._meta(n_all // F, F))
+        self._catchup(srows, n_all, F, "rlctr_rows_catchup[ShardedGroup]")
         self.barrier()                                        # B1: all owners caught their rows up | forward reads
-        arr, logits, rows = self._member_structs(B, F, dev, True)
+        arr, logits, rows = self._member_structs(B, F, x.device, True)
         t = self._global_struct()
         sums = buf["sums"]
         _lib.call("rlctr_group_fwd", lib.rlctr_group_fwd, _lib.ptr(x), C.byref(t), arr, M, _lib.ptr(sums), self.SUMS_PITCH, B, F, st,
                   key="rlctr_group_fwd[ShardedGroup]", meta=dict(self._meta(B, F), n_rows=self.feature_nums))
-        losses = torch.empty(M, dtype=torch.float32, device=dev)
-        ws = self._reduce_ws(dev)
-        for p in self.parameters():
-            p.grad = None
-        extras, pitches = [None] * M, [0] * M
-        for i, m in enumerate(self.members):
-            dl = torch.empty(B, dtype=torch.float32, device=dev)
-            bias = getattr(m, "bias", None)
-            dbias = torch.empty(1, dtype=torch.float32, device=dev) if bias is not None else None
-            z = leaf = None
-            if rows[i] is None:                               # LR, FM: the table logit is the logit
-                zz = logits[i]
-            else:                                             # dense tail: the member's own _tail, autograd over it only
-                leaf = rows[i][:, :F * self._cols[i][2]].detach().requires_grad_(True)
-                z = m._tail(self._z(logits[i], B), leaf)
-                zz = z.detach().reshape(-1).contiguous()
-            _lib.check(lib.rlctr_bce_fwd_bwd(_lib.ptr(zz), _lib.ptr(yi), _lib.ptr(yf), None, losses.data_ptr() + 4 * i, _lib.ptr(dl),
-                                             _lib.ptr(dbias), _lib.ptr(ws), B, st), "rlctr_bce_fwd_bwd")
-            if G > 1:                                         # gradient of the GLOBAL mean loss
-                dl.mul_(1.0 / G)
-                if dbias is not None:
-                    dbias.mul_(1.0 / G)
+        losses, dlogits, extras = self._heads(F, logits, rows, y, scale=1.0 / G)
+        for i, dl in enumerate(dlogits):
             if self._uses_dz(i):
                 sums[:, self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX + i] = dl    # dL/dlogit rides in the sample's exchange row
-            if z is not None:
-                z.backward(dl.view_as(z))
-                extras[i] = leaf.grad.contiguous()
-            if bias is not None:
-                bias.grad = dbias
+        pitches = [0] * M
         if G > 1:
-            dense = [p for p in self.parameters() if p is not self.table and p.grad is not None]
-            flat = torch.cat([p.grad.reshape(-1) for p in dense])
-            dist.all_reduce(flat, group=self.group)
-            o = 0
-            for p in dense:
-                p.grad = flat[o:o + p.numel()].view_as(p).clone()
-                o += p.numel()
+            self._allreduce_dense()
             dist.all_gather_into_tensor(buf["sums_all"], sums, group=self.group)
-            sums_all = buf["sums_all"]
+            sums = buf["sums_all"]
             if buf["recv"] is not None:                       # ONE push of every tail member's per-occurrence rows, in the routed
                 pm, ptrs = buf["recv"]                        # bucket order: interleaved rows, coalesced posted writes
                 n = B * F
@@ -833,28 +716,9 @@ class ShardedGroup(nn.Module):
                           meta={"n": n, "width": pitch, "sources": len(keep)})
                 for i, off, _ in tails:
                     extras[i], pitches[i] = pm.local[off:], pitch
-        else:
-            sums_all = sums
         self.barrier()                                        # B2: every rank's gradient-side buffers are complete
-        self._stash = {"sorted_ids": srows, "sorted_slots": sslots, "n": n_all, "fields": F, "sums": sums_all, "extra": extras,
-                       "extra_pitch": pitches, "slot_of": view["slot_of"] if view is not None else None}
+        self._stash = _co.GroupStash(sorted_ids=srows, sorted_slots=sslots, n=n_all, fields=F, sums=sums, dlogit=[None] * M,
+                                     extra=extras, sums_pitch=self.SUMS_PITCH, world=G, extra_pitch=pitches,
+                                     slot_of=view["slot_of"] if view is not None else None)
         optimizer.step()
         return losses
-
-    def _group_update(self, stash, opt_state, st):
-        lib = _lib.load()
-        arr = (_lib.Member * len(self.kinds))()
-        for i, (m, (lin, emb, dim)) in enumerate(zip(self.members, self._cols)):
-            s = arr[i]
-            s.lin_col, s.emb_col, s.dim = lin, emb, dim
-            s.flags = _lib.RLCTR_FM_TERM if m._fm_term else 0
-            s.dlogit = None                                   # in the exchange rows
-            s.extra = _lib.ptr(stash["extra"][i])
-            s.extra_pitch = stash["extra_pitch"][i]
-        t, a = table_struct(self.table.data, self._geom), opt_state.struct()
-        n, F = stash["n"], stash["fields"]
-        ws_bytes = lib.rlctr_rows_ws_bytes(n)
-        ws = self._rows_ws(ws_bytes)
-        _lib.call("rlctr_group_rows_adam", lib.rlctr_group_rows_adam, _lib.ptr(stash["sorted_ids"]), _lib.ptr(stash["sorted_slots"]),
-                  n, C.byref(t), C.byref(a), arr, len(self.kinds), _lib.ptr(stash["sums"]), self.SUMS_PITCH, F, self.world,
-                  _lib.ptr(stash["slot_of"]), _lib.ptr(ws), ws_bytes, st, key="rlctr_group_rows_adam[ShardedGroup]", meta=self._meta(n // F, F))

@@ -401,3 +401,28 @@ def test_sharded_refusals(one_rank):
     sg = sharded.ShardedGroup.from_group(cg)
     assert [type(m).__name__ for m in sg.members] == ["AFM", "LR", "DCN"]
     assert sg.biases[2] is None and isinstance(sg.mlps[0], torch.nn.Identity)
+
+
+# ---- 7. ShardedCTR.from_model carries DeepFM's dropout state -----------------------------------------------------------------------
+def test_sharded_deepfm_from_model_copies_tower_dropout_state(one_rank):
+    """A DeepFM whose tower is in train() and has already drawn masks (one Dropout switched to eval): the sharded copy has the
+    tower's dropout counter and train / eval flags, so its first step draws the same masks and takes the same loss."""
+    from rl_ctr_prediction_b200 import graphs, optim, pretrain_main as PM, sharded
+    N, B = 3001, 256
+    torch.manual_seed(12)
+    single = PM.get_model("DeepFM", N, F, D).to(DEV).train()
+    single.mlp[5].eval()
+    (x0, _), (x, y) = _batches(N, B, 2, seed=13)
+    with torch.no_grad():
+        single(x0)                                         # the tower draws masks: its counter moves off zero
+    assert int(single.mlp._rlctr_rng[1]) > 0
+    m = sharded.ShardedCTR.from_model(single)
+    assert torch.equal(m.mlp._rlctr_rng, single.mlp._rlctr_rng)
+    assert [u.training for u in m.mlp.modules()] == [v.training for v in single.mlp.modules()]
+    assert not m.mlp[5].training and m.mlp[2].training
+    opt_s = optim.Adam(single.parameters(), lr=1e-3, weight_decay=1e-5)
+    opt_m = optim.Adam(m.parameters(), lr=1e-3, weight_decay=1e-5)
+    ls = graphs.fused_logit_step(single, opt_s, x, y)
+    lm = m.train_step(x, y, opt_m)
+    assert torch.equal(ls, lm)
+    assert torch.equal(m.mlp._rlctr_rng, single.mlp._rlctr_rng)
