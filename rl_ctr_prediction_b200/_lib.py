@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_PKG, "librlctr_sm100a.so")
 RLCTR_FM_TERM = 1
 RLCTR_STAGED_PARTNER = 1
 RLCTR_DZ_IN_SUMS = 2
+RLCTR_EUNSUPPORTED = -2
 RLCTR_REDUCE_WS_BYTES = 16640
 RLCTR_DENSE_MAX = 24
 RLCTR_MLP_RELU = 1
@@ -163,10 +164,22 @@ def load() -> C.CDLL:
     return lib
 
 
+# the shape limits behind RLCTR_EUNSUPPORTED of the entry points the latent size reaches (F = 15: D <= 32 for every model)
+SHAPE_LIMITS = {
+    "rlctr_embed_fwd": "fused rows of at most 36 floats (D <= 32 with a first-order column, 36 without)",
+    "rlctr_afm_fwd": "AFM: D <= 32, F <= 23",
+    "rlctr_afm_bwd": "AFM: D <= 32, F <= 23",
+    "rlctr_cross_fwd": "DCN: F*D <= 512, at most 8 cross layers",
+    "rlctr_cross_bwd": "DCN: F*D <= 512, at most 6 cross layers",
+    "rlctr_rows_adam": "fused rows of at most 512 floats (FFM: F*D + 1 <= 512)",
+}
+
+
 def check(code: int, what: str) -> None:
     if code != 0:
         msg = load().rlctr_strerror(code).decode()
-        raise RlctrError(f"{what} failed: {msg} (code {code})")
+        limit = SHAPE_LIMITS.get(what.split("[")[0]) if code == RLCTR_EUNSUPPORTED else None
+        raise RlctrError(f"{what} failed: {msg} (code {code})" + (f"; supported: {limit}" if limit else ""))
 
 
 def ptr(t):

@@ -105,6 +105,17 @@ __device__ __forceinline__ float afm_scores(const float* __restrict__ stage, con
     return afm_warp_sum(sum);
 }
 
+__device__ __forceinline__ void afm_pair_tables(unsigned char* pi, unsigned char* pj, unsigned char* pidx, int fields) {
+    for (int i = threadIdx.x; i < fields; i += blockDim.x) {
+        const int base = i * fields - i * (i + 1) / 2;
+        for (int j = i + 1; j < fields; ++j) {
+            const int p = base + j - i - 1;
+            pi[p] = (unsigned char)i; pj[p] = (unsigned char)j;
+            if (pidx) { pidx[i * fields + j] = (unsigned char)p; pidx[j * fields + i] = (unsigned char)p; }
+        }
+    }
+}
+
 // dynamic smem: PAR floats | AFM_WARPS * (fd + npair_pad) floats | 2 * npair bytes
 template <int D>
 __global__ void __launch_bounds__(AFM_WARPS * 32)
@@ -189,15 +200,9 @@ afm_bwd_kernel(const float* __restrict__ rows, int64_t ld_rows, const float* __r
     unsigned char* pj = pi + npair;
     unsigned char* pidx = pj + npair;
     static_assert(PAR % 4 == 0, "the per-warp arrays follow the parameters at a 16-byte boundary");
+    static_assert(D * CHK <= 32, "one dW_a chunk per lane: D <= 10 (afm_bwd_wide_kernel serves larger D)");
     AfmSmem<D>::load(par, params);
-    for (int i = threadIdx.x; i < fields; i += blockDim.x) {
-        const int base = i * fields - i * (i + 1) / 2;
-        for (int j = i + 1; j < fields; ++j) {
-            const int p = base + j - i - 1;
-            pi[p] = (unsigned char)i; pj[p] = (unsigned char)j;
-            pidx[i * fields + j] = (unsigned char)p; pidx[j * fields + i] = (unsigned char)p;
-        }
-    }
+    afm_pair_tables(pi, pj, pidx, fields);
     __syncthreads();
     uint64_t seed = 0, ctr = 0;
     if (dr.rng && !dr.masks) { seed = dr.rng[0]; ctr = dr.rng[1]; }
@@ -334,6 +339,240 @@ afm_bwd_kernel(const float* __restrict__ rows, int64_t ld_rows, const float* __r
     if (lane == 0) { mine[D * D + 2 * D] = sbs; mine[D * D + 3 * D + 1] = dfcb; }
 }
 
+// D = 11..32.  The per-lane layout above keeps ip_p, the attention output and its gradient as D floats per lane and lets the
+// compiler keep W_a in registers; past D = 10 that spills.  Here every pass that touches the D x D attention weight is turned
+// around: a lane OWNS one output unit k (one input dimension d) and walks all pairs of the sample, reading v_i, v_j, d a_p ... as
+// shared-memory broadcasts.  A lane keeps three D-float vectors (row k and column d of W_a, its row of d W_a) and nothing else
+// of size D:
+//     scores  (lane = k):     a_p[k] = b_a[k] + <W_a[k, :], ip_p>   staged [P, AP];  then lane = pair: s_p = b_s + <w_s, relu(a_p)>
+//     forward (lane = d):     attn_d = sum_p sd_p ip_p[d];  y = fc_b + sum over lanes of fc_w[d] attn_d m2_d
+//     pass A  (lane = k):     d a_p[k], d W_a[k, :] += d a_p[k] ip_p,  d a_p overwrites a_p
+//     pass B  (lane = d):     d ip_p[d] = sd_p d attn[d] + sum_k W_a[k][d] d a_p[k],  overwrites d a_p once every lane has read it
+// The staged rows have an odd pitch AP, so the pair-per-lane reads are free of bank conflicts.  Every sum has a fixed order and
+// the per-warp partials are reduced by the fixed-order pass: bit-identical from run to run.  The dropout masks are the same
+// (seed, counter) indices as the other kernels, or the given `masks`.
+template <int D>
+struct AfmWide {
+    static constexpr int AP = D | 1;                      // floats per staged pair row
+};
+// exp(s_p - max) of one sample into sc (and a_p into aS); returns sum_p exp(s_p - max).  wrow / ba_k: lane k's row of W_a, b_a[k]
+template <int D>
+__device__ __forceinline__ float afm_scores_wide(const float* __restrict__ stage, const float* __restrict__ par, const float (&wrow)[D],
+                                                 float ba_k, const unsigned char* __restrict__ pi, const unsigned char* __restrict__ pj,
+                                                 float* __restrict__ aS, float* __restrict__ sc, int npair, int lane) {
+    constexpr int DP = AfmSmem<D>::DP, AP = AfmWide<D>::AP;
+    for (int p = 0; p < npair; ++p) {
+        const float* vi = stage + pi[p] * D;
+        const float* vj = stage + pj[p] * D;
+        float a = ba_k;
+#pragma unroll
+        for (int d = 0; d < D; ++d) a = fmaf(wrow[d], vi[d] * vj[d], a);
+        if (lane < D) aS[p * AP + lane] = a;
+    }
+    __syncwarp();
+    const float* ws = par + D * DP + DP;
+    const float bs = par[D * DP + 3 * DP];
+    float mx = -INFINITY;
+    for (int p = lane; p < npair; p += 32) {
+        float s = bs;
+        for (int k = 0; k < D; ++k) s = fmaf(ws[k], fmaxf(aS[p * AP + k], 0.f), s);
+        sc[p] = s;
+        mx = fmaxf(mx, s);
+    }
+    mx = afm_warp_max(mx);
+    float sum = 0.f;
+    for (int p = lane; p < npair; p += 32) {
+        const float e = expf(sc[p] - mx);
+        sc[p] = e;
+        sum += e;
+    }
+    return afm_warp_sum(sum);
+}
+
+// dynamic smem: PAR | nw * (fd_pad + npair_pad + npair * AP) floats | 2 * npair bytes
+template <int D>
+__global__ void __launch_bounds__(AFM_WARPS * 32)
+afm_fwd_wide_kernel(const float* __restrict__ rows, int64_t ld_rows, const float* __restrict__ params, AfmDrop dr,
+                    float* __restrict__ out, int64_t batch, int fields) {
+    extern __shared__ __align__(16) float smem[];
+    constexpr int DP = AfmSmem<D>::DP, PAR = AfmSmem<D>::PAR, AP = AfmWide<D>::AP;
+    static_assert(D <= 32, "one lane per output unit");
+    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    const int fd = fields * D, npair = fields * (fields - 1) / 2, npp = (npair + 3) / 4 * 4;
+    const int per_warp = ((fd + 3) & ~3) + npp + npair * AP;
+    float* par = smem;
+    float* stage = smem + PAR + wib * per_warp;
+    float* sc = stage + ((fd + 3) & ~3);
+    float* aS = sc + npp;
+    unsigned char* pi = reinterpret_cast<unsigned char*>(smem + PAR + nw * per_warp);
+    unsigned char* pj = pi + npair;
+    AfmSmem<D>::load(par, params);
+    afm_pair_tables(pi, pj, nullptr, fields);
+    __syncthreads();
+    uint64_t seed = 0, ctr = 0;
+    if (dr.rng && !dr.masks) { seed = dr.rng[0]; ctr = dr.rng[1]; }
+    const bool own = lane < D;
+    float wrow[D];
+#pragma unroll
+    for (int d = 0; d < D; ++d) wrow[d] = own ? par[lane * DP + d] : 0.f;
+    const float ba_k = own ? par[D * DP + lane] : 0.f;
+    const float fcw_d = own ? par[D * DP + 2 * DP + lane] : 0.f;
+    const float fcb = par[D * DP + 3 * DP + 1];
+    const int width = npair + D;
+    for (int64_t b = (int64_t)blockIdx.x * nw + wib; b < batch; b += (int64_t)gridDim.x * nw) {
+        const float* r = rows + b * ld_rows;
+        for (int i = lane; i < fd; i += 32) stage[i] = __ldg(r + i);
+        __syncwarp();
+        const float sum = afm_scores_wide<D>(stage, par, wrow, ba_k, pi, pj, aS, sc, npair, lane);
+        for (int p = lane; p < npair; p += 32) sc[p] = sc[p] / sum * afm_mask(dr, seed, ctr, b, width, p);     // sd_p
+        __syncwarp();
+        float y = 0.f;
+        if (own) {
+            float at = 0.f;
+            for (int p = 0; p < npair; ++p) at = fmaf(sc[p], stage[pi[p] * D + lane] * stage[pj[p] * D + lane], at);
+            y = fcw_d * (at * afm_mask(dr, seed, ctr, b, width, npair + lane));
+        }
+        y = afm_warp_sum(y);
+        if (lane == 0) out[b] = fcb + y;
+        __syncwarp();
+    }
+}
+
+// dynamic smem: PAR | nw * (fd_pad + 2 * npair_pad + DP + npair * AP) floats | 2 * npair + fields * fields bytes
+template <int D>
+__global__ void __launch_bounds__(AFM_WARPS * 32)
+afm_bwd_wide_kernel(const float* __restrict__ rows, int64_t ld_rows, const float* __restrict__ params, AfmDrop dr,
+                    const float* __restrict__ gout, float* __restrict__ grows, int64_t ld_grows, float* __restrict__ part,
+                    int64_t batch, int fields) {
+    extern __shared__ __align__(16) float smem[];
+    constexpr int DP = AfmSmem<D>::DP, PAR = AfmSmem<D>::PAR, AP = AfmWide<D>::AP;
+    constexpr int NP = D * D + 3 * D + 2;
+    static_assert(D <= 32, "one lane per output unit");
+    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    const int fd = fields * D, npair = fields * (fields - 1) / 2, npp = (npair + 3) / 4 * 4;
+    const int fdp = (fd + 3) & ~3;
+    const int per_warp = fdp + 2 * npp + DP + npair * AP;
+    float* par = smem;
+    float* stage = smem + PAR + wib * per_warp;
+    float* sc = stage + fdp;                // exp(s_p - max) -> score_p -> sd_p = score_p m1_p
+    float* dsc = sc + npp;                  // sd_p -> d L / d(score_p m1_p) -> d L / d s_p
+    float* dat = dsc + npp;                 // d L / d attn  [D]
+    float* aS = dat + DP;                   // a_p -> d a_p -> d ip_p   [npair, AP]
+    unsigned char* pi = reinterpret_cast<unsigned char*>(smem + PAR + nw * per_warp);
+    unsigned char* pj = pi + npair;
+    unsigned char* pidx = pj + npair;
+    AfmSmem<D>::load(par, params);
+    afm_pair_tables(pi, pj, pidx, fields);
+    __syncthreads();
+    uint64_t seed = 0, ctr = 0;
+    if (dr.rng && !dr.masks) { seed = dr.rng[0]; ctr = dr.rng[1]; }
+    const int width = npair + D;
+    const bool own = lane < D;
+    float wrow[D], wcol[D], dwa[D];
+#pragma unroll
+    for (int d = 0; d < D; ++d) {
+        wrow[d] = own ? par[lane * DP + d] : 0.f;
+        wcol[d] = own ? par[d * DP + lane] : 0.f;
+        dwa[d] = 0.f;
+    }
+    const float ba_k = own ? par[D * DP + lane] : 0.f;
+    const float ws_k = own ? par[D * DP + DP + lane] : 0.f;
+    const float fcw_d = own ? par[D * DP + 2 * DP + lane] : 0.f;
+    float dba_k = 0.f, dws_k = 0.f, dfcw_d = 0.f, dbs = 0.f, dfcb = 0.f;
+
+    for (int64_t b = (int64_t)blockIdx.x * nw + wib; b < batch; b += (int64_t)gridDim.x * nw) {
+        const float* r = rows + b * ld_rows;
+        for (int i = lane; i < fd; i += 32) stage[i] = __ldg(r + i);
+        __syncwarp();
+        const float sum = afm_scores_wide<D>(stage, par, wrow, ba_k, pi, pj, aS, sc, npair, lane);
+        for (int p = lane; p < npair; p += 32) {
+            const float score = sc[p] / sum;
+            sc[p] = score;
+            dsc[p] = score * afm_mask(dr, seed, ctr, b, width, p);
+        }
+        __syncwarp();
+        // lane d: attention output, d fc_w, d attn
+        const float g = __ldg(gout + b);
+        if (own) {
+            float at = 0.f;
+            for (int p = 0; p < npair; ++p) at = fmaf(dsc[p], stage[pi[p] * D + lane] * stage[pj[p] * D + lane], at);
+            const float m2 = afm_mask(dr, seed, ctr, b, width, npair + lane);
+            dfcw_d = fmaf(g, at * m2, dfcw_d);
+            dat[lane] = g * fcw_d * m2;
+        }
+        dfcb += g;
+        __syncwarp();
+        // lane = pair: d L / d s_p = score_p (t_p - sum_q score_q t_q),  t_p = <d attn, ip_p> m1_p
+        float dot = 0.f;
+        for (int p = lane; p < npair; p += 32) {
+            const float* vi = stage + pi[p] * D;
+            const float* vj = stage + pj[p] * D;
+            float t = 0.f;
+            for (int d = 0; d < D; ++d) t = fmaf(dat[d], vi[d] * vj[d], t);
+            t *= afm_mask(dr, seed, ctr, b, width, p);
+            dsc[p] = t;
+            dot = fmaf(sc[p], t, dot);
+        }
+        dot = afm_warp_sum(dot);
+        for (int p = lane; p < npair; p += 32) {
+            const float score = sc[p];
+            const float dsp = score * (dsc[p] - dot);
+            dbs += dsp;
+            dsc[p] = dsp;
+            sc[p] = score * afm_mask(dr, seed, ctr, b, width, p);
+        }
+        __syncwarp();
+        // pass A: lane k
+        for (int p = 0; p < npair; ++p) {
+            const float* vi = stage + pi[p] * D;
+            const float* vj = stage + pj[p] * D;
+            const float a = own ? aS[p * AP + lane] : 0.f;
+            const float dsp = dsc[p];
+            const float da = a > 0.f ? dsp * ws_k : 0.f;
+            dws_k = fmaf(dsp, fmaxf(a, 0.f), dws_k);
+            dba_k += da;
+#pragma unroll
+            for (int d = 0; d < D; ++d) dwa[d] = fmaf(da, vi[d] * vj[d], dwa[d]);
+            if (own) aS[p * AP + lane] = da;
+        }
+        __syncwarp();
+        // pass B: lane d; every lane reads row p of d a before it is overwritten by d ip_p
+        const float my_dat = own ? dat[lane] : 0.f;
+        for (int p = 0; p < npair; ++p) {
+            float dip = sc[p] * my_dat;
+#pragma unroll
+            for (int k = 0; k < D; ++k) dip = fmaf(wcol[k], aS[p * AP + k], dip);
+            __syncwarp();
+            if (own) aS[p * AP + lane] = dip;
+        }
+        __syncwarp();
+        // d v_i[d] = sum_{j != i} d ip_{pair(i,j)}[d] * v_j[d], j in order (as afm_bwd_kernel)
+        for (int t = lane; t < fd; t += 32) {
+            const int i = t / D, d = t - i * D;
+            const unsigned char* prow = pidx + i * fields;
+            float a0 = 0.f, a1 = 0.f;
+            int j = 0;
+            for (; j + 1 < fields; j += 2) {
+                if (j != i) a0 = fmaf(aS[prow[j] * AP + d], stage[j * D + d], a0);
+                if (j + 1 != i) a1 = fmaf(aS[prow[j + 1] * AP + d], stage[(j + 1) * D + d], a1);
+            }
+            if (j < fields && j != i) a0 = fmaf(aS[prow[j] * AP + d], stage[j * D + d], a0);
+            grows[b * ld_grows + t] = a0 + a1;
+        }
+        __syncwarp();
+    }
+    float* mine = part + ((int64_t)blockIdx.x * nw + wib) * NP;
+    if (own) {
+#pragma unroll
+        for (int d = 0; d < D; ++d) mine[lane * D + d] = dwa[d];
+        mine[D * D + lane] = dba_k;
+        mine[D * D + D + lane] = dws_k;
+        mine[D * D + 2 * D + 1 + lane] = dfcw_d;
+    }
+    const float sbs = afm_warp_sum(dbs);
+    if (lane == 0) { mine[D * D + 2 * D] = sbs; mine[D * D + 3 * D + 1] = dfcb; }
+}
+
 static int afm_blocks(int64_t batch, int per_sm) {
     int64_t want = (batch + AFM_WARPS - 1) / AFM_WARPS;
     const int64_t cap = (int64_t)RLCTR_SMS * per_sm;
@@ -369,6 +608,63 @@ static int afm_bwd_launch(const float* rows, int64_t ld_rows, const float* param
     return RLCTR_OK;
 }
 
+// D <= 10: the per-lane kernels; above that the wide kernels, with AFM_WARPS warps per block or fewer when their staging does not
+// fit (F = 23 at D = 32 takes two in the backward).  The partials never outnumber rlctr_afm_ws_bytes' blocks * AFM_WARPS.
+constexpr int AFM_LANE_MAX_D = 10;
+static int afm_wide_warps(size_t fixed, size_t per_warp, size_t* smem) {
+    int nw = AFM_WARPS;
+    while (nw > 1 && fixed + nw * per_warp > 200 * 1024) nw >>= 1;
+    *smem = fixed + nw * per_warp;
+    return *smem > 200 * 1024 ? 0 : nw;
+}
+template <int D>
+static int afm_fwd_dispatch(const float* rows, int64_t ld_rows, const float* params, const AfmDrop& dr, float* out, int64_t batch,
+                            int fields, cudaStream_t st) {
+    if constexpr (D <= AFM_LANE_MAX_D) {
+        return afm_fwd_launch<D>(rows, ld_rows, params, dr, out, batch, fields, st);
+    } else {
+        const int fd = fields * D, npair = fields * (fields - 1) / 2, npp = (npair + 3) / 4 * 4;
+        size_t smem;
+        const int nw = afm_wide_warps((size_t)AfmSmem<D>::PAR * sizeof(float) + 2 * (size_t)npair,
+                                      (size_t)(((fd + 3) & ~3) + npp + npair * AfmWide<D>::AP) * sizeof(float), &smem);
+        if (!nw) return RLCTR_EUNSUPPORTED;
+        if (smem > 48 * 1024)
+            RLCTR_CUDA(cudaFuncSetAttribute(afm_fwd_wide_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int64_t want = (batch + nw - 1) / nw;
+        const int64_t cap = (int64_t)RLCTR_SMS * 8;
+        afm_fwd_wide_kernel<D><<<(int)(want < cap ? want : cap), nw * 32, smem, st>>>(rows, ld_rows, params, dr, out, batch, fields);
+        RLCTR_LAUNCH_CHECK();
+        return RLCTR_OK;
+    }
+}
+template <int D>
+static int afm_bwd_dispatch(const float* rows, int64_t ld_rows, const float* params, const AfmDrop& dr, const float* gout,
+                            float* grows, int64_t ld_grows, float* dparams, float* part, int64_t batch, int fields, cudaStream_t st) {
+    if constexpr (D <= AFM_LANE_MAX_D) {
+        return afm_bwd_launch<D>(rows, ld_rows, params, dr, gout, grows, ld_grows, dparams, part, batch, fields, st);
+    } else {
+        const int fd = fields * D, npair = fields * (fields - 1) / 2, npp = (npair + 3) / 4 * 4;
+        size_t smem;
+        const int nw = afm_wide_warps((size_t)AfmSmem<D>::PAR * sizeof(float) + 2 * (size_t)npair + (size_t)fields * fields,
+                                      (size_t)(((fd + 3) & ~3) + 2 * npp + AfmSmem<D>::DP + npair * AfmWide<D>::AP) * sizeof(float),
+                                      &smem);
+        if (!nw) return RLCTR_EUNSUPPORTED;
+        if (smem > 48 * 1024)
+            RLCTR_CUDA(cudaFuncSetAttribute(afm_bwd_wide_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const int blocks = afm_blocks(batch, 3);
+        constexpr int NP = D * D + 3 * D + 2;
+        afm_bwd_wide_kernel<D><<<blocks, nw * 32, smem, st>>>(rows, ld_rows, params, dr, gout, grows, ld_grows, part, batch, fields);
+        RLCTR_LAUNCH_CHECK();
+        colsum_parts_kernel<<<colsum_parts_grid(NP), 256, 0, st>>>(part, dparams, nullptr, NP, 0, NP, blocks * nw);
+        RLCTR_LAUNCH_CHECK();
+        return RLCTR_OK;
+    }
+}
+
+#define AFM_DIMS(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) \
+                    X(17) X(18) X(19) X(20) X(21) X(22) X(23) X(24) X(25) X(26) X(27) X(28) X(29) X(30) X(31) X(32)
+constexpr int AFM_MAX_D = 32;
+
 }  // namespace rlctr
 
 using namespace rlctr;
@@ -391,7 +687,7 @@ static int afm_drop(AfmDrop* dr, float dropout_p, const uint64_t* rng_state, con
 extern "C" int rlctr_afm_fwd(const float* rows, int64_t ld_rows, const float* params, float* out, int64_t batch, int32_t fields,
                              int32_t dim, float dropout_p, const uint64_t* rng_state, const float* masks, rlctr_stream_t stream) {
     if (!rows || !params || !out || batch < 0 || fields < 2 || dim <= 0) return RLCTR_EINVAL;
-    if (fields > 23) return RLCTR_EUNSUPPORTED;
+    if (fields > 23 || dim > AFM_MAX_D) return RLCTR_EUNSUPPORTED;
     if (ld_rows < (int64_t)fields * dim) return RLCTR_EINVAL;
     AfmDrop dr;
     int rc = afm_drop(&dr, dropout_p, rng_state, masks);
@@ -399,9 +695,9 @@ extern "C" int rlctr_afm_fwd(const float* rows, int64_t ld_rows, const float* pa
     if (batch == 0) return RLCTR_OK;
     cudaStream_t st = (cudaStream_t)stream;
     switch (dim) {
-        case 4: return afm_fwd_launch<4>(rows, ld_rows, params, dr, out, batch, fields, st);
-        case 8: return afm_fwd_launch<8>(rows, ld_rows, params, dr, out, batch, fields, st);
-        case 10: return afm_fwd_launch<10>(rows, ld_rows, params, dr, out, batch, fields, st);
+#define AFM_FWD_CASE(DD) case DD: return afm_fwd_dispatch<DD>(rows, ld_rows, params, dr, out, batch, fields, st);
+        AFM_DIMS(AFM_FWD_CASE)
+#undef AFM_FWD_CASE
         default: return RLCTR_EUNSUPPORTED;
     }
 }
@@ -410,7 +706,7 @@ extern "C" int rlctr_afm_bwd(const float* rows, int64_t ld_rows, const float* pa
                              int64_t ld_grows, float* dparams, int64_t batch, int32_t fields, int32_t dim, float dropout_p,
                              const uint64_t* rng_state, const float* masks, void* ws, size_t ws_bytes, rlctr_stream_t stream) {
     if (!rows || !params || !gout || !grows || !dparams || batch <= 0 || fields < 2 || dim <= 0) return RLCTR_EINVAL;
-    if (fields > 23) return RLCTR_EUNSUPPORTED;
+    if (fields > 23 || dim > AFM_MAX_D) return RLCTR_EUNSUPPORTED;
     if (ld_rows < (int64_t)fields * dim || ld_grows < (int64_t)fields * dim) return RLCTR_EINVAL;
     if (!ws || ws_bytes < rlctr_afm_ws_bytes(batch, dim)) return RLCTR_EWORKSPACE;
     AfmDrop dr;
@@ -419,9 +715,10 @@ extern "C" int rlctr_afm_bwd(const float* rows, int64_t ld_rows, const float* pa
     cudaStream_t st = (cudaStream_t)stream;
     float* part = reinterpret_cast<float*>(ws);
     switch (dim) {
-        case 4: return afm_bwd_launch<4>(rows, ld_rows, params, dr, gout, grows, ld_grows, dparams, part, batch, fields, st);
-        case 8: return afm_bwd_launch<8>(rows, ld_rows, params, dr, gout, grows, ld_grows, dparams, part, batch, fields, st);
-        case 10: return afm_bwd_launch<10>(rows, ld_rows, params, dr, gout, grows, ld_grows, dparams, part, batch, fields, st);
+#define AFM_BWD_CASE(DD) \
+        case DD: return afm_bwd_dispatch<DD>(rows, ld_rows, params, dr, gout, grows, ld_grows, dparams, part, batch, fields, st);
+        AFM_DIMS(AFM_BWD_CASE)
+#undef AFM_BWD_CASE
         default: return RLCTR_EUNSUPPORTED;
     }
 }

@@ -27,7 +27,7 @@ extern unsigned long long g_rlctr_launches;
 
 static inline bool rlctr_aligned16(const void* p) { return (((uintptr_t)p) & 15u) == 0; }
 
-// lanes-per-row for a fused row of `rs` floats read as float4 chunks: 1,2,4 or 8 (rs <= 32)
+// lanes-per-row for a fused row of `rs` floats read as float4 chunks: 1, 2, 4, 8 (rs <= 32) or 16 (rs <= 64)
 static inline int rlctr_lanes_per_row(int rs) {
     int chunks = rs / 4;
     int l = 1;

@@ -8,12 +8,17 @@
 // x_l from them.  Parameter gradients (dw_l = sum_b ds_l * x_l, db_l = sum_b g_{l+1}) are accumulated per warp in
 // registers, combined per block through shared memory in a fixed order and written as per-block partials, which a
 // fixed-order pass (colsum_parts_kernel) reduces: bit-identical from run to run.
+//
+// C columns per lane: C = 8 serves F*D <= 256, C = 16 serves F*D <= 512 (D up to 32 at F = 15).  At C = 16 the 2*L*C gradient
+// accumulators (160 floats at L = 5) no longer fit beside x_l in registers: each lane accumulates them in its own columns of the
+// warp's shared-memory slice instead -- the same per-element fma sequence, so the same numbers.
 #include "common.cuh"
 
 namespace rlctr {
 
 constexpr int CROSS_MAX_L = 8;         // layers
 constexpr int CROSS_C = 8;             // columns per lane: F*D <= 256
+constexpr int CROSS_C_WIDE = 16;       // F*D <= 512
 constexpr int CROSS_WARPS = 4;
 
 __device__ __forceinline__ float warp_sum(float x) {
@@ -22,6 +27,7 @@ __device__ __forceinline__ float warp_sum(float x) {
     return x;
 }
 
+template <int C>
 __global__ void __launch_bounds__(CROSS_WARPS * 32)
 cross_fwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restrict__ w, const float* __restrict__ b, int layers,
                  float* __restrict__ out, int64_t ld_out, float* __restrict__ s_saved, int64_t batch, int dim) {
@@ -29,9 +35,9 @@ cross_fwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restr
     const int64_t warp0 = (int64_t)blockIdx.x * CROSS_WARPS + (threadIdx.x >> 5);
     const int64_t nwarps = (int64_t)gridDim.x * CROSS_WARPS;
     for (int64_t r = warp0; r < batch; r += nwarps) {
-        float a0[CROSS_C], a[CROSS_C];
+        float a0[C], a[C];
 #pragma unroll
-        for (int c = 0; c < CROSS_C; ++c) {
+        for (int c = 0; c < C; ++c) {
             const int k = lane + 32 * c;
             a0[c] = k < dim ? __ldg(x0 + r * ldx + k) : 0.f;
             a[c] = a0[c];
@@ -39,20 +45,20 @@ cross_fwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restr
         for (int l = 0; l < layers; ++l) {
             float d = 0.f;
 #pragma unroll
-            for (int c = 0; c < CROSS_C; ++c) {
+            for (int c = 0; c < C; ++c) {
                 const int k = lane + 32 * c;
                 if (k < dim) d = fmaf(a[c], __ldg(w + l * dim + k), d);
             }
             const float s = warp_sum(d);
             if (lane == 0 && s_saved) s_saved[r * layers + l] = s;
 #pragma unroll
-            for (int c = 0; c < CROSS_C; ++c) {
+            for (int c = 0; c < C; ++c) {
                 const int k = lane + 32 * c;
                 if (k < dim) a[c] = a0[c] * s + __ldg(b + l * dim + k) + a[c];      // (x0 * s + b) + x, the reference's order
             }
         }
 #pragma unroll
-        for (int c = 0; c < CROSS_C; ++c) {
+        for (int c = 0; c < C; ++c) {
             const int k = lane + 32 * c;
             if (k < dim) out[r * ld_out + k] = a[c];
         }
@@ -60,7 +66,7 @@ cross_fwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restr
 }
 
 // dynamic smem: CROSS_WARPS * 2 * layers * dim floats (per-warp dw | db partials)
-template <int L>
+template <int L, int C>
 __global__ void __launch_bounds__(CROSS_WARPS * 32)
 cross_bwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restrict__ w, const float* __restrict__ b,
                  const float* __restrict__ s_saved, const float* __restrict__ gout, int64_t ld_g, float* __restrict__ gx0,
@@ -69,15 +75,21 @@ cross_bwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restr
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int64_t warp0 = (int64_t)blockIdx.x * CROSS_WARPS + wib;
     const int64_t nwarps = (int64_t)gridDim.x * CROSS_WARPS;
-    float dw[L][CROSS_C], db[L][CROSS_C];
+    constexpr bool REG = C <= CROSS_C;                                     // gradient accumulators in registers, or in `mine`
+    float* mine = red + (size_t)wib * 2 * L * dim;
+    float dw[REG ? L : 1][C], db[REG ? L : 1][C];
 #pragma unroll
-    for (int l = 0; l < L; ++l)
+    for (int l = 0; l < (REG ? L : 1); ++l)
 #pragma unroll
-        for (int c = 0; c < CROSS_C; ++c) { dw[l][c] = 0.f; db[l][c] = 0.f; }
+        for (int c = 0; c < C; ++c) { dw[l][c] = 0.f; db[l][c] = 0.f; }
+    if (!REG) {
+        for (int i = lane; i < 2 * L * dim; i += 32) mine[i] = 0.f;
+        __syncwarp();
+    }
     for (int64_t r = warp0; r < batch; r += nwarps) {
-        float a0[CROSS_C], xl[L][CROSS_C], g[CROSS_C], g0[CROSS_C], s[L];
+        float a0[C], xl[L][C], g[C], g0[C], s[L];
 #pragma unroll
-        for (int c = 0; c < CROSS_C; ++c) {
+        for (int c = 0; c < C; ++c) {
             const int k = lane + 32 * c;
             a0[c] = k < dim ? __ldg(x0 + r * ldx + k) : 0.f;
             g[c] = k < dim ? __ldg(gout + r * ld_g + k) : 0.f;
@@ -90,7 +102,7 @@ cross_bwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restr
 #pragma unroll
         for (int l = 0; l + 1 < L; ++l)
 #pragma unroll
-            for (int c = 0; c < CROSS_C; ++c) {
+            for (int c = 0; c < C; ++c) {
                 const int k = lane + 32 * c;
                 xl[l + 1][c] = k < dim ? a0[c] * s[l] + __ldg(b + l * dim + k) + xl[l][c] : 0.f;
             }
@@ -98,32 +110,38 @@ cross_bwd_kernel(const float* __restrict__ x0, int64_t ldx, const float* __restr
         for (int l = L - 1; l >= 0; --l) {
             float d = 0.f;
 #pragma unroll
-            for (int c = 0; c < CROSS_C; ++c) d = fmaf(g[c], a0[c], d);
+            for (int c = 0; c < C; ++c) d = fmaf(g[c], a0[c], d);
             const float ds = warp_sum(d);                                  // dL/ds_l = <g_{l+1}, x_0>
 #pragma unroll
-            for (int c = 0; c < CROSS_C; ++c) {
+            for (int c = 0; c < C; ++c) {
                 const int k = lane + 32 * c;
-                db[l][c] += g[c];                                          // dL/db_l
-                dw[l][c] = fmaf(ds, xl[l][c], dw[l][c]);                   // dL/dw_l
+                if constexpr (REG) {
+                    db[l][c] += g[c];                                      // dL/db_l
+                    dw[l][c] = fmaf(ds, xl[l][c], dw[l][c]);               // dL/dw_l
+                } else if (k < dim) {                                      // lane-private columns: no race
+                    mine[(L + l) * dim + k] += g[c];
+                    mine[l * dim + k] = fmaf(ds, xl[l][c], mine[l * dim + k]);
+                }
                 g0[c] = fmaf(g[c], s[l], g0[c]);                           // dL/dx_0 through the explicit x_0 factor
                 if (k < dim) g[c] = fmaf(ds, __ldg(w + l * dim + k), g[c]);    // g_l = g_{l+1} + ds * w_l
             }
         }
 #pragma unroll
-        for (int c = 0; c < CROSS_C; ++c) {
+        for (int c = 0; c < C; ++c) {
             const int k = lane + 32 * c;
             if (k < dim) gx0[r * ld_gx + k] = g0[c] + g[c];                // + g_0 (x_0 is also the first x_l)
         }
     }
     // block partials: warps in a fixed order
-    float* mine = red + (size_t)wib * 2 * L * dim;
+    if constexpr (REG) {
 #pragma unroll
-    for (int l = 0; l < L; ++l)
+        for (int l = 0; l < L; ++l)
 #pragma unroll
-        for (int c = 0; c < CROSS_C; ++c) {
-            const int k = lane + 32 * c;
-            if (k < dim) { mine[l * dim + k] = dw[l][c]; mine[(L + l) * dim + k] = db[l][c]; }
-        }
+            for (int c = 0; c < C; ++c) {
+                const int k = lane + 32 * c;
+                if (k < dim) { mine[l * dim + k] = dw[l][c]; mine[(L + l) * dim + k] = db[l][c]; }
+            }
+    }
     __syncthreads();
     const int per = L * dim;
     for (int i = threadIdx.x; i < per; i += blockDim.x) {
@@ -152,11 +170,15 @@ extern "C" size_t rlctr_cross_ws_bytes(int64_t batch, int32_t dim, int32_t layer
 extern "C" int rlctr_cross_fwd(const float* x0, int64_t ldx, const float* w, const float* b, int32_t layers, float* out,
                                int64_t ld_out, float* s_saved, int64_t batch, int32_t dim, rlctr_stream_t stream) {
     if (!x0 || !w || !b || !out || batch < 0 || dim <= 0 || layers <= 0) return RLCTR_EINVAL;
-    if (dim > 32 * CROSS_C || layers > CROSS_MAX_L) return RLCTR_EUNSUPPORTED;
+    if (dim > 32 * CROSS_C_WIDE || layers > CROSS_MAX_L) return RLCTR_EUNSUPPORTED;
     if (ldx < dim || ld_out < dim) return RLCTR_EINVAL;
     if (batch == 0) return RLCTR_OK;
-    cross_fwd_kernel<<<cross_blocks(batch), CROSS_WARPS * 32, 0, (cudaStream_t)stream>>>(x0, ldx, w, b, layers, out, ld_out, s_saved,
-                                                                                        batch, dim);
+    if (dim <= 32 * CROSS_C)
+        cross_fwd_kernel<CROSS_C><<<cross_blocks(batch), CROSS_WARPS * 32, 0, (cudaStream_t)stream>>>(x0, ldx, w, b, layers, out, ld_out,
+                                                                                                     s_saved, batch, dim);
+    else
+        cross_fwd_kernel<CROSS_C_WIDE><<<cross_blocks(batch), CROSS_WARPS * 32, 0, (cudaStream_t)stream>>>(x0, ldx, w, b, layers, out,
+                                                                                                          ld_out, s_saved, batch, dim);
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
 }
@@ -165,7 +187,7 @@ extern "C" int rlctr_cross_bwd(const float* x0, int64_t ldx, const float* w, con
                                const float* gout, int64_t ld_g, float* gx0, int64_t ld_gx, float* dw, float* db, int64_t batch,
                                int32_t dim, void* ws, size_t ws_bytes, rlctr_stream_t stream) {
     if (!x0 || !w || !b || !s_saved || !gout || !gx0 || !dw || !db || batch <= 0 || dim <= 0) return RLCTR_EINVAL;
-    if (dim > 32 * CROSS_C) return RLCTR_EUNSUPPORTED;
+    if (dim > 32 * CROSS_C_WIDE) return RLCTR_EUNSUPPORTED;
     if (ldx < dim || ld_g < dim || ld_gx < dim) return RLCTR_EINVAL;
     if (!ws || ws_bytes < rlctr_cross_ws_bytes(batch, dim, layers)) return RLCTR_EWORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -174,10 +196,18 @@ extern "C" int rlctr_cross_bwd(const float* x0, int64_t ldx, const float* w, con
     float* dw_part = reinterpret_cast<float*>(ws);
     float* db_part = dw_part + (size_t)blocks * per;
     const size_t smem = (size_t)CROSS_WARPS * 2 * per * sizeof(float);
-    if (smem > 48 * 1024) return RLCTR_EUNSUPPORTED;
+    const bool wide = dim > 32 * CROSS_C;
+    if (smem > (wide ? 128 : 48) * 1024) return RLCTR_EUNSUPPORTED;          // wide: 4 x 2 x 6 x 512 floats at most
 #define LAUNCH_CROSS(LL)                                                                                                   \
-    cross_bwd_kernel<LL><<<blocks, CROSS_WARPS * 32, smem, st>>>(x0, ldx, w, b, s_saved, gout, ld_g, gx0, ld_gx, dw_part, db_part, \
-                                                                 batch, dim)
+    if (!wide) {                                                                                                           \
+        cross_bwd_kernel<LL, CROSS_C><<<blocks, CROSS_WARPS * 32, smem, st>>>(x0, ldx, w, b, s_saved, gout, ld_g, gx0, ld_gx, dw_part, \
+                                                                              db_part, batch, dim);                        \
+    } else {                                                                                                               \
+        if (smem > 48 * 1024)                                                                                              \
+            RLCTR_CUDA(cudaFuncSetAttribute(cross_bwd_kernel<LL, CROSS_C_WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+        cross_bwd_kernel<LL, CROSS_C_WIDE><<<blocks, CROSS_WARPS * 32, smem, st>>>(x0, ldx, w, b, s_saved, gout, ld_g, gx0, ld_gx,  \
+                                                                                   dw_part, db_part, batch, dim);          \
+    }
     switch (layers) {
         case 1: LAUNCH_CROSS(1); break;
         case 2: LAUNCH_CROSS(2); break;

@@ -2,7 +2,8 @@
 // and K5 the Feature_Embedding RL state encoder.  sm_100a.
 //
 // Thread mapping (all three kernels): one warp per sample, LPR lanes per gathered row, each
-// lane reading one aligned float4 (128-bit) chunk of the fused row.  For the default
+// lane reading one aligned float4 (128-bit) chunk of the fused row (K1 also takes LPR = 16 for the
+// 36-float rows of D = 32 with a first-order column: lanes 9..15 of a row slot idle).  For the default
 // latent_dims=10 the row is [w, v0..v9, pad] = 12 floats = 3 chunks -> LPR=4, 8 rows per warp
 // request, the 15 fields of a sample in two requests.  Lanes of one row hit one or two 32 B
 // sectors in a single request (1.25 L1 wavefronts/row instead of 3 for a lane-per-row map).
@@ -568,7 +569,7 @@ extern "C" int rlctr_embed_fwd(const int64_t* ids, const rlctr_table* table, con
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
     }
-    if (rs > 32) return RLCTR_EUNSUPPORTED;
+    if (rs > 36) return RLCTR_EUNSUPPORTED;      // 36: a first-order column + 32 latent floats, padded
     if (sums && !rlctr_aligned16(sums)) return RLCTR_EALIGN;
     int grid = grid_for_warps(batch, 8, 5);      // 5 resident CTAs of 8 warps per SM (48 registers)
 #define LAUNCH_EMBED(L)                                                                              \
@@ -579,7 +580,8 @@ extern "C" int rlctr_embed_fwd(const int64_t* ids, const rlctr_table* table, con
         case 1: LAUNCH_EMBED(1); break;
         case 2: LAUNCH_EMBED(2); break;
         case 4: LAUNCH_EMBED(4); break;
-        default: LAUNCH_EMBED(8); break;
+        case 8: LAUNCH_EMBED(8); break;
+        default: LAUNCH_EMBED(16); break;        // 33..36 floats: 9 chunks on 16 lanes, two rows per warp request
     }
 #undef LAUNCH_EMBED
     RLCTR_LAUNCH_CHECK();

@@ -752,11 +752,12 @@ rows_long_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __rest
     }
 }
 
-// wide rows (row_stride > 32 floats: the interleaved FFM table): one WARP per sorted position,
+// wide rows (row_stride > 32 floats: the interleaved FFM table, 36-float FM rows): one WARP per sorted position,
 // lanes stride the float4 chunks of the row (WCH chunks per lane); runs are walked sequentially
-// in slot order so the sum is bit-identical from run to run.
-constexpr int WCH = 2;                                   // rows up to 32*4*WCH = 256 floats
-template <int APPLY>
+// in slot order so the sum is bit-identical from run to run.  WCH = 2: rows up to 256 floats; WCH = 4: up to 512
+// (FFM at F = 15, D = 18..33).
+constexpr int WCH_MAX = 4;
+template <int APPLY, int WCH>
 __global__ void __launch_bounds__(256)
 rows_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                  GradView g, TableView t, AdamView a, float* __restrict__ dense_grad) {
@@ -1433,9 +1434,12 @@ static int launch_rows(const uint32_t* sorted_ids, const uint32_t* sorted_slots,
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
     }
-    if (t.rs % 4 != 0 || t.rs > 128 * WCH) return RLCTR_EUNSUPPORTED;
+    if (t.rs % 4 != 0 || t.rs > 128 * WCH_MAX) return RLCTR_EUNSUPPORTED;
     if (t.rs > 32) {
-        rows_wide_kernel<APPLY><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
+        if (t.rs <= 256)
+            rows_wide_kernel<APPLY, 2><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
+        else
+            rows_wide_kernel<APPLY, 4><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
     }
