@@ -1,30 +1,27 @@
-// mlp_tma.cu -- K4 (second generation): the dense-layer GEMMs with TMA-fed operand tiles.
+// mlp_tma.cu -- K4: the dense-layer GEMMs with TMA-fed operand tiles and tcgen05 MMAs.
 //
 //     C[M,N] = A[M,K] * B[N,K]^T (+ bias[N]) (ReLU)        fp32 in, fp32 out, 3xTF32 split (see mlp.cu)
 //
-// What changed against gemm3x_tf32_kernel (mlp.cu), which ncu showed latency-bound at 14 % tensor-pipe
-// activity with every warp parked on an mbarrier (profiles/r1_ncu_top_kernels.md):
-//   * operand tiles are fetched by TMA (cp.async.bulk.tensor, SWIZZLE_128B, zero fill outside the tensor): one
-//     elected thread issues whole boxes, no per-thread address arithmetic, no LDGSTS issue slots;
-//   * the small operand of forward / dgrad -- the WEIGHT -- is split into (hi, lo) ONCE per call by a tiny
-//     elementwise kernel and arrives ready-made through two tensor maps: nothing to convert on the B side;
-//   * the converter warps only touch the streamed activation tile: raw -> hi (in place) and lo, elementwise at
-//     identical byte offsets, so they are independent of the swizzle and of the operand's major-ness;
-//   * operands that are contiguous along M/N instead of K (dgrad's W, wgrad's dY^T and X) are consumed in place
-//     as MN-major UMMA operands (TMA boxes of 32 mn x 32 k in the SWIZZLE_128B_BASE32B layout): no 4-byte
-//     transposing copies.
-//
-// Third generation (this file's default data path; profiles/r1e_*):
-//   * the A operand lives in TENSOR MEMORY: a converter thread owns one row of the raw 128 x 32 tile, reads its 32 k-values from
-//     the swizzled shared-memory tile, splits them and writes (A_hi, A_lo) with tcgen05.st; the MMAs take A from TMEM
-//     (tcgen05.mma ... [d_tmem], [a_tmem], b_desc), so A crosses the shared-memory port once instead of four times per k-block;
+// The software-staged gemm3x_tf32_kernel (mlp.cu) is latency-bound at 14 % tensor-pipe activity with every warp parked on an
+// mbarrier (profiles/r1_ncu_top_kernels.md).  This kernel keeps the tensor pipe fed:
+//   * operand tiles are fetched by TMA (cp.async.bulk.tensor, SWIZZLE_128B, zero fill outside the tensor): one elected thread
+//     issues whole boxes, no per-thread address arithmetic, no LDGSTS issue slots;
+//   * the small operand of forward / dgrad -- the WEIGHT -- is split into (hi, lo) ONCE per call by a tiny elementwise kernel
+//     and arrives ready-made through two tensor maps; wgrad's raw B tile is split in shared memory by the converter warps
+//     (raw -> hi in place and lo, elementwise at identical byte offsets: independent of the swizzle and of the major-ness);
+//   * operands that are contiguous along M/N instead of K (dgrad's W, wgrad's dY^T and X) are consumed in place as MN-major
+//     UMMA operands (TMA boxes of 32 mn x 32 k in the SWIZZLE_128B_BASE32B layout): no 4-byte transposing copies;
+//   * the streamed A operand lives in TENSOR MEMORY: a converter thread owns one row of the raw 128 x 32 tile, reads its 32
+//     k-values from the swizzled shared-memory tile, splits them and writes (A_hi, A_lo) with tcgen05.st; the MMAs take A from
+//     TMEM (tcgen05.mma ... [d_tmem], [a_tmem], b_desc), so A crosses the shared-memory port once per k-block (profiles/r1e_*);
+//     for wgrad the same thread's sum over its row is the bias gradient;
 //   * C leaves through per-warp 32 x 32 staging blocks and TMA stores (cp.async.bulk.tensor ... global.shared::cta): full
-//     128-byte row segments instead of 16-byte pieces of 32 different lines per store instruction;
+//     128-byte row segments instead of 16-byte pieces of 32 different lines per store instruction.  Split-K partials, C that
+//     TMA cannot address and the 16-column tail of a tile are stored per thread;
 //   * dgrad takes the ReLU / dropout mask of the layer below from TMA-loaded 32 x 32 blocks, one per epilogue warp, requested a
-//     chunk ahead (instantiation <PAIR = false, MASK = true>; RLCTR_GEMM_M_TMA=0 reads it per thread as before, same bits);
+//     chunk ahead (instantiation MASK = true); a mask TMA cannot address is read per thread, with the same bits;
 //   * the all-zero k-steps of a ragged last k-block (K % 32 != 0: TMA zero fill) are not issued;
-//   * kept behind switches: A from shared memory + direct stores (RLCTR_GEMM_A_TMEM=0, RLCTR_GEMM_C_TMA=0), the B tile multicast
-//     to a CTA pair (RLCTR_GEMM_CLUSTER=2), L2 prefetch of A (RLCTR_GEMM_L2_AHEAD), per-stage clock stamps (RLCTR_GEMM_DBG).
+//   * RLCTR_GEMM_DBG records per-stage clock stamps of block 0 (scratch/gemm_trace.py).
 //
 // Warp roles (320 threads, one CTA per SM, persistent over output tiles):
 //     warps 0-3  converters        wait raw[s] -> row of A: split -> tcgen05.st (hi | lo) -> arrive full[s]
@@ -64,14 +61,8 @@ struct Args {
     int a_mn, b_mn;                       // 1: operand is contiguous along M (N) instead of K
     int b_presplit;                       // 1: B arrives as (hi, lo) through mapB / mapBlo
     int relu;
-    int a_tmem;                           // 1: the converters write (A_hi, A_lo) into TENSOR MEMORY and the MMAs read A from there
     int acc_stride, a_col0;               // TMEM columns: accumulator stage s at s*acc_stride, A stage s at a_col0 + 64*s (hi | lo)
-    int pair;                             // 1: cta_group::2 -- a CTA pair computes 256 rows per MMA, each CTA staging HALF of the B tile
-    int cluster;                          // CTAs per cluster (1 or 2): the B tile is fetched once per cluster (TMA multicast), each CTA
-                                          // owning a different m-tile of the same (n-tile, split)
-    int l2_ahead;                         // stages of A the producer prefetches into L2 ahead of the pipeline (0: off)
     int c_tma;                            // 1: the epilogue stages 32x32 blocks of C in shared memory and TMA-stores them (mapC)
-    int m_tma;                            // 1: the dgrad mask arrives as TMA-loaded 32x32 blocks (mapM), one block per epilogue warp
     long long* dbg;                       // RLCTR_GEMM_DBG: per-stage clock64 stamps of block 0 (scratch/gemm_trace.py), else null
     float* colsum_part;                   // wgrad only: [splits][M] partial column sums of the MN-major A operand (db), or null
     Epilogue epi;                         // fused dropout (forward) / ReLU-dropout mask of the layer below (dgrad)
@@ -126,13 +117,6 @@ __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t cols) {
 }
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc),
-        "r"(accumulate) : "memory");
 }
 // A operand from tensor memory (lanes = rows of A, one 32-bit column per k): no shared-memory read for A
 __device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
@@ -204,79 +188,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t sr
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-// pull one box into L2 only (no shared-memory destination, no barrier): the later cp.async.bulk.tensor of the same box hits L2
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* map, int c0, int c1) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(map)), "r"(c0),
-                 "r"(c1) : "memory");
-}
-// the same box delivered to the same shared-memory offset (and signalled on the same barrier offset) of every CTA in `mask`
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], [%4], %5;"
-        ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(bar), "h"(mask) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(mask) : "memory");
-}
-// ---- cta_group::2: one MMA spans the CTA pair (M = 256: 128 rows in each CTA's tensor memory), B is read half from each CTA's
-// shared memory (same offsets), issued by the leader CTA (cluster rank 0) alone
-__device__ __forceinline__ void tmem_alloc2(uint32_t dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_tf32_ts2(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    const uint32_t z = 0;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::tf32 [%0], [%1], %2, %3, {%5, %5, %5, %5, %5, %5, %5, %5}, p;\n\t}" ::"r"(tmem_d), "r"(tmem_a),
-        "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(z) : "memory");
-}
-__device__ __forceinline__ void umma_commit2_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(mask) : "memory");
-}
-// arrive on the barrier at the same shared-memory offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t rank) {
-    asm volatile(
-        "{\n\t.reg .b32 ra;\n\t"
-        "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-        "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}" ::"r"(bar), "r"(rank) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint32_t bar, uint32_t parity) {       // barriers that peers arrive on
-    uint64_t t0 = 0;
-    uint32_t spins = 0;
-    while (!mbar_try_cluster(bar, parity)) {
-        if ((++spins & 0x3fffu) == 0) {
-            uint64_t now;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
-            if (t0 == 0) t0 = now;
-            else if (now - t0 > 4000000000ull) mbar_timeout(bar, parity);
-        }
-    }
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
 }
@@ -340,28 +251,7 @@ __device__ __forceinline__ void split_tile(uint32_t hi, uint32_t lo, int bytes, 
     }
 }
 
-// The same split for the MN-major A tile of wgrad (dY^T: [32 k-rows][128 m] as four 4096-byte blocks of 32 m) that ALSO
-// accumulates the raw values per column: the bias gradient db[m] = sum_k dY[k, m] falls out of the pass the converters
-// make anyway.  A thread always meets the same four logical columns of each m-block (the 32-byte-chunk swizzle XORs the
-// chunk index with (k & 3), and a thread's k-rows keep k & 3 fixed), so four float4 accumulators suffice.
-__device__ __forceinline__ void split_tile_colsum(uint32_t hi, uint32_t lo, int tid, float4 (&acc)[BM / 32]) {
-    constexpr int STEP = CONV_WARPS * 32 * 16;                    // 2048 B = 16 k-rows of one m-block
-#pragma unroll
-    for (int j = 0; j < BM / 32; ++j) {
-        const int off = tid * 16 + j * 4096;
-        const float4 x0 = lds128(hi + off), x1 = lds128(hi + off + STEP);
-        float4 h, l;
-        split4(x0, h, l);
-        sts128(hi + off, h);
-        sts128(lo + off, l);
-        split4(x1, h, l);
-        sts128(hi + off + STEP, h);
-        sts128(lo + off + STEP, l);
-        acc[j].x += x0.x + x1.x; acc[j].y += x0.y + x1.y; acc[j].z += x0.z + x1.z; acc[j].w += x0.w + x1.w;
-    }
-}
-
-// A-in-TMEM converters: thread t owns row m = t of the 128 x 32 raw A tile.  It reads its 32 k-values from the swizzled
+// Converters: thread t owns row m = t of the 128 x 32 raw A tile.  It reads its 32 k-values from the swizzled
 // shared-memory tile (K-major: eight 16-byte chunks, chunk c stored at c ^ (t & 7) -- a quarter-warp covers all 32 banks;
 // MN-major: one 4-byte element per k-row, a warp reads 128 contiguous bytes), splits them and writes hi to TMEM columns
 // [col, col + 32) and lo to [col + 32, col + 64) of its lane.  Returns the sum of the raw values (wgrad's bias gradient).
@@ -406,18 +296,13 @@ __device__ __forceinline__ float split_row_to_tmem(uint32_t raw, bool a_mn, int 
 struct TileWalk {                          // this CTA's (tile, k-block) sequence, identical in every role
     int tile, kb0, kb1, mt, nt, split;
 };
-// With clusters, `tile` counts CLUSTER tiles (cluster consecutive m-tiles of one (n-tile, split)): every CTA of a cluster walks
-// the same sequence, CTA `rank` taking m-tile mt*cluster + rank (possibly past the end: it then computes on zero-filled rows and
-// stores nothing, but still takes part in the shared B loads).
-__device__ __forceinline__ bool tile_decode(TileWalk& w, const Args& g, int total_tiles, int rank = 0) {
+__device__ __forceinline__ bool tile_decode(TileWalk& w, const Args& g, int total_tiles) {
     if (w.tile >= total_tiles) return false;
-    const int mtc = (g.m_tiles + g.cluster - 1) / g.cluster;
-    const int mn = mtc * g.n_tiles;
+    const int mn = g.m_tiles * g.n_tiles;
     w.split = w.tile / mn;
     const int r = w.tile - w.split * mn;
     w.mt = r / g.n_tiles;
     w.nt = r - w.mt * g.n_tiles;
-    w.mt = w.mt * g.cluster + rank;
     const int kb_total = (g.K + BK - 1) / BK;
     w.kb0 = w.split * g.kb_per_split;
     w.kb1 = min(w.kb0 + g.kb_per_split, kb_total);
@@ -607,11 +492,9 @@ __device__ __forceinline__ void epilogue_tile_tma(const EpiCtx& e, uint32_t tadd
     }
 }
 
-// PAIR: the cta_group::2 instantiation (must be launched in clusters of two; the PAIR = false instantiation contains no 2-CTA
-// instruction and runs with any cluster size)
 // MASK: the dgrad instantiation whose epilogue takes the mask of the layer below from TMA-loaded blocks (its own instantiation:
 // the mask pipeline's registers must not cost the other GEMMs theirs -- measured +2-3 us each when it was a runtime switch)
-template <bool PAIR, bool MASK>
+template <bool MASK>
 __global__ void __launch_bounds__(THREADS, 1)
 gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                   const __grid_constant__ CUtensorMap mapBlo, const __grid_constant__ CUtensorMap mapC,
@@ -628,24 +511,20 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
     const bool bias_in_smem = g.bias != nullptr && g.n_tiles * g.n_tile <= BIAS_SMEM;
     if (bias_in_smem)
         for (int i = threadIdx.x; i < g.n_tiles * g.n_tile; i += THREADS) s_bias[i] = i < g.N ? __ldg(g.bias + i) : 0.f;
-    const uint32_t b_bytes = (uint32_t)g.n_tile * (PAIR ? 64u : 128u);     // pair: this CTA stages half of the B tile's rows
-    const uint32_t a_bytes = g.a_tmem ? A_TILE_BYTES : 2 * A_TILE_BYTES;       // raw A only when (hi, lo) live in TMEM
-    const uint32_t stage_bytes = a_bytes + 2 * b_bytes;
-    const int rank = g.cluster > 1 ? (int)cluster_ctarank() : 0;
-    const int cluster_id = (int)blockIdx.x / g.cluster, n_clusters = (int)gridDim.x / g.cluster;
-    const int total_tiles = ((g.m_tiles + g.cluster - 1) / g.cluster) * g.n_tiles * g.splits;
-    const uint16_t cmask = (uint16_t)((1u << g.cluster) - 1u);
+    const uint32_t b_bytes = (uint32_t)g.n_tile * 128u;
+    const uint32_t stage_bytes = A_TILE_BYTES + 2 * b_bytes;         // raw A, then B (hi, lo)
+    const int total_tiles = g.m_tiles * g.n_tiles * g.splits;
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < g.stages; ++s) {
             mbar_init(smem_u32(&raw_bar[s]), 1);
-            mbar_init(smem_u32(&full_bar[s]), (uint32_t)(CONV_WARPS * 32 * (PAIR ? 2 : 1)));   // pair: both CTAs' converters (leader's copy)
-            mbar_init(smem_u32(&empty_bar[s]), (uint32_t)(PAIR ? 1 : g.cluster));   // every CTA of the cluster has retired its MMAs on the slot
+            mbar_init(smem_u32(&full_bar[s]), (uint32_t)(CONV_WARPS * 32));
+            mbar_init(smem_u32(&empty_bar[s]), 1);
         }
         for (int s = 0; s < EPI_WARPS; ++s) mbar_init(smem_u32(&mask_bar[s]), 1);
         for (int s = 0; s < 2; ++s) {
             mbar_init(smem_u32(&tmem_full_bar[s]), 1);
-            mbar_init(smem_u32(&tmem_empty_bar[s]), (uint32_t)(EPI_WARPS * 32 * (PAIR ? 2 : 1)));
+            mbar_init(smem_u32(&tmem_empty_bar[s]), (uint32_t)(EPI_WARPS * 32));
         }
         fence_barrier_init();
     }
@@ -654,15 +533,11 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         tma_prefetch_desc(&mapB);
         if (g.b_presplit) tma_prefetch_desc(&mapBlo);
         if (g.c_tma) tma_prefetch_desc(&mapC);
-        if (g.m_tma) tma_prefetch_desc(&mapM);
+        if (MASK) tma_prefetch_desc(&mapM);
     }
-    if (warp == MMA_WARP) {
-        if (PAIR) tmem_alloc2(smem_u32(&tmem_base_smem), TMEM_COLS);
-        else tmem_alloc(smem_u32(&tmem_base_smem), TMEM_COLS);
-    }
+    if (warp == MMA_WARP) tmem_alloc(smem_u32(&tmem_base_smem), TMEM_COLS);
     tc_fence_before();
     __syncthreads();
-    if (g.cluster > 1) cluster_sync_all();                 // the peer's barriers exist before anything is multicast at them
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_smem;
     if (g.dbg && threadIdx.x == 0) {                       // RLCTR_GEMM_DBG: per-CTA (start, end, SM) behind the stage stamps
@@ -678,69 +553,33 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         const int tid = threadIdx.x;
         int stage = 0, dbg_it = 0;
         uint32_t phase = 0;
-        TileWalk w{cluster_id, 0, 0, 0, 0, 0};
+        TileWalk w{(int)blockIdx.x, 0, 0, 0, 0, 0};
         const bool colsum = g.colsum_part != nullptr && g.a_mn;
-        for (; tile_decode(w, g, total_tiles, rank); w.tile += n_clusters) {
+        for (; tile_decode(w, g, total_tiles); w.tile += (int)gridDim.x) {
             const bool sum_tile = colsum && w.nt == 0;     // every (split, m-tile) is met exactly once with nt == 0
-            float4 acc[BM / 32];
-#pragma unroll
-            for (int j = 0; j < BM / 32; ++j) acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
             float row_sum = 0.f;
             for (int kb = w.kb0; kb < w.kb1; ++kb) {
                 mbar_wait(smem_u32(&raw_bar[stage]), phase);
                 if (tid == 0) DBG_STAMP(dbg_it, 1);
                 if (tid == 96) DBG_STAMP(dbg_it, 12);
                 const uint32_t st = smem_u32(smem + (size_t)stage * stage_bytes);
-                if (g.a_tmem) {
-                    // this TMEM slot was last read by the MMAs of the previous round of this stage: they retired before the
-                    // producer refilled the stage (empty_bar), i.e. before raw_bar flipped
-                    tc_fence_after();
-                    const uint32_t ta = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(g.a_col0 + stage * 2 * BK);
-                    row_sum += split_row_to_tmem(st, g.a_mn != 0, tid, ta);
-                    if (!g.b_presplit) split_tile(st + a_bytes, st + a_bytes + b_bytes, b_bytes, tid);
-                    tc_fence_before();
-                } else {
-                    if (sum_tile) split_tile_colsum(st, st + A_TILE_BYTES, tid, acc);
-                    else split_tile(st, st + A_TILE_BYTES, A_TILE_BYTES, tid);
-                    if (!g.b_presplit) split_tile(st + a_bytes, st + a_bytes + b_bytes, b_bytes, tid);
-                }
-                if (!(g.a_tmem && g.b_presplit)) fence_proxy_async();   // generic-proxy smem stores -> visible to the tensor core
+                // this TMEM slot was last read by the MMAs of the previous round of this stage: they retired before the
+                // producer refilled the stage (empty_bar), i.e. before raw_bar flipped
+                tc_fence_after();
+                const uint32_t ta = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(g.a_col0 + stage * 2 * BK);
+                row_sum += split_row_to_tmem(st, g.a_mn != 0, tid, ta);
+                if (!g.b_presplit) split_tile(st + A_TILE_BYTES, st + A_TILE_BYTES + b_bytes, b_bytes, tid);
+                tc_fence_before();
+                if (!g.b_presplit) fence_proxy_async();       // generic-proxy smem stores -> visible to the tensor core
                 if (tid == 0) DBG_STAMP(dbg_it, 2);
                 if (tid == 96) DBG_STAMP(dbg_it, 11);
                 ++dbg_it;
-                if (PAIR && rank != 0) mbar_arrive_remote(smem_u32(&full_bar[stage]), 0);      // the leader issues the MMAs of the pair
-                else mbar_arrive(smem_u32(&full_bar[stage]));
+                mbar_arrive(smem_u32(&full_bar[stage]));
                 if (++stage == g.stages) { stage = 0; phase ^= 1; }
             }
-            if (sum_tile && g.a_tmem) {
+            if (sum_tile) {
                 const int m = w.mt * BM + tid;             // thread t owns row m: its k-sum IS the partial column sum
                 if (m < g.M) g.colsum_part[(int64_t)w.split * g.M + m] = row_sum;
-            } else if (sum_tile) {
-                // 16 threads hold partial sums of the same columns: 4 lanes of every warp (the k-row residues r = 0..3,
-                // at lane r*8 + (((lc ^ r) << 1) | half)), times 4 warps.  Butterfly over r, then a fixed-order sum over
-                // the warps through shared memory (the bias staging area: wgrad has no bias).
-                const int r = (tid >> 3) & 3, half = tid & 1, lc = ((tid & 7) >> 1) ^ r, wq = tid >> 5;
-#pragma unroll
-                for (int step = 1; step <= 2; step <<= 1) {
-                    const int rp = r ^ step;
-                    const int src = rp * 8 + (((lc ^ rp) << 1) | half);
-#pragma unroll
-                    for (int j = 0; j < BM / 32; ++j) {
-                        acc[j].x += __shfl_sync(RLCTR_FULL, acc[j].x, src);
-                        acc[j].y += __shfl_sync(RLCTR_FULL, acc[j].y, src);
-                        acc[j].z += __shfl_sync(RLCTR_FULL, acc[j].z, src);
-                        acc[j].w += __shfl_sync(RLCTR_FULL, acc[j].w, src);
-                    }
-                }
-                asm volatile("bar.sync 1, %0;" ::"n"(CONV_WARPS * 32) : "memory");      // previous tile's readers are done
-                if (r == 0) {
-#pragma unroll
-                    for (int j = 0; j < BM / 32; ++j)
-                        *reinterpret_cast<float4*>(&s_bias[wq * BM + j * 32 + lc * 8 + half * 4]) = acc[j];
-                }
-                asm volatile("bar.sync 1, %0;" ::"n"(CONV_WARPS * 32) : "memory");
-                const int m = w.mt * BM + tid;
-                if (m < g.M) g.colsum_part[(int64_t)w.split * g.M + m] = s_bias[tid] + s_bias[BM + tid] + s_bias[2 * BM + tid] + s_bias[3 * BM + tid];
             }
         }
     } else if (warp == PRODUCER_WARP) {
@@ -749,38 +588,16 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         uint32_t phase = 0;
         const uint32_t tx = A_TILE_BYTES + (g.b_presplit ? 2 * b_bytes : b_bytes);
         int dbg_it = 0;
-        // The streamed A operand comes from DRAM (1-2 us under load) while a stage can only be requested once its slot is free;
-        // with 3 slots that latency sits on the critical path.  So the A boxes are pulled into L2 `g.l2_ahead` stages ahead of
-        // their real request (the weights are L2-resident anyway).
-        TileWalk pw{cluster_id, 0, 0, 0, 0, 0};
-        bool pw_ok = g.l2_ahead > 0 && tile_decode(pw, g, total_tiles, rank);
-        int pkb = pw.kb0;
-        auto prefetch_next = [&]() {
-            if (!pw_ok) return;
-            if (pkb < pw.kb1) {
-                const int pm0 = pw.mt * BM, pk0 = pkb * BK;
-                if (g.a_mn) { for (int j = 0; j < BM / 32; ++j) tma_prefetch_l2_2d(&mapA, pm0 + 32 * j, pk0); }
-                else tma_prefetch_l2_2d(&mapA, pk0, pm0);
-            }
-            if (++pkb >= pw.kb1) {
-                pw.tile += n_clusters;
-                pw_ok = tile_decode(pw, g, total_tiles, rank);
-                pkb = pw.kb0;
-            }
-        };
-        if (lane == 0)
-            for (int i = 0; i < g.l2_ahead; ++i) prefetch_next();
-        TileWalk w{cluster_id, 0, 0, 0, 0, 0};
-        for (; tile_decode(w, g, total_tiles, rank); w.tile += n_clusters) {
+        TileWalk w{(int)blockIdx.x, 0, 0, 0, 0, 0};
+        for (; tile_decode(w, g, total_tiles); w.tile += (int)gridDim.x) {
             const int m0 = w.mt * BM, n0 = w.nt * g.n_tile;
             for (int kb = w.kb0; kb < w.kb1; ++kb) {
-                if (lane == 0) prefetch_next();
                 mbar_wait(smem_u32(&empty_bar[stage]), phase ^ 1);
                 if (lane == 0) {
                     DBG_STAMP(dbg_it, 0);
                     const uint32_t bar = smem_u32(&raw_bar[stage]);
                     const uint32_t sa = smem_u32(smem + (size_t)stage * stage_bytes);
-                    const uint32_t sb = sa + a_bytes;
+                    const uint32_t sb = sa + A_TILE_BYTES;
                     const int k0 = kb * BK;
                     mbar_expect_tx(bar, tx);
                     if (g.a_mn) {
@@ -788,26 +605,7 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
                     } else {
                         tma_load_2d(sa, &mapA, k0, m0, bar);
                     }
-                    if (PAIR) {
-                        // K-major pre-split B: this CTA stages rows [rank * n_tile/2, (rank + 1) * n_tile/2) of the tile (box = half)
-                        const int rows = g.n_tile / 2;
-                        tma_load_2d(sb, &mapB, k0, n0 + rank * rows, bar);
-                        tma_load_2d(sb + b_bytes, &mapBlo, k0, n0 + rank * rows, bar);
-                    } else if (g.cluster > 1) {
-                        // this CTA fetches its share of the B tile and multicasts it to the whole cluster; the peers' shares land
-                        // here the same way (raw_bar counts the bytes of the full tile either way)
-                        if (g.b_mn) {
-                            for (int j = rank; j < g.n_tile / 32; j += g.cluster) {
-                                tma_load_2d_mc(sb + j * 4096, &mapB, n0 + 32 * j, k0, bar, cmask);
-                                if (g.b_presplit) tma_load_2d_mc(sb + b_bytes + j * 4096, &mapBlo, n0 + 32 * j, k0, bar, cmask);
-                            }
-                        } else {
-                            const int rows = g.n_tile / g.cluster;                   // box rows of mapB (a multiple of 8)
-                            const uint32_t off = (uint32_t)(rank * rows) * 128u;
-                            tma_load_2d_mc(sb + off, &mapB, k0, n0 + rank * rows, bar, cmask);
-                            if (g.b_presplit) tma_load_2d_mc(sb + b_bytes + off, &mapBlo, k0, n0 + rank * rows, bar, cmask);
-                        }
-                    } else if (g.b_mn) {
+                    if (g.b_mn) {
                         for (int j = 0; j < g.n_tile / 32; ++j) {
                             tma_load_2d(sb + j * 4096, &mapB, n0 + 32 * j, k0, bar);
                             if (g.b_presplit) tma_load_2d(sb + b_bytes + j * 4096, &mapBlo, n0 + 32 * j, k0, bar);
@@ -825,90 +623,54 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
     } else if (warp == MMA_WARP) {
         // ================= MMA issuer =================
         // instruction descriptor (cute::UMMA::InstrDescriptor): D = f32, A = B = tf32, M = 128, N = n_tile,
-        // bit 15 / 16 = A / B is MN-major
-        const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)((g.a_mn && !g.a_tmem) ? 1 : 0) << 15) |
-                               ((uint32_t)(g.b_mn ? 1 : 0) << 16) | ((uint32_t)(g.n_tile >> 3) << 17) |
-                               ((uint32_t)((PAIR ? 2 * BM : BM) >> 4) << 24);          // pair: M = 256 over the two CTAs
-        const uint32_t a_step = g.a_mn ? 1024u : (uint32_t)UK * 4u;      // bytes per MMA along K
-        const uint32_t b_step = g.b_mn ? 1024u : (uint32_t)UK * 4u;
+        // bit 15 / 16 = A / B is MN-major (A comes from TMEM: always K-major)
+        const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(g.b_mn ? 1 : 0) << 16) |
+                               ((uint32_t)(g.n_tile >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+        const uint32_t b_step = g.b_mn ? 1024u : (uint32_t)UK * 4u;      // bytes per MMA along K
         int stage = 0;
         uint32_t phase = 0;
         int acc = 0, dbg_it = 0;
         uint32_t acc_phase = 0;
-        TileWalk w{cluster_id, 0, 0, 0, 0, 0};
-        if (PAIR && rank != 0) w.tile = total_tiles;                      // the leader CTA issues for the pair
-        for (; tile_decode(w, g, total_tiles, rank); w.tile += n_clusters) {
+        TileWalk w{(int)blockIdx.x, 0, 0, 0, 0, 0};
+        for (; tile_decode(w, g, total_tiles); w.tile += (int)gridDim.x) {
             if (lane == 0) DBG_STAMP(dbg_it, 5);
-            if (PAIR) mbar_wait_cluster(smem_u32(&tmem_empty_bar[acc]), acc_phase ^ 1);     // BOTH CTAs' epilogues drained it
-            else mbar_wait(smem_u32(&tmem_empty_bar[acc]), acc_phase ^ 1);  // epilogue drained this accumulator
+            mbar_wait(smem_u32(&tmem_empty_bar[acc]), acc_phase ^ 1);  // epilogue drained this accumulator
             if (lane == 0) DBG_STAMP(dbg_it, 6);
             tc_fence_after();
             const uint32_t d_tmem = tmem_base + (uint32_t)(acc * g.acc_stride);
             for (int kb = w.kb0; kb < w.kb1; ++kb) {
                 mbar_wait(smem_u32(&raw_bar[stage]), phase);                 // TMA bytes (the pre-split B tiles) landed
                 if (lane == 0) DBG_STAMP(dbg_it, 8);
-                if (PAIR) mbar_wait_cluster(smem_u32(&full_bar[stage]), phase);    // both CTAs' converters (hence both halves of B)
-                else mbar_wait(smem_u32(&full_bar[stage]), phase);           // converters done
+                mbar_wait(smem_u32(&full_bar[stage]), phase);                // converters done
                 if (lane == 0) DBG_STAMP(dbg_it, 9);
                 tc_fence_after();
                 if (lane == 0) DBG_STAMP(dbg_it, 3);
                 if (lane == 0) {
-                    const uint32_t sa = smem_u32(smem + (size_t)stage * stage_bytes);
-                    const uint32_t a_hi = sa, a_lo = sa + A_TILE_BYTES, b_hi = sa + a_bytes, b_lo = b_hi + b_bytes;
+                    const uint32_t b_hi = smem_u32(smem + (size_t)stage * stage_bytes) + A_TILE_BYTES, b_lo = b_hi + b_bytes;
+                    const uint32_t ta_hi = tmem_base + (uint32_t)(g.a_col0 + stage * 2 * BK), ta_lo = ta_hi + (uint32_t)BK;
                     // the last k-block of a K that is no multiple of 32 is zero-filled by TMA: its all-zero k-steps are not issued
                     const int ksteps = min(BK / UK, (g.K - kb * BK + UK - 1) / UK);
-                    if (g.a_tmem) {
-                        const uint32_t ta_hi = tmem_base + (uint32_t)(g.a_col0 + stage * 2 * BK), ta_lo = ta_hi + (uint32_t)BK;
-#pragma unroll
-                        for (int k = 0; k < BK / UK; ++k) {
-                            if (k >= ksteps) break;
-                            const uint32_t bo = (uint32_t)k * b_step;
-                            const uint64_t dbh = g.b_mn ? desc_mn_major(b_hi + bo) : desc_k_major(b_hi + bo);
-                            const uint64_t dbl = g.b_mn ? desc_mn_major(b_lo + bo) : desc_k_major(b_lo + bo);
-                            const uint32_t first = (kb > w.kb0 || k > 0) ? 1u : 0u;
-                            if (PAIR) {
-                                umma_tf32_ts2(d_tmem, ta_lo + (uint32_t)(k * UK), dbh, idesc, first);
-                                umma_tf32_ts2(d_tmem, ta_hi + (uint32_t)(k * UK), dbl, idesc, 1u);
-                                umma_tf32_ts2(d_tmem, ta_hi + (uint32_t)(k * UK), dbh, idesc, 1u);
-                            } else {
-                                umma_tf32_ts(d_tmem, ta_lo + (uint32_t)(k * UK), dbh, idesc, first);
-                                umma_tf32_ts(d_tmem, ta_hi + (uint32_t)(k * UK), dbl, idesc, 1u);
-                                umma_tf32_ts(d_tmem, ta_hi + (uint32_t)(k * UK), dbh, idesc, 1u);
-                            }
-                        }
-                    } else
 #pragma unroll
                     for (int k = 0; k < BK / UK; ++k) {
                         if (k >= ksteps) break;
-                        const uint32_t ao = (uint32_t)k * a_step, bo = (uint32_t)k * b_step;
-                        const uint64_t dah = g.a_mn ? desc_mn_major(a_hi + ao) : desc_k_major(a_hi + ao);
-                        const uint64_t dal = g.a_mn ? desc_mn_major(a_lo + ao) : desc_k_major(a_lo + ao);
+                        const uint32_t bo = (uint32_t)k * b_step;
                         const uint64_t dbh = g.b_mn ? desc_mn_major(b_hi + bo) : desc_k_major(b_hi + bo);
                         const uint64_t dbl = g.b_mn ? desc_mn_major(b_lo + bo) : desc_k_major(b_lo + bo);
                         const uint32_t first = (kb > w.kb0 || k > 0) ? 1u : 0u;
-                        umma_tf32(d_tmem, dal, dbh, idesc, first);
-                        umma_tf32(d_tmem, dah, dbl, idesc, 1u);
-                        umma_tf32(d_tmem, dah, dbh, idesc, 1u);
+                        umma_tf32_ts(d_tmem, ta_lo + (uint32_t)(k * UK), dbh, idesc, first);
+                        umma_tf32_ts(d_tmem, ta_hi + (uint32_t)(k * UK), dbl, idesc, 1u);
+                        umma_tf32_ts(d_tmem, ta_hi + (uint32_t)(k * UK), dbh, idesc, 1u);
                     }
                     DBG_STAMP(dbg_it, 10);
-                    if (PAIR) {                                            // both CTAs' slots / accumulators, one arrival each
-                        umma_commit2_mc(smem_u32(&empty_bar[stage]), cmask);
-                        if (kb == w.kb1 - 1) umma_commit2_mc(smem_u32(&tmem_full_bar[acc]), cmask);
-                    } else {
-                        if (g.cluster > 1) umma_commit_mc(smem_u32(&empty_bar[stage]), cmask);   // ... in every CTA that writes into it
-                        else umma_commit(smem_u32(&empty_bar[stage]));       // frees the smem slot when these MMAs retire
-                        if (kb == w.kb1 - 1) umma_commit(smem_u32(&tmem_full_bar[acc]));
-                    }
+                    umma_commit(smem_u32(&empty_bar[stage]));                // frees the smem slot when these MMAs retire
+                    if (kb == w.kb1 - 1) umma_commit(smem_u32(&tmem_full_bar[acc]));
                     DBG_STAMP(dbg_it, 4);
                 }
                 ++dbg_it;
                 __syncwarp();
                 if (++stage == g.stages) { stage = 0; phase ^= 1; }
             }
-            if (w.kb1 <= w.kb0 && lane == 0) {                                                  // empty split
-                if (PAIR) umma_commit2_mc(smem_u32(&tmem_full_bar[acc]), cmask);
-                else umma_commit(smem_u32(&tmem_full_bar[acc]));
-            }
+            if (w.kb1 <= w.kb0 && lane == 0) umma_commit(smem_u32(&tmem_full_bar[acc]));     // empty split
             __syncwarp();
             if (++acc == 2) { acc = 0; acc_phase ^= 1; }
         }
@@ -921,12 +683,12 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         const uint32_t cstage = smem_u32(smem + (size_t)g.stages * stage_bytes) + (uint32_t)q * 8192u;   // 2 x 4 KB per warp
         uint32_t acc_phase = 0;
         uint32_t mphase = 0;
-        TileWalk w{cluster_id, 0, 0, 0, 0, 0};
-        for (; tile_decode(w, g, total_tiles, rank); w.tile += n_clusters) {
+        TileWalk w{(int)blockIdx.x, 0, 0, 0, 0, 0};
+        for (; tile_decode(w, g, total_tiles); w.tile += (int)gridDim.x) {
             const bool empty_split = w.kb1 <= w.kb0;
             // the previous tile's last chunk ended behind a __syncwarp: the block is free for this tile's first chunk
-            const uint32_t mbuf = (MASK && g.m_tma) ? cstage + (uint32_t)((EPI_WARPS - q) * 8192 + q * 4096) : 0u;   // behind the C staging blocks
-            if (MASK && mbuf && w.nt * g.n_tile < g.N && g.n_tile >= 32)
+            const uint32_t mbuf = MASK ? cstage + (uint32_t)((EPI_WARPS - q) * 8192 + q * 4096) : 0u;   // behind the C staging blocks
+            if (MASK && w.nt * g.n_tile < g.N && g.n_tile >= 32)
                 mask_request(&mapM, mbuf, smem_u32(&mask_bar[q]), w.nt * g.n_tile, w.mt * BM + q * 32, lane);
             mbar_wait(smem_u32(&tmem_full_bar[acc]), acc_phase);
             tc_fence_after();
@@ -958,8 +720,7 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
             tc_fence_before();
             if (warp == CONV_WARPS + 2 && lane == 0) DBG_STAMP(dbg_tile * (w.kb1 - w.kb0) + 1, 7);
             ++dbg_tile;
-            if (PAIR && rank != 0) mbar_arrive_remote(smem_u32(&tmem_empty_bar[acc]), 0);
-            else mbar_arrive(smem_u32(&tmem_empty_bar[acc]));
+            mbar_arrive(smem_u32(&tmem_empty_bar[acc]));
             if (++acc == 2) { acc = 0; acc_phase ^= 1; }
         }
         if (g.c_tma && lane == 0) bulk_wait_read<0>();      // the staging blocks must outlive the stores that read them
@@ -971,11 +732,7 @@ gemm3x_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now));
         g.dbg[4096 + 4 * blockIdx.x + 1] = (long long)now;
     }
-    if (g.cluster > 1) cluster_sync_all();                 // no CTA leaves while a peer may still signal its barriers
-    if (warp == MMA_WARP) {
-        if (PAIR) tmem_dealloc2(tmem_base, TMEM_COLS);
-        else tmem_dealloc(tmem_base, TMEM_COLS);
-    }
+    if (warp == MMA_WARP) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
 // (hi, lo) images of a weight matrix [rows, cols] -> [rows, pitch] (pitch % 4 == 0, zero padded): the B
@@ -1034,22 +791,27 @@ int enabled() {
     return env_int("RLCTR_GEMM_TMA", 1) != 0 && encode_fn() != nullptr;   // env read per call: tests switch paths
 }
 
-static int round_to(int n, int q) { return (n + q - 1) / q * q; }
+static constexpr int round_to(int n, int q) { return (n + q - 1) / q * q; }
+
+// Tile-width cap: a 160-column tile leaves three 56 KB stages in shared memory and three (A_hi | A_lo) stages in tensor memory;
+// 128 measured slower (profiles/r2p_gemm_probes.md).
+constexpr int NT_MAX = 160;
+static_assert(NT_MAX % 32 == 0 && NT_MAX <= 256, "every tile width make_plan picks must be a UMMA N for both operand majors");
+// A always lives in tensor memory, behind the two accumulator stages: the widest tile must leave it room for two stages
+static_assert((TMEM_COLS - 2 * round_to(NT_MAX, 32)) / (2 * BK) >= 2, "a full-width tile must leave two TMEM stages of A");
 
 struct Plan {
     int n_tile, n_tiles, m_tiles, splits, kb_per_split, stages;
-    int a_tmem, acc_stride, a_col0, c_tma, cluster, pair;
+    int acc_stride, a_col0, c_tma;
     size_t smem;
 };
 constexpr size_t C_STAGE_BYTES = (size_t)EPI_WARPS * 2 * 4096;     // two 32 x 32 fp32 blocks per epilogue warp
 constexpr size_t M_STAGE_BYTES = (size_t)EPI_WARPS * 4096;         // one 32 x 32 mask block per epilogue warp (dgrad, behind C's)
-static Plan make_plan(int M, int N, int K, bool b_mn, bool allow_split, bool c_tma_ok = false, bool b_presplit = false) {
+static Plan make_plan(int M, int N, int K, bool b_mn, bool allow_split, bool c_tma_ok = false) {
     Plan p;
-    const int nt_max = env_int("RLCTR_GEMM_NT_MAX", 160);           // <= 160 keeps three 72 KB stages in flight
     const int q = b_mn ? 32 : 16;
-    p.n_tiles = (N + nt_max - 1) / nt_max;
+    p.n_tiles = (N + NT_MAX - 1) / NT_MAX;
     p.n_tile = round_to((N + p.n_tiles - 1) / p.n_tiles, q);
-    if (p.n_tile > 256) { p.n_tile = 256; p.n_tiles = (N + 255) / 256; }
     p.m_tiles = (M + BM - 1) / BM;
     const int kb_total = (K + BK - 1) / BK;
     p.splits = 1;
@@ -1065,34 +827,20 @@ static Plan make_plan(int M, int N, int K, bool b_mn, bool allow_split, bool c_t
     if (p.kb_per_split < 1) p.kb_per_split = 1;
     p.splits = (kb_total + p.kb_per_split - 1) / p.kb_per_split;
     if (p.splits < 1) p.splits = 1;
-    // A in tensor memory: the accumulator stages shrink to the tile width and the rest of the 512 columns holds up to
-    // (512 - 2 * acc_stride) / 64 stages of (A_hi | A_lo); shared memory then carries only the raw A tile and B
+    // tensor memory: two accumulator stages of the tile width, then (512 - 2 * acc_stride) / 64 stages of (A_hi | A_lo);
+    // shared memory carries the raw A tile and B (hi, lo) per stage
     p.acc_stride = round_to(p.n_tile, 32);
     p.a_col0 = 2 * p.acc_stride;
     const int tmem_stages = (TMEM_COLS - p.a_col0) / (2 * BK);
-    p.a_tmem = (env_int("RLCTR_GEMM_A_TMEM", 1) != 0 && tmem_stages >= 2) ? 1 : 0;
-    if (!p.a_tmem) { p.acc_stride = 256; p.a_col0 = 0; }
-    // cta_group::2 (RLCTR_GEMM_PAIR=1): forward-type GEMMs (K-major pre-split B, A in tensor memory, no split-K) whose tile width
-    // the 2-CTA MMA accepts; each CTA then stages half of the B tile
-    p.pair = (env_int("RLCTR_GEMM_PAIR", 0) != 0 && p.a_tmem && b_presplit && !b_mn && p.splits == 1 && p.m_tiles >= 2 &&
-              p.n_tile % 32 == 0) ? 1 : 0;
-    const size_t stage_bytes = (p.a_tmem ? 1 : 2) * (size_t)A_TILE_BYTES + 2 * (size_t)p.n_tile * (p.pair ? 64 : 128);
+    const size_t stage_bytes = (size_t)A_TILE_BYTES + 2 * (size_t)p.n_tile * 128;
     int st = (int)((size_t)(220 * 1024) / stage_bytes);
     if (st > MAX_STAGES) st = MAX_STAGES;
-    if (p.a_tmem && st > tmem_stages) st = tmem_stages;
-    if (st < 1) st = 1;
+    if (st > tmem_stages) st = tmem_stages;
     p.stages = st;
     // TMA-stored C: only when the staging blocks fit beside the pipeline without costing it a stage, and never for split-K
     // partials (a box clipped at the tensor bound, not at the split's M rows, would spill into the next split)
-    p.c_tma = (c_tma_ok && p.splits == 1 && env_int("RLCTR_GEMM_C_TMA", 1) != 0 &&
-               stage_bytes * st + C_STAGE_BYTES <= (size_t)(220 * 1024)) ? 1 : 0;
+    p.c_tma = (c_tma_ok && p.splits == 1 && stage_bytes * st + C_STAGE_BYTES <= (size_t)(220 * 1024)) ? 1 : 0;
     p.smem = stage_bytes * st + (p.c_tma ? C_STAGE_BYTES : 0) + 1024;
-    // CTA pairs sharing every B tile by TMA multicast (RLCTR_GEMM_CLUSTER=2; needs two m-tiles to pair and a B tile that halves on
-    // a swizzle-atom boundary).  Off by default: measured no gain -- the kernel is bound by the shared-memory port of each SM, and a
-    // multicast tile is still written into (and read by the MMAs from) every CTA's own shared memory.
-    p.cluster = p.pair ? 2 : 1;
-    if (!p.pair && env_int("RLCTR_GEMM_CLUSTER", 1) >= 2 && p.m_tiles >= 2 && (b_mn || p.n_tile % 16 == 0))
-        p.cluster = 2;
     return p;
 }
 int plan_splits(int M, int N, int K, bool b_mn) { return make_plan(M, N, K, b_mn, true).splits; }
@@ -1118,24 +866,22 @@ int gemm(const Operand& A, const Operand& B, float* C, int64_t ldc, const float*
     if (!enabled()) return RLCTR_EUNSUPPORTED;
     if (!tma_ok(A.ptr, A.pitch) || !tma_ok(B.ptr, B.pitch) || (B.lo && !tma_ok(B.lo, B.pitch))) return RLCTR_EUNSUPPORTED;
     if (A.lo) return RLCTR_EUNSUPPORTED;                  // the streamed operand is always converted in the kernel
-    const Plan p = make_plan(M, N, K, B.mn_major, allow_split, tma_ok(C, ldc), B.lo != nullptr);
-    if (p.n_tile > 256 || (B.mn_major && p.n_tile % 32 != 0)) return RLCTR_EUNSUPPORTED;
+    const Plan p = make_plan(M, N, K, B.mn_major, allow_split, tma_ok(C, ldc));
     CUtensorMap mA, mB, mBlo;
     // K-major operand [R rows][K]: dims {K, R}, box {32, tile rows}.  MN-major operand [K rows][R]: dims {R, K}, box {32, 32}.
     bool ok = A.mn_major ? make_map(&mA, A.ptr, M, K, A.pitch, 32, true) : make_map(&mA, A.ptr, K, M, A.pitch, BM);
-    const int b_box = p.n_tile / p.cluster;            // K-major B: each CTA of a cluster fetches 1/cluster of the tile's rows
-    ok = ok && (B.mn_major ? make_map(&mB, B.ptr, N, K, B.pitch, 32, true) : make_map(&mB, B.ptr, K, N, B.pitch, b_box));
-    if (B.lo) ok = ok && (B.mn_major ? make_map(&mBlo, B.lo, N, K, B.pitch, 32, true) : make_map(&mBlo, B.lo, K, N, B.pitch, b_box));
+    ok = ok && (B.mn_major ? make_map(&mB, B.ptr, N, K, B.pitch, 32, true) : make_map(&mB, B.ptr, K, N, B.pitch, p.n_tile));
+    if (B.lo) ok = ok && (B.mn_major ? make_map(&mBlo, B.lo, N, K, B.pitch, 32, true) : make_map(&mBlo, B.lo, K, N, B.pitch, p.n_tile));
     else mBlo = mB;
     CUtensorMap mC = mA, mM = mA;
     if (p.c_tma) ok = ok && make_map(&mC, C, N, M, ldc, 32);          // box {32 n, 32 m}, SWIZZLE_128B
     if (!ok) return RLCTR_EUNSUPPORTED;
     // the dgrad mask through TMA: beside TMA-stored C, when its blocks fit behind the pipeline and the mask rows are addressable
     size_t smem = p.smem;
-    int m_tma = 0;
+    bool m_tma = false;
     if (epi && epi->mask_src && p.c_tma && p.splits == 1 && tma_ok(epi->mask_src, epi->mask_ld) && p.smem + M_STAGE_BYTES <= (size_t)(221 * 1024) &&
-        env_int("RLCTR_GEMM_M_TMA", 1) != 0 && make_map(&mM, epi->mask_src, N, M, epi->mask_ld, 32)) {
-        m_tma = 1;
+        make_map(&mM, epi->mask_src, N, M, epi->mask_ld, 32)) {
+        m_tma = true;
         smem += M_STAGE_BYTES;
     }
     Args g;
@@ -1143,9 +889,7 @@ int gemm(const Operand& A, const Operand& B, float* C, int64_t ldc, const float*
     g.M = M; g.N = N; g.K = K;
     g.n_tile = p.n_tile; g.m_tiles = p.m_tiles; g.n_tiles = p.n_tiles; g.splits = p.splits; g.kb_per_split = p.kb_per_split;
     g.stages = p.stages;
-    g.a_tmem = p.a_tmem; g.acc_stride = p.acc_stride; g.a_col0 = p.a_col0; g.c_tma = p.c_tma; g.m_tma = m_tma;
-    g.cluster = p.cluster; g.pair = p.pair;
-    g.l2_ahead = env_int("RLCTR_GEMM_L2_AHEAD", 0);     // measured: no gain (the pipeline is L2->SM bandwidth bound, not DRAM-latency bound)
+    g.acc_stride = p.acc_stride; g.a_col0 = p.a_col0; g.c_tma = p.c_tma;
     g.a_mn = A.mn_major ? 1 : 0; g.b_mn = B.mn_major ? 1 : 0; g.b_presplit = B.lo ? 1 : 0; g.relu = relu;
     g.colsum_part = (colsum_part && A.mn_major && !bias) ? colsum_part : nullptr;
     if (colsum_part && !g.colsum_part) return RLCTR_EUNSUPPORTED;
@@ -1156,39 +900,10 @@ int gemm(const Operand& A, const Operand& B, float* C, int64_t ldc, const float*
     g.epi = epi ? *epi : Epilogue{};
     if ((g.epi.drop_state || g.epi.mask_src) && p.splits != 1) return RLCTR_EUNSUPPORTED;
     if (g.epi.mask_src) g.epi.mvec = vec_of(g.epi.mask_src, g.epi.mask_ld);
-    if (p.pair) RLCTR_CUDA(cudaFuncSetAttribute(gemm3x_tma_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    else if (m_tma) RLCTR_CUDA(cudaFuncSetAttribute(gemm3x_tma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    else RLCTR_CUDA(cudaFuncSetAttribute(gemm3x_tma_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int total = ((p.m_tiles + p.cluster - 1) / p.cluster) * p.n_tiles * p.splits;      // cluster tiles
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(RLCTR_SMS / p.cluster * p.cluster));
-    cfg.blockDim = dim3(THREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)p.cluster;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    int max_clusters = RLCTR_SMS / p.cluster;
-    if (p.cluster > 1) {                                   // clusters that can be resident at once (GPCs with an odd SM count lose one)
-        static int cached_smem = -1, cached = 0;
-        if (cached_smem != (int)smem * 2 + p.pair) {
-            int n = 0;
-            if ((p.pair ? cudaOccupancyMaxActiveClusters(&n, gemm3x_tma_kernel<true, false>, &cfg)
-                        : cudaOccupancyMaxActiveClusters(&n, gemm3x_tma_kernel<false, false>, &cfg)) == cudaSuccess && n > 0) cached = n;
-            else cached = RLCTR_SMS / p.cluster;
-            cached_smem = (int)smem * 2 + p.pair;
-        }
-        if (cached < max_clusters) max_clusters = cached;
-    }
-    const int grid = (total < max_clusters ? total : max_clusters) * p.cluster;
-    cfg.gridDim = dim3((unsigned)grid);
-    if (p.pair) RLCTR_CUDA(cudaLaunchKernelEx(&cfg, gemm3x_tma_kernel<true, false>, mA, mB, mBlo, mC, mM, g));
-    else if (m_tma) RLCTR_CUDA(cudaLaunchKernelEx(&cfg, gemm3x_tma_kernel<false, true>, mA, mB, mBlo, mC, mM, g));
-    else RLCTR_CUDA(cudaLaunchKernelEx(&cfg, gemm3x_tma_kernel<false, false>, mA, mB, mBlo, mC, mM, g));
+    const auto kernel = m_tma ? gemm3x_tma_kernel<true> : gemm3x_tma_kernel<false>;
+    RLCTR_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int total = p.m_tiles * p.n_tiles * p.splits;    // persistent CTAs, one per SM
+    kernel<<<total < RLCTR_SMS ? total : RLCTR_SMS, THREADS, smem, st>>>(mA, mB, mBlo, mC, mM, g);
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
 }
