@@ -345,14 +345,19 @@ int rlctr_rows_adam(const uint32_t* sorted_ids, const uint32_t* sorted_slots, in
  *     [ p: member columns .. | stamp ]  [ exp_avg ]  [ exp_avg_sq ]      three blocks, `block` floats apart
  * A random HBM access costs the same whether it returns 4 or 128 bytes (profiles/r2_rowprobe.md), so the gather of LR + FM +
  * DeepFM (4 + 44 + 44 bytes) is ONE 128-byte line instead of three, and the optimizer touches three lines per id instead of
- * seven.  The joint table is an ordinary rlctr_table (row_stride = active floats rounded to 4, <= 32; lin_col = -1, emb_col = 0,
- * dim = used columns; rlctr_adam.exp_avg / exp_avg_sq = data + block / + 2*block, stamp_col = the first unused column), so
- * rlctr_rows_catchup / rlctr_adam_flush serve it unchanged; the two calls below are its forward and its update.
+ * seven.  The joint table is an ordinary rlctr_table (row_stride = active floats rounded to 4, <= RLCTR_GROUP_MAX_FLOATS;
+ * lin_col = -1, emb_col = 0, dim = used columns; rlctr_adam.exp_avg / exp_avg_sq = data + block / + 2*block, stamp_col = the first
+ * unused column), so rlctr_rows_catchup / rlctr_adam_flush serve it unchanged; the two calls below are its forward and its update.
+ * A record whose row fits one 128-byte line keeps each block in its own line (block 32, pitch 96).  A wider row (up to four
+ * lines, 128 floats) is packed [p | exp_avg | exp_avg_sq] with block = row_stride and the pitch rounded up to whole lines.
+ * Past RLCTR_GROUP_MAX_FLOATS the calls below, rlctr_rows_catchup and rlctr_adam_flush return RLCTR_EUNSUPPORTED for a joint
+ * table with an in-record stamp.
  * A member is one model's view of the record: the columns it owns, where its outputs go, where its gradient side comes from.
  * Members with an FM term keep the chunk alignment of their stand-alone row (emb_col % 4 as in the stand-alone table): their
  * logits and updates are then bit-identical to the stand-alone kernels'.
  * ------------------------------------------------------------------------------------ */
 #define RLCTR_GROUP_MAX 4
+#define RLCTR_GROUP_MAX_FLOATS 128      /* joint row: four 128-byte lines */
 typedef struct rlctr_member {
     int32_t      lin_col;      /* column of the first-order weight in the joint row, -1 = none */
     int32_t      emb_col;      /* first latent column */

@@ -172,6 +172,10 @@ SHAPE_LIMITS = {
     "rlctr_cross_fwd": "DCN: F*D <= 512, at most 8 cross layers",
     "rlctr_cross_bwd": "DCN: F*D <= 512, at most 6 cross layers",
     "rlctr_rows_adam": "fused rows of at most 512 floats (FFM: F*D + 1 <= 512)",
+    "rlctr_group_fwd": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats",
+    "rlctr_group_rows_adam": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats",
+    "rlctr_rows_catchup": "records with an in-record stamp: rows of at most 128 floats",
+    "rlctr_adam_flush": "records with an in-record stamp: rows of at most 128 floats",
 }
 
 

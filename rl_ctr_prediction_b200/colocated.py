@@ -111,17 +111,26 @@ def loss_head(m, logit, rows, y, loss, ws, dl=None, scale=1.0):
     return dl, grad
 
 
-def _layout(members):
+MAX_LINES = 4                          # a joint row spans at most four 128-byte lines (rlctr.h RLCTR_GROUP_MAX_FLOATS)
+
+
+def _layout(members, max_lines=1):
     """Columns of the joint row.  Vector members (FM-type rows: [w, v_0 .. v_{D-1}]) take consecutive 16-byte aligned blocks
-    with their stand-alone layout; scalar members (LR) fill the padding columns those blocks leave, else open a new chunk.
-    Returns ([(lin_col, emb_col, dim)] per member, used columns)."""
+    with their stand-alone layout; scalar members (LR) fill the padding columns those blocks leave, else open a new chunk.  The
+    row, with the stamp in the last active chunk, must fit ``max_lines`` 128-byte lines (1..4); a one-line record holds only
+    members whose stand-alone rows are at most 16 floats.  Returns ([(lin_col, emb_col, dim)] per member, used columns)."""
+    if not 1 <= max_lines <= MAX_LINES:
+        raise ValueError(f"max_lines must be 1..{MAX_LINES} (128-byte lines per joint row), got {max_lines}")
     cols, taken, nxt = [None] * len(members), set(), 0
     for i, m in enumerate(members):
         g = m._geom
         if g.row_stride == 1:
             continue
-        if g.row_stride > 16:
-            raise _lib.RlctrError(f"{type(m).__name__}: rows wider than 16 floats (FFM) cannot be co-located")
+        if g.lin_col > g.emb_col or g.row_stride > 36:
+            raise _lib.RlctrError(f"{type(m).__name__}: FFM rows (F field-aware blocks) cannot be co-located")
+        if g.row_stride > 16 and max_lines == 1:
+            raise _lib.RlctrError(f"{type(m).__name__}: rows of {g.row_stride} floats do not fit the one-line record (32 floats) "
+                                  "beside the stamp of members with rows of at most 16 floats; pass max_lines=2..4 for a wider record")
         lin = nxt + g.lin_col if g.lin_col >= 0 else -1
         cols[i] = (lin, nxt + g.emb_col, g.dim)
         for c in ([lin] if lin >= 0 else []) + list(range(nxt + g.emb_col, nxt + g.emb_col + g.dim)):
@@ -139,9 +148,42 @@ def _layout(members):
     used = max(taken) + 1
     if used % 4 == 0:
         used += 1                       # the stamp needs a padding column in the last active chunk: open one
-    if round4(used + 1) > 32:
-        raise _lib.RlctrError("co-located record wider than 32 floats (one 128-byte line): too many members")
+    rs = round4(used + 1)
+    if rs > 32 * max_lines:
+        need = (rs + 31) // 32
+        hint = f"; pass max_lines={need}" if need <= MAX_LINES else f" (at most {MAX_LINES} lines, {32 * MAX_LINES} floats)"
+        raise _lib.RlctrError(f"co-located record of {rs} floats wider than {32 * max_lines} floats "
+                              f"({'one 128-byte line' if max_lines == 1 else f'{max_lines} 128-byte lines'}): too many members{hint}")
     return cols, used
+
+
+def _wide(members, used):
+    """The record needs the wide kernels: more than one line, or a member whose stand-alone row is wider than 16 floats."""
+    return round4(used + 1) > 32 or any(m._geom.row_stride > 16 for m in members)
+
+
+def _record(n_rows, used):
+    """Geometry of the joint record over ``used`` columns (stamp at ``used``).  One line: [p | exp_avg | exp_avg_sq] each in its own
+    128-byte line (block 32, pitch 96).  Wider: the three blocks packed (block = row_stride), the pitch rounded up to whole lines,
+    so every record and its p block start on a line: fewer lines per record than line-aligned blocks (DESIGN §6b)."""
+    rs = round4(used + 1)
+    if rs <= 32:
+        return Geometry(n_rows, rs, -1, 0, used, pitch=96, block=32, stamp_at=used)
+    return Geometry(n_rows, rs, -1, 0, used, pitch=(3 * rs + 31) // 32 * 32, block=rs, stamp_at=used)
+
+
+def _member_view(m, rec, col, wide):
+    """Member ``m``'s view of the joint record ``rec`` at columns ``col`` = (lin, emb, dim).  One-line records keep the joint row
+    (the one-line gather serves it); a wide record gives each member its stand-alone row -- from its first chunk, its own
+    row_stride, the joint pitch -- so that its own forward, state_dict and load_state_dict work on rows of at most 36 floats."""
+    lin, emb, dim = col
+    if not wide:
+        return Geometry(rec.n_rows, rec.row_stride, lin, emb, dim, pitch=rec.row_pitch, block=rec.block_floats)
+    if dim == 0:                                             # LR: its one column
+        return Geometry(rec.n_rows, 1, 0, 0, 0, pitch=rec.row_pitch, block=rec.block_floats, offset=lin)
+    base = (emb if lin < 0 else min(lin, emb)) // 4 * 4
+    return Geometry(rec.n_rows, m._geom.row_stride, lin - base if lin >= 0 else -1, emb - base, dim, pitch=rec.row_pitch,
+                    block=rec.block_floats, offset=base)
 
 
 class _GroupStep:
@@ -236,7 +278,7 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
     _kind = "group"
     _UPDATE_KEY = "rlctr_group_rows_adam"
 
-    def __init__(self, models):
+    def __init__(self, models, max_lines=1):
         super().__init__()
         models = list(models)
         if not 1 <= len(models) <= _lib.RLCTR_GROUP_MAX:
@@ -254,10 +296,10 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
         if dev.type != "cuda":
             raise _lib.RlctrError("move the models to the CUDA device before co-locating them")
         self.feature_nums = n_rows.pop()
-        cols, used = _layout(models)
-        rs = round4(used + 1)
-        self._geom = Geometry(self.feature_nums, rs, -1, 0, used, pitch=96, block=32, stamp_at=used)
-        joint = torch.zeros(self.feature_nums, 96, dtype=torch.float32, device=dev)
+        cols, used = _layout(models, max_lines)
+        self._geom = _record(self.feature_nums, used)
+        wide = _wide(models, used)
+        joint = torch.zeros(self.feature_nums, self._geom.row_pitch, dtype=torch.float32, device=dev)
         with torch.no_grad():
             for m, (lin, emb, dim) in zip(models, cols):
                 m.flush()                                    # settle what a previous optimizer still owes the stand-alone table
@@ -270,10 +312,10 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
         self.table._rlctr_owner = self
         self._opt, self._stash, self._ws = None, None, {}
         self._sort_stream, self._claim = None, None
-        self._cols = cols
-        for m, (lin, emb, dim) in zip(models, cols):
+        self._cols, self._max_lines = cols, max_lines
+        for m, col in zip(models, cols):
             m.table = self.table                             # shared Parameter: the member's view of the joint record
-            m._geom = Geometry(self.feature_nums, rs, lin, emb, dim, pitch=96, block=32)
+            m._geom = _member_view(m, self._geom, col, wide)
             m._opt, m._stash = None, None
             m.__dict__["_group"] = self                      # not a sub-module of the member: no cycle in parameters()
         self.members = nn.ModuleList(models)
@@ -327,7 +369,7 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
         # order (rlctr_rows_catchup_ids: a claim bit per row tells the occurrences of an id apart) the sort runs on its own
         # stream -- a parallel branch of a captured step -- beside catch-up, gather and tower instead of in front of them.
         side = None
-        if UNSORTED_CATCHUP and opt.lazy and opt.stamp_col >= 0 and (g.used + 3) // 4 >= 5:    # joint records of 5..8 chunks
+        if UNSORTED_CATCHUP and opt.lazy and opt.stamp_col >= 0 and 5 <= (g.used + 3) // 4 <= 8:    # joint records of 5..8 chunks
             cur = torch.cuda.current_stream(dev)
             side = self._sort_stream
             if side is None or side.device != dev:
@@ -361,5 +403,8 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
         return losses
 
 
-def colocate(models) -> ColocatedCTR:
-    return ColocatedCTR(models)
+def colocate(models, max_lines=1) -> ColocatedCTR:
+    """One joint record per id for ``models`` (``MEMBER_KINDS``, up to RLCTR_GROUP_MAX, same vocabulary and device).  The record
+    takes the fewest 128-byte lines that hold the members' columns, up to ``max_lines`` (1..4).  The default, one line, is the
+    measured layout; a group that needs more lines is refused with a message that names the ``max_lines`` it needs."""
+    return ColocatedCTR(models, max_lines)

@@ -35,6 +35,19 @@ static inline int rlctr_lanes_per_row(int rs) {
     return l;
 }
 
+// co-located records (rlctr_group_fwd / rlctr_group_rows_adam): 16-byte chunks of the widest joint row
+#define RLCTR_GROUP_CHUNKS (RLCTR_GROUP_MAX_FLOATS / 4)
+// lanes per row of a vector member's STAND-ALONE table (tables.Geometry.fm: [w?, v_0 .. v_{D-1}] padded to 16 floats, else to 4):
+// its row starts at the chunk of its first column in the joint row.  The stand-alone kernels' reduction trees depend on it.
+// 0: a stand-alone row wider than 36 floats, which no FM-type model has.
+static inline int rlctr_member_lpr(int lin_col, int emb_col, int dim) {
+    const int first = (lin_col >= 0 && lin_col < emb_col) ? lin_col : emb_col;
+    const int last = lin_col > emb_col + dim - 1 ? lin_col : emb_col + dim - 1;
+    const int used = last + 1 - 4 * (first >> 2);
+    if (used > 36) return 0;
+    return rlctr_lanes_per_row(used <= 16 ? 16 : (used + 3) & ~3);
+}
+
 namespace rlctr {
 
 // 128-bit read-only gather of one row chunk.  Rows are touched once per kernel (random ids),

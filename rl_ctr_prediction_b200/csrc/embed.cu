@@ -136,8 +136,10 @@ struct GroupFwdView {
     float* rows_out[RLCTR_GROUP_MAX];
     int rows_pitch[RLCTR_GROUP_MAX];
     int tile_off[RLCTR_GROUP_MAX];           // float offset of the member's tower-input tile in the warp's shared memory, -1 = none
-    int chunk_member[8];                     // vector member whose latent columns chunk c holds, -1 = none (one member per chunk)
-    int warp_floats;                         // shared memory per warp: 32 (column sums) + 8 (per-chunk t) + the tiles
+    int chunk_member[RLCTR_GROUP_CHUNKS];    // vector member whose latent columns chunk c holds, -1 = none (one member per chunk)
+    int lpr[RLCTR_GROUP_MAX];                // lanes per row of the member's stand-alone table (embed_fwd_kernel<LPR>): 4, 8 or 16
+    int warp_floats;                         // shared memory per warp: 32 (column sums) + 8 (per-chunk t) + the tiles; wide records:
+                                             // per sample of the warp, 128 (column sums) + 32 (per-chunk t) + the tiles
 };
 template <int LD>
 __device__ __forceinline__ float4 group_ld(const float* p) {
@@ -329,6 +331,157 @@ group_fwd_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tab,
             }
             group_finish(sA, sB, qA, qB, L, wsm, gv, sums, sums_pitch, b, fields);
         }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
+// K1 over a WIDE co-located record: joint rows of up to four lines (128 floats), or members whose stand-alone rows are wider than
+// 16 floats.  W lanes per joint row, one 16-byte chunk each (W = 16: two samples per warp; W = 32: one), and each lane walks ALL
+// fields of its sample, 16 row loads in flight per block of fields.  A lane reproduces in registers the reduction tree of
+// embed_fwd_kernel<LPR> for the stand-alone table of the member that owns its chunk: RPW = 32 / LPR row slots, slot j adds
+// (row f0 + j + row f0 + RPW + j) per block of 2 RPW fields, then the slots pair as the butterflies xor 1, 2, .. RPW / 2 do; the
+// per-chunk FM terms pair over the member's LPR chunks.  Column sums, sums of squares and logits are bit-identical to the
+// stand-alone kernel's for every member, whatever its row width.
+// ------------------------------------------------------------------------------------------
+template <int RPW>
+__device__ __forceinline__ void wide_block(const float4 (&r)[16], int f0, int fields, const int (&dk)[4], bool fm, float4 (&s)[8],
+                                           float (&q)[8]) {
+#pragma unroll
+    for (int h = 0; h < 16; h += 2 * RPW) {
+        if (f0 + h >= fields) break;                 // the stand-alone loop stops at the last field
+#pragma unroll
+        for (int j = 0; j < RPW; ++j) {
+            const float4 ra = r[h + j], rb = r[h + RPW + j];
+            s[j] = f4add(s[j], f4add(ra, rb));
+            if (fm) {
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    if (dk[k] >= 0) { float x = f4get(ra, k), y = f4get(rb, k); q[j] = fmaf(x, x, q[j]); q[j] = fmaf(y, y, q[j]); }
+            }
+        }
+    }
+}
+template <int RPW>
+__device__ __forceinline__ void wide_slots(float4 (&s)[8], float (&q)[8]) {
+#pragma unroll
+    for (int off = 1; off < RPW; off <<= 1) {
+#pragma unroll
+        for (int j = 0; j < RPW; j += 2 * off) { s[j] = f4add(s[j], s[j + off]); q[j] += q[j + off]; }
+    }
+}
+template <int W>
+__global__ void __launch_bounds__(256)
+group_fwd_wide_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tab, const __grid_constant__ ShardView sv,
+                      int64_t n_rows, int pitch, int rs, const __grid_constant__ GroupFwdView gv, float* __restrict__ sums,
+                      int sums_pitch, int64_t batch, int fields) {
+    constexpr int SPW = 32 / W;                      // samples per warp
+    constexpr int SLOT = 128 + RLCTR_GROUP_CHUNKS;   // staging of one sample: column sums | per-chunk t (the tiles follow)
+    extern __shared__ __align__(16) float gsm[];
+    const int lane = threadIdx.x & 31;
+    const int c = lane % W, slot = lane / W, col0 = 4 * c;
+    const bool chunk_on = col0 < rs;
+    const int slot_floats = gv.warp_floats / SPW;
+    float* wsm = gsm + (threadIdx.x >> 5) * gv.warp_floats + slot * slot_floats;
+    const int mem = chunk_on ? gv.chunk_member[c] : -1;
+    const int m_dim = mem >= 0 ? gv.dim[mem] : 0;
+    const bool m_fm = mem >= 0 && gv.fm[mem] != 0;
+    const int form = mem >= 0 ? gv.lpr[mem] : 4;    // a chunk without a vector member (LR's own): the 16-float form
+    float* tile = (mem >= 0 && gv.tile_off[mem] >= 0) ? wsm + gv.tile_off[mem] : nullptr;
+    int dk[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const int d = col0 + k - (mem >= 0 ? gv.emb_col[mem] : 0);
+        dk[k] = (mem >= 0 && d >= 0 && d < m_dim) ? d : -1;
+    }
+    for (int i = lane; i < gv.warp_floats; i += 32) gsm[(threadIdx.x >> 5) * gv.warp_floats + i] = 0.f;
+    __syncwarp();
+    const int64_t warp0 = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t bw = warp0 * SPW; bw < batch; bw += nwarps * SPW) {        // warp-uniform trip count
+        const int64_t b = bw + slot;
+        const bool live = b < batch;
+        float4 s[8];
+        float q[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) { s[j] = f4zero(); q[j] = 0.f; }
+        for (int f0 = 0; f0 < fields; f0 += 16) {
+            const int fl = f0 + (lane & 15);
+            const int64_t my_id = (live && fl < fields) ? __ldg(ids + b * fields + fl) : -1;
+            float4 r[16];
+            unsigned ok = 0;                             // bit u: field f0 + u has a row
+#pragma unroll
+            for (int u = 0; u < 16; ++u) {               // unconditional loads, dropped below (see group_issue)
+                const int64_t id = __shfl_sync(RLCTR_FULL, my_id, slot * W + u);
+                const bool in = (uint64_t)id < (uint64_t)n_rows;
+                ok |= (unsigned)(in && chunk_on) << u;
+                r[u] = ldg4(row_ptr(tab, sv, in ? id : 0, pitch) + (chunk_on ? col0 : 0));
+            }
+#pragma unroll
+            for (int u = 0; u < 16; ++u) {
+                if (!((ok >> u) & 1)) r[u] = f4zero();
+                if (tile && f0 + u < fields) {
+#pragma unroll
+                    for (int k = 0; k < 4; ++k)
+                        if (dk[k] >= 0) tile[(f0 + u) * m_dim + dk[k]] = f4get(r[u], k);
+                }
+            }
+            if (form == 4) wide_block<8>(r, f0, fields, dk, m_fm, s, q);
+            else if (form == 8) wide_block<4>(r, f0, fields, dk, m_fm, s, q);
+            else wide_block<2>(r, f0, fields, dk, m_fm, s, q);
+        }
+        if (form == 4) wide_slots<8>(s, q);
+        else if (form == 8) wide_slots<4>(s, q);
+        else wide_slots<2>(s, q);
+        float t = 0.f;
+        if (m_fm) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if (dk[k] >= 0) { float x = f4get(s[0], k); t = fmaf(x, x, t); }
+        }
+        t -= q[0];                                   // this chunk's sum of (S_d^2 - sum_f v_d^2)
+        if (chunk_on) {
+            *reinterpret_cast<float4*>(wsm + col0) = s[0];
+            wsm[128 + c] = t;
+            if (sums && live) st4(sums + b * sums_pitch + col0, s[0]);
+        }
+        __syncwarp();
+        if (c < gv.n && live) {                      // lane m of the sample finishes member m
+            const int m = c;
+            float tm = 0.f;
+            if (gv.fm[m] && gv.dim[m] > 0) {         // the member's chunks paired as its stand-alone butterfly xor 1 .. LPR / 2
+                const int base = gv.emb_col[m] >> 2, last = (gv.emb_col[m] + gv.dim[m] - 1) >> 2, L = gv.lpr[m];
+                float v[16];
+#pragma unroll
+                for (int i = 0; i < 16; ++i) v[i] = (i < L && base + i <= last) ? wsm[128 + base + i] : 0.f;
+#pragma unroll
+                for (int w = 1; w < 16; w <<= 1) {
+#pragma unroll
+                    for (int i = 0; i < 16; i += 2 * w)
+                        if (w < L) v[i] = v[i] + v[i + w];
+                }
+                tm = v[0];
+            }
+            const float first = gv.lin_col[m] >= 0 ? wsm[gv.lin_col[m]] : 0.f;
+            const float b0 = gv.bias[m] ? __ldg(gv.bias[m]) : 0.f;
+            const float z = fmaf(0.5f, tm, b0 + first);
+            if (gv.logit[m]) gv.logit[m][b] = z;
+            if (gv.pctr[m]) gv.pctr[m][b * gv.pctr_stride[m]] = sigmoidf_ref(z);
+        }
+        if (live) {
+#pragma unroll
+            for (int m = 0; m < RLCTR_GROUP_MAX; ++m) {      // tower inputs: whole rows, 16 bytes per lane
+                if (m < gv.n && gv.tile_off[m] >= 0) {
+                    const float* src = wsm + gv.tile_off[m];
+                    float* dst = gv.rows_out[m] + b * (int64_t)gv.rows_pitch[m];
+                    if ((gv.rows_pitch[m] & 3) == 0) {
+                        for (int i = c; 4 * i < fields * gv.dim[m]; i += W) st4(dst + 4 * i, *reinterpret_cast<const float4*>(src + 4 * i));
+                    } else {
+                        for (int i = c; i < fields * gv.dim[m]; i += W) dst[i] = src[i];
+                    }
+                }
+            }
+        }
+        __syncwarp();                                // the next sample overwrites the staging area
     }
 }
 
@@ -594,7 +747,7 @@ extern "C" int rlctr_group_fwd(const int64_t* ids, const rlctr_table* table, con
     if (rc) return rc;
     if (!ids || !members || n_members < 1 || n_members > RLCTR_GROUP_MAX || batch < 0 || fields <= 0) return RLCTR_EINVAL;
     const int rs = table->row_stride;
-    if (rs == 1 || rs > 32) return RLCTR_EUNSUPPORTED;
+    if (rs == 1 || rs > RLCTR_GROUP_MAX_FLOATS) return RLCTR_EUNSUPPORTED;
     if (sums && !rlctr_aligned16(sums)) return RLCTR_EALIGN;
     if (sums_pitch == 0) sums_pitch = rs;
     if (sums_pitch < rs || sums_pitch % 4 != 0) return RLCTR_EINVAL;
@@ -603,8 +756,10 @@ extern "C" int rlctr_group_fwd(const int64_t* ids, const rlctr_table* table, con
     if (!shard_view_of(table, &sv)) return RLCTR_EUNSUPPORTED;
     GroupFwdView gv{};
     gv.n = n_members;
-    int fm_owner[8];                                     // chunk -> the FM-term member whose latent columns it holds
-    for (int ch = 0; ch < 8; ++ch) fm_owner[ch] = -1;
+    // one line and every vector member a 16-float stand-alone row: group_fwd_kernel; anything else: group_fwd_wide_kernel
+    bool wide = rs > 32;
+    int fm_owner[RLCTR_GROUP_CHUNKS];                    // chunk -> the FM-term member whose latent columns it holds
+    for (int ch = 0; ch < RLCTR_GROUP_CHUNKS; ++ch) fm_owner[ch] = -1;
     for (int m = 0; m < n_members; ++m) {
         const rlctr_member& mm = members[m];
         if (mm.lin_col >= rs || mm.dim < 0 || mm.emb_col < 0 || mm.emb_col + mm.dim > rs) return RLCTR_EINVAL;
@@ -614,16 +769,19 @@ extern "C" int rlctr_group_fwd(const int64_t* ids, const rlctr_table* table, con
         gv.lin_col[m] = mm.lin_col; gv.emb_col[m] = mm.emb_col; gv.dim[m] = mm.dim; gv.fm[m] = (mm.flags & RLCTR_FM_TERM) ? 1 : 0;
         gv.bias[m] = mm.bias; gv.logit[m] = mm.logit; gv.pctr[m] = mm.pctr; gv.pctr_stride[m] = mm.pctr_stride;
         gv.rows_out[m] = mm.rows_out; gv.rows_pitch[m] = (int)rp;
+        gv.lpr[m] = mm.dim > 0 ? rlctr_member_lpr(mm.lin_col, mm.emb_col, mm.dim) : 4;
+        if (gv.lpr[m] == 0) return RLCTR_EUNSUPPORTED;                     // stand-alone rows of at most 36 floats
+        if (gv.lpr[m] != 4) wide = true;
         if (gv.fm[m] && mm.dim > 0) {
-            if (((mm.emb_col + mm.dim - 1) >> 2) - (mm.emb_col >> 2) > 3) return RLCTR_EUNSUPPORTED;
+            if (((mm.emb_col + mm.dim - 1) >> 2) - (mm.emb_col >> 2) > gv.lpr[m] - 1) return RLCTR_EUNSUPPORTED;
             for (int ch = mm.emb_col >> 2; ch <= (mm.emb_col + mm.dim - 1) >> 2; ++ch) {
                 if (fm_owner[ch] >= 0) return RLCTR_EUNSUPPORTED;       // a chunk's sum of squares belongs to one member
                 fm_owner[ch] = m;
             }
         }
     }
-    for (int ch = 0; ch < 8; ++ch) gv.chunk_member[ch] = -1;
-    int wf = 40;                                         // [column sums 32 | per-chunk t 8]
+    for (int ch = 0; ch < RLCTR_GROUP_CHUNKS; ++ch) gv.chunk_member[ch] = -1;
+    int wf = wide ? 128 + RLCTR_GROUP_CHUNKS : 40;       // [column sums | per-chunk t] (per sample of the warp when wide)
     for (int m = 0; m < n_members; ++m) {
         gv.tile_off[m] = -1;
         if (gv.dim[m] <= 0) continue;
@@ -636,6 +794,32 @@ extern "C" int rlctr_group_fwd(const int64_t* ids, const rlctr_table* table, con
             gv.tile_off[m] = wf;
             wf += (fields * gv.dim[m] + 3) & ~3;
         }
+    }
+    if (wide) {
+        // W lanes per joint row: 16 (two samples per warp) when it has at most 16 chunks, else 32
+        const int W = rs <= 64 ? 16 : 32;
+        gv.warp_floats = (32 / W) * wf;
+        const size_t smem = (size_t)8 * gv.warp_floats * sizeof(float);
+        if (smem > 227 * 1024) return RLCTR_EUNSUPPORTED;
+        const int grid = grid_for_warps((batch + 32 / W - 1) / (32 / W), 8, 8);
+        // tower tiles past 48 KB: the opt-in to the whole 227 KB is set once per device (not per launch, which may be captured)
+        int dev = 0;
+        RLCTR_CUDA(cudaGetDevice(&dev));
+        static bool opted[2][64] = {};
+#define LAUNCH_WIDE(WW)                                                                                                        \
+        {                                                                                                                      \
+            bool& done = opted[WW == 32][dev & 63];                                                                            \
+            if (smem > 48 * 1024 && !done) {                                                                                   \
+                RLCTR_CUDA(cudaFuncSetAttribute(group_fwd_wide_kernel<WW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)); \
+                done = true;                                                                                                   \
+            }                                                                                                                  \
+            group_fwd_wide_kernel<WW><<<grid, 256, smem, (cudaStream_t)stream>>>(ids, table->data, sv, table->n_rows, pitch_of(table), \
+                                                                                rs, gv, sums, sums_pitch, batch, fields);      \
+        }
+        if (W == 16) LAUNCH_WIDE(16) else LAUNCH_WIDE(32)
+#undef LAUNCH_WIDE
+        RLCTR_LAUNCH_CHECK();
+        return RLCTR_OK;
     }
     gv.warp_floats = wf;
     const size_t smem = (size_t)8 * wf * sizeof(float);

@@ -73,8 +73,9 @@ struct GroupCols {
                                              // (-> sample, for S and dL/dlogit) is slot_of[r], the dense-tail row is extra_m[r]
     int sums_pitch;                          // floats between the sums rows; dz[m] == NULL: dL/dlogit of member m rides in column
                                              // sums_pitch - RLCTR_GROUP_MAX + m of the sample's sums row
-    signed char member[32];                  // column -> member, -1: padding / stamp
-    signed char role[32];                    // 0 none, 1 first-order weight, 2 latent column with the FM term, 3 latent column without
+    signed char member[RLCTR_GROUP_MAX_FLOATS];  // column -> member, -1: padding / stamp
+    signed char role[RLCTR_GROUP_MAX_FLOATS];    // 0 none, 1 first-order weight, 2 latent column with the FM term, 3 latent column without
+    signed char lpr[RLCTR_GROUP_MAX];        // lanes per row of member m's stand-alone table (rlctr_member_lpr): its long-run tree
     int dz_used;                             // bit m: a column of member m (role 1 or 2) uses its dL/dlogit.  A member whose row
                                              // gradient is all dense tail (FNN, PNN, DCN: role 3 only) has no dL/dlogit load
 };
@@ -217,8 +218,8 @@ __device__ __forceinline__ GroupLane group_lane(const GradView& g, int col0) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const int col = col0 + k;
-        gl.mem[k] = col < 32 ? (int)g.grp.member[col] : -1;
-        gl.role[k] = col < 32 ? (int)g.grp.role[col] : 0;
+        gl.mem[k] = col < RLCTR_GROUP_MAX_FLOATS ? (int)g.grp.member[col] : -1;
+        gl.role[k] = col < RLCTR_GROUP_MAX_FLOATS ? (int)g.grp.role[col] : 0;
     }
     return gl;
 }
@@ -296,7 +297,7 @@ __device__ __forceinline__ void finish_row(int64_t id, int col0, float4 p, const
 
 // one lane-group (LPR lanes, a float4 chunk each) per sorted position; only run heads work
 template <int LPR, int APPLY, bool GROUP = false>
-__global__ void __launch_bounds__(256, 5)
+__global__ void __launch_bounds__(256, (LPR > 8 ? 4 : 5))      // 16 / 32 lanes: wide co-located records, 64 registers: no spills
 rows_short_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                   const __grid_constant__ GradView g, TableView t, AdamView a, float* __restrict__ dense_grad,
                   int32_t* __restrict__ long_count, uint32_t* __restrict__ long_list) {
@@ -752,6 +753,67 @@ rows_long_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __rest
     }
 }
 
+// Heavy hitters of a WIDE co-located record (rlctr_group_rows_adam: more than one line, or members whose stand-alone rows are wider
+// than 16 floats): block per long run, thread = (chunk, sub-group).  Chunk c sums the run in the sub-groups of its member's
+// stand-alone update and pairs them in that kernel's tree: 64 sub-groups for a 16-float row (rows_long_kernel<4>), 32 for 20..32
+// floats (rows_long_kernel<8>), one walked in slot order for 36 floats (rows_wide_kernel).  Same per-column arithmetic
+// (group_col_grad) and the same Adam step: bit-identical to each member's stand-alone update.
+__global__ void __launch_bounds__(256)
+group_long_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
+                       const __grid_constant__ GradView g, const __grid_constant__ TableView t, const __grid_constant__ AdamView a,
+                       const int32_t* __restrict__ long_count, const uint32_t* __restrict__ long_list) {
+    constexpr int SUBS = 64, C = RLCTR_GROUP_CHUNKS, PER = SUBS * C / 256;   // (sub-group, chunk) pairs per thread
+    __shared__ float4 red[SUBS * C];
+    __shared__ int64_t s_end;
+    const int c = threadIdx.x % C, s0 = threadIdx.x / C, col0 = 4 * c;
+    const bool chunk_on = c < ((t.used + 3) >> 2);
+    const GroupLane gl = group_lane(g, col0);
+    int form = 4;                                        // a chunk without latent columns (LR's own): the 16-float form
+#pragma unroll
+    for (int k = 0; k < 4; ++k)
+        if (gl.role[k] >= 2) form = g.grp.lpr[gl.mem[k]];
+    const int nsub = form == 4 ? 64 : (form == 8 ? 32 : 1);
+    const int nlong = *long_count;
+    for (int li = blockIdx.x; li < nlong; li += gridDim.x) {
+        const int64_t k = long_list[li];
+        const uint32_t id = __ldg(sorted_ids + k);
+        if (threadIdx.x == 0) {                          // upper bound of the run by bisection
+            int64_t lo = k, hi = n;
+            while (hi - lo > 1) {
+                int64_t mid = (lo + hi) >> 1;
+                if (__ldg(sorted_ids + mid) == id) lo = mid; else hi = mid;
+            }
+            s_end = hi;
+        }
+        __syncthreads();
+        const int64_t end = s_end;
+        const float4 p = chunk_on ? ld4(t.data + (int64_t)id * t.pitch + col0) : f4zero();
+#pragma unroll
+        for (int j = 0; j < PER; ++j) {
+            const int sub = s0 + j * (256 / C);
+            float4 acc = f4zero();
+            if (chunk_on && sub < nsub)
+                for (int64_t kk = k + sub; kk < end; kk += nsub) acc = f4add(acc, rowgrad_group(g, gl, __ldg(sorted_slots + kk), col0, p, t));
+            red[sub * C + c] = acc;
+        }
+        const int step = __ldg(a.step) + 1;
+        int stamp_in = 0;
+        if (s0 == 0 && chunk_on && is_lazy(a)) stamp_in = load_stamp(t, a, id);
+        __syncthreads();
+        for (int half = SUBS / 2; half > 0; half >>= 1) {
+#pragma unroll
+            for (int j = 0; j < PER; ++j) {
+                const int sub = s0 + j * (256 / C);
+                if (sub < half && half < nsub) red[sub * C + c] = f4add(red[sub * C + c], red[(sub + half) * C + c]);
+            }
+            __syncthreads();
+        }
+        if (s0 == 0 && chunk_on) finish_row<0>(id, col0, p, red[c], t, a, nullptr, step, stamp_in);
+        __syncthreads();
+        if (a.stamp && threadIdx.x == 0) a.stamp[id] = step;      // a separate stamp array (the in-record stamp rides in p)
+    }
+}
+
 // wide rows (row_stride > 32 floats: the interleaved FFM table, 36-float FM rows): one WARP per sorted position,
 // lanes stride the float4 chunks of the row (WCH chunks per lane); runs are walked sequentially
 // in slot order so the sum is bit-identical from run to run.  WCH = 2: rows up to 256 floats; WCH = 4: up to 512
@@ -905,7 +967,8 @@ __device__ __forceinline__ int64_t replay_row_of(int64_t k, int64_t n_items, int
 }
 // issue the loads of a whole record WITHOUT looking at its stamp first: one DRAM round trip instead of two, and
 // nothing in the caller depends on the data until the item becomes current (a full replay of another row later).
-// LPRR lanes share a row (co-located records of 5..8 chunks): lane slice h owns chunks h*CH .. h*CH+CH-1, `live` of them active.
+// LPRR lanes share a row (co-located records of 5..32 chunks): lane slice h owns chunks h*CH .. h*CH+CH-1, `live` of them active
+// (none for the last slices of a record that does not fill them).
 template <int CH, bool UNSORTED = false>
 __device__ __forceinline__ void replay_row_issue(ReplayRow<CH>& it, int64_t row, const TableView& t, const AdamView& a, int first_col,
                                                  int live, uint32_t* __restrict__ claim = nullptr, bool claimer = false) {
@@ -962,7 +1025,7 @@ __device__ __forceinline__ void replay_row_arm(ReplayRow<CH>& it, const AdamView
     if (st >= upto) it.off = -1; else it.t = st;
 }
 template <int CH, int LPRR, bool CATCHUP, bool UNSORTED = false>
-__global__ void __launch_bounds__(128, (CH == 3 ? 4 : 3))
+__global__ void __launch_bounds__(128, (LPRR > 2 ? (CH == 3 ? 3 : 2) : (CH == 3 ? 4 : 3)))   // wide records (LPRR 4, 8): no spills
 replay_rows_kernel(TableView t, AdamView a, int64_t r0, int64_t n_items, const uint32_t* __restrict__ sorted_ids,
                    const int64_t* __restrict__ ids64 = nullptr, uint32_t* __restrict__ claim = nullptr) {
     const int64_t stride = ((int64_t)gridDim.x * blockDim.x) / LPRR;  // rows between two items of one lane
@@ -1014,7 +1077,7 @@ template <bool CATCHUP>
 static int launch_replay_rows(const TableView& t, const AdamView& a, int64_t r0, int64_t n_items,
                               const uint32_t* sorted_ids, cudaStream_t st, const int64_t* ids64 = nullptr, uint32_t* claim = nullptr) {
     const int ch = (t.used + 3) >> 2;
-    const int lprr = ch > 4 ? 2 : 1;                     // co-located records (5..8 chunks): two lanes per row
+    const int lprr = ch > 16 ? 8 : (ch > 8 ? 4 : (ch > 4 ? 2 : 1));   // co-located records (5..32 chunks): 2, 4 or 8 lanes per row
     if (a.stamp_col >> 2 != ch - 1) return RLCTR_EUNSUPPORTED;        // the stamp rides in the last active chunk
     int64_t blocks = (n_items * lprr + 127) / 128;
     static int rgrid_env = -1;
@@ -1037,7 +1100,13 @@ static int launch_replay_rows(const TableView& t, const AdamView& a, int64_t r0,
         case 4: replay_rows_kernel<4, 1, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
         case 5: case 6: replay_rows_kernel<3, 2, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
         case 7: case 8: replay_rows_kernel<4, 2, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        default: return RLCTR_EUNSUPPORTED;
+        case 9: case 10: case 11: case 12: replay_rows_kernel<3, 4, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 13: case 14: case 15: case 16: replay_rows_kernel<4, 4, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        default:
+            if (ch > 32) return RLCTR_EUNSUPPORTED;      // wider than four lines
+            if (ch <= 24) replay_rows_kernel<3, 8, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids);
+            else replay_rows_kernel<4, 8, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids);
+            break;
     }
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
@@ -1593,7 +1662,7 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
     cudaStream_t st = (cudaStream_t)stream;
     TableView t = view_of(table);
     AdamView a = view_of(opt, t);
-    if (t.rs % 4 != 0 || t.rs <= 8 || t.rs > 32) return RLCTR_EUNSUPPORTED;
+    if (t.rs % 4 != 0 || t.rs <= 8 || t.rs > RLCTR_GROUP_MAX_FLOATS) return RLCTR_EUNSUPPORTED;
     if (opt->stamp_col >= t.pitch) return RLCTR_EINVAL;
     if (!rlctr_aligned16(sums)) return RLCTR_EALIGN;
     if (sums_pitch == 0) sums_pitch = t.rs;
@@ -1603,7 +1672,9 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
     g.grp.n = n_members;
     g.grp.sums_pitch = sums_pitch;
     g.grp.slot_of = slot_of;
-    for (int col = 0; col < 32; ++col) { g.grp.member[col] = -1; g.grp.role[col] = 0; }
+    for (int col = 0; col < RLCTR_GROUP_MAX_FLOATS; ++col) { g.grp.member[col] = -1; g.grp.role[col] = 0; }
+    // one line and every vector member a 16-float stand-alone row: the one-line kernels; anything else: the wide ones
+    bool wide = t.rs > 32;
     for (int m = 0; m < n_members; ++m) {
         const rlctr_member& mm = members[m];
         if (mm.dim < 0 || mm.emb_col < 0 || mm.emb_col + mm.dim > t.rs || mm.lin_col >= t.rs) return RLCTR_EINVAL;
@@ -1613,6 +1684,9 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
         if (uses_dz) g.grp.dz_used |= 1 << m;
         g.grp.dz[m] = mm.dlogit; g.grp.extra[m] = mm.extra; g.grp.emb_col[m] = mm.emb_col; g.grp.dim[m] = mm.dim;
         g.grp.ex_pitch[m] = mm.extra_pitch ? (int)mm.extra_pitch : mm.dim;
+        g.grp.lpr[m] = (signed char)(mm.dim > 0 ? rlctr_member_lpr(mm.lin_col, mm.emb_col, mm.dim) : 4);
+        if (g.grp.lpr[m] == 0) return RLCTR_EUNSUPPORTED;                // stand-alone rows of at most 36 floats
+        if (g.grp.lpr[m] != 4) wide = true;
         if (mm.lin_col >= 0) {
             if (g.grp.member[mm.lin_col] >= 0) return RLCTR_EINVAL;              // two members claim one column
             g.grp.member[mm.lin_col] = (signed char)m; g.grp.role[mm.lin_col] = 1;
@@ -1623,10 +1697,23 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
             g.grp.member[col] = (signed char)m; g.grp.role[col] = (mm.flags & RLCTR_FM_TERM) ? 2 : 3;
         }
     }
-    if (opt->stamp_col >= 0 && opt->stamp_col < 32 && g.grp.member[opt->stamp_col] >= 0) return RLCTR_EINVAL;
+    if (opt->stamp_col >= 0 && opt->stamp_col < RLCTR_GROUP_MAX_FLOATS && g.grp.member[opt->stamp_col] >= 0) return RLCTR_EINVAL;
     if (ws_bytes < rows_ws_bytes(n) || !ws) return RLCTR_EWORKSPACE;
     RowsWs w{reinterpret_cast<int32_t*>(ws), reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(ws) + 16)};
     RLCTR_CUDA(cudaMemsetAsync(w.long_count, 0, sizeof(int32_t), st));
+    if (wide) {
+        // short runs: a lane per chunk walks the occurrences in slot order (the order of every stand-alone form), 16 or 32 lanes per
+        // record; long runs: each chunk in its member's stand-alone tree (group_long_wide_kernel)
+        const int lanes = t.rs <= 64 ? 16 : 32;
+        unsigned blocks = capped_blocks((n * lanes + 255) / 256, world);
+        if (rows_grid_env() > 0 && blocks > (unsigned)(RLCTR_SMS * 5 * rows_grid_env())) blocks = RLCTR_SMS * 5 * rows_grid_env();
+        if (lanes == 16) rows_short_kernel<16, 0, true><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        else rows_short_kernel<32, 0, true><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        group_long_wide_kernel<<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
+        RLCTR_COUNT_LAUNCH(1);                          // two kernels, one check
+        RLCTR_LAUNCH_CHECK();
+        return RLCTR_OK;
+    }
     const int lpr = rlctr_lanes_per_row(t.rs);
     // RLCTR_GROUP_ROWS2=0: the eight-lanes-per-record kernel.  Both take ~250 us for 936 K records at B = 65536 (read per call: the
     // tests switch it): 2.5x fewer instructions and 1.7x more records in flight buy nothing, because the update already runs at the
@@ -1770,7 +1857,7 @@ extern "C" int rlctr_rows_catchup_ids(const int64_t* ids, int64_t n, const rlctr
     cudaStream_t st = (cudaStream_t)stream;
     TableView t = view_of(table);
     AdamView a = view_of(opt, t);
-    if (t.rs % 4 != 0 || ((t.used + 3) >> 2) < 5) return RLCTR_EUNSUPPORTED;
+    if (t.rs % 4 != 0 || ((t.used + 3) >> 2) < 5 || ((t.used + 3) >> 2) > 8) return RLCTR_EUNSUPPORTED;   // records of 5..8 chunks
     RLCTR_CUDA(cudaMemsetAsync(claim, 0, rlctr_rows_claim_bytes(table->n_rows), st));
     return launch_replay_rows<true>(t, a, 0, n, nullptr, st, ids, reinterpret_cast<uint32_t*>(claim));
 }

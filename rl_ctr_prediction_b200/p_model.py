@@ -279,8 +279,9 @@ class _TableModel(nn.Module):
             if name != "table" and p is not None:
                 destination[prefix + name] = p if keep_vars else p.detach()
         tab = self.table.detach()
+        off = self._geom.offset
         for key, col, w in self._ref_items():
-            destination[prefix + key] = tab[:, col:col + w].clone()
+            destination[prefix + key] = tab[:, off + col:off + col + w].clone()
 
     def _load_from_state_dict(self, state_dict, prefix, local_metadata, strict, missing_keys, unexpected_keys,
                               error_msgs):
@@ -298,7 +299,8 @@ class _TableModel(nn.Module):
                     error_msgs.append(f"size mismatch for {k}: checkpoint {tuple(src.shape)} vs model "
                                       f"{(self._geom.n_rows, w)}")
                     continue
-                self.table.data[:, col:col + w].copy_(src)
+                off = self._geom.offset + col
+                self.table.data[:, off:off + w].copy_(src)
             for name, p in self._parameters.items():
                 if name == "table" or p is None:
                     continue
@@ -413,10 +415,11 @@ class FFM(_TableModel):
         return self._run(x, False, True)[0]
 
 
-def colocate(models):
-    """Re-home LR / FM-type models trained on the same id stream into ONE joint table (colocated.ColocatedCTR)."""
+def colocate(models, max_lines=1):
+    """Re-home LR / FM-type models trained on the same id stream into ONE joint table (colocated.ColocatedCTR) of at most
+    ``max_lines`` 128-byte lines per row (1..4)."""
     from .colocated import ColocatedCTR
-    return ColocatedCTR(models)
+    return ColocatedCTR(models, max_lines)
 
 
 def _tower(in_dims: int, device=None) -> nn.Sequential:
@@ -535,8 +538,9 @@ class FNN(_TableModel):
     def load_embedding(self, pretrain_params):
         self.flush()
         g = self._geom
+        c = g.offset + g.emb_col                 # a member of a wide co-located record: its view starts at g.offset
         with torch.no_grad():
-            self.table.data[:, g.emb_col:g.emb_col + g.dim].copy_(pretrain_params["feature_embedding.weight"])
+            self.table.data[:, c:c + g.dim].copy_(pretrain_params["feature_embedding.weight"])
 
     def _tower_input(self, rows):
         return rows

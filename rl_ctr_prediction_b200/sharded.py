@@ -572,10 +572,12 @@ class ShardedGroup(_co._GroupStep, _ShardedTable):
     the single-GPU group step on the concatenated global batch.  ``members[i]`` is the member's p_model module without a table of
     its own: its bias, tower, cross network or attention, and the ``_tail`` the group step runs."""
 
-    SUMS_PITCH = 32                    # one 128-byte line per sample: S (<= 28 floats) | dL/dlogit of members 0..3
+    SUMS_PITCH = 32                    # floats per sample of the exchange row: S | dL/dlogit of members 0..3 in the last four columns.
+                                       # One line (S <= 28 floats); with max_lines > 1 the instance widens it to the whole lines
+                                       # that hold rs + 4 floats
     _UPDATE_KEY = "rlctr_group_rows_adam[ShardedGroup]"
 
-    def __init__(self, kinds, feature_nums, field_nums, latent_dims, group=None, device=None):
+    def __init__(self, kinds, feature_nums, field_nums, latent_dims, group=None, device=None, max_lines=1):
         kinds = tuple(_ALIASES.get(k, k) for k in kinds)
         names = tuple(c.__name__ for c in _co.MEMBER_KINDS)
         if not all(k in names for k in kinds) or not 1 <= len(kinds) <= _lib.RLCTR_GROUP_MAX:
@@ -583,14 +585,19 @@ class ShardedGroup(_co._GroupStep, _ShardedTable):
         super().__init__(feature_nums, group, device)
         self.kinds, self.field_nums, self.latent_dims = kinds, int(field_nums), int(latent_dims)
         members = [_dense_member(k, self.field_nums, self.latent_dims, self._dev) for k in kinds]
-        self._cols, used = _co._layout(members)
+        self._cols, used = _co._layout(members, max_lines)
         rs = (used + 1 + 3) // 4 * 4
-        if rs > self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX:
-            raise _lib.RlctrError("joint row too wide for the per-sample exchange row (28 floats)")
-        self._geom = Geometry(self._n_local, rs, -1, 0, used, pitch=96, block=32, stamp_at=used)
+        if max_lines == 1 and rs > self.SUMS_PITCH - _lib.RLCTR_GROUP_MAX:
+            raise _lib.RlctrError("joint row too wide for the per-sample exchange row (28 floats); pass max_lines=2 for a "
+                                  "two-line exchange row")
+        if max_lines > 1:
+            self.SUMS_PITCH = (rs + _lib.RLCTR_GROUP_MAX + 31) // 32 * 32
+        self._geom = _co._record(self._n_local, used)
+        self._max_lines = max_lines
         self._alloc_table([([lin] if lin >= 0 else []) + list(range(emb, emb + dim)) for lin, emb, dim in self._cols])
-        for m, (lin, emb, dim) in zip(members, self._cols):
-            _rehome(m, self, Geometry(self._n_local, rs, lin, emb, dim, pitch=96, block=32))
+        wide = _co._wide(members, used)
+        for m, col in zip(members, self._cols):
+            _rehome(m, self, _co._member_view(m, self._geom, col, wide))
         self.members = nn.ModuleList(members)
         self._buf = {}
 
@@ -616,7 +623,7 @@ class ShardedGroup(_co._GroupStep, _ShardedTable):
         kinds = [type(m).__name__ for m in cg.members]
         F = next((m.field_nums for m in cg.members if hasattr(m, "field_nums")), 15)
         self = cls(kinds, cg.feature_nums, F, max(getattr(m, "latent_dims", 1) for m in cg.members),
-                   group=group, device=cg.table.device)
+                   group=group, device=cg.table.device, max_lines=cg._max_lines)
         assert self._cols == cg._cols
         cg.flush()
         self._copy_shard(cg.table.data)

@@ -47,6 +47,8 @@ class Geometry:
     block: int = 0            # floats between the p / exp_avg / exp_avg_sq blocks of a record; 0 = row_stride.  A co-located
                               # record (colocated.py) keeps each block in its own 128-byte line: row_stride 24, block 32, pitch 96
     stamp_at: int = -1        # >= 0: the lazy-Adam stamp's column, chosen by whoever laid the record out (colocated.py)
+    offset: int = 0           # floats from the start of the record to this view's column 0: a member's stand-alone view of a wide
+                              # co-located record (colocated.py), whose own row starts at its first chunk
 
     @property
     def row_pitch(self):
@@ -103,7 +105,8 @@ class Geometry:
 
 
 def table_struct(data: torch.Tensor, g: Geometry) -> _lib.Table:
-    return _lib.Table(_lib.ptr(data), g.n_rows, g.row_stride, g.lin_col, g.emb_col, g.dim, g.row_pitch)
+    p = _lib.ptr(data)
+    return _lib.Table(p + 4 * g.offset if g.offset else p, g.n_rows, g.row_stride, g.lin_col, g.emb_col, g.dim, g.row_pitch)
 
 
 class AdamSchedule:
