@@ -165,7 +165,7 @@ int rlctr_embed_fwd(const int64_t* ids, const rlctr_table* table, const float* b
 /* Pairwise inner products over already-gathered rows: the InnerPNN tower input (p_model.py:178-198)
  *   out[b, :] = [ E (fields*dim) | ip (P = fields*(fields-1)/2) ]   (ip_first != 0: [ ip | E ], Feature_embedding.py:51-59)
  *   ip[p] = <E[i], E[j]> for the p-th pair (i < j, row-major)      rows: [batch, fields*dim] at pitch ld_rows
- * and its backward  grows[b, i, :] = g_E[i, :] + sum_{j != i} g_ip[pair(i, j)] * E[j, :].  fields <= 23. */
+ * and its backward  grows[b, i, :] = g_E[i, :] + sum_{j != i} g_ip[pair(i, j)] * E[j, :].  2 <= fields <= 64. */
 int rlctr_pairdots_fwd(const float* rows, int64_t ld_rows, float* out, int64_t ld_out, int64_t batch,
                        int32_t fields, int32_t dim, int32_t ip_first, rlctr_stream_t stream);
 int rlctr_pairdots_bwd(const float* rows, int64_t ld_rows, const float* gout, int64_t ld_g, float* grows,
@@ -219,6 +219,8 @@ int rlctr_gather_rows(const int64_t* ids, int64_t n, const rlctr_table* table, f
  * partners (optional, training; [B*F, row_stride]): partners[b*F+i, block j] = T_i[x_j] for
  * j != i, 0 on the diagonal, 1 at lin_col -- d logit / d row_i, the autograd of :91 (SURVEY
  * section 3.7 FFM).  Feed it to rlctr_rows_adam as `staged` with RLCTR_STAGED_PARTNER.
+ * 2 <= fields <= 64; one sample's fields rows (plus the pair and partner tables) must fit in
+ * 227 KB of shared memory, which every row of at most 512 floats does.
  * ------------------------------------------------------------------------------------ */
 int rlctr_ffm_fwd(const int64_t* ids, const rlctr_table* table, const float* bias,
                   float* logit, float* pctr, int64_t pctr_stride, float* partners,

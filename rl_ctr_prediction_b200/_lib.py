@@ -164,15 +164,20 @@ def load() -> C.CDLL:
     return lib
 
 
-# the shape limits behind RLCTR_EUNSUPPORTED of the entry points the latent size reaches (F = 15: D <= 32 for every model)
+# the shape limits behind RLCTR_EUNSUPPORTED of the entry points the field count F and the latent size D reach: every model serves
+# 2 <= F <= 64 and 1 <= D <= 32 within these (AFM only up to F = 23, DCN and FFM only up to their per-row limits)
 SHAPE_LIMITS = {
+    "rlctr_pairdots_fwd": "InnerPNN pair dots: 2 <= F <= 64",
+    "rlctr_pairdots_bwd": "InnerPNN pair dots: 2 <= F <= 64",
+    "rlctr_ffm_fwd": "FFM: 2 <= F <= 64 (one sample's F rows in at most 227 KB of shared memory)",
     "rlctr_embed_fwd": "fused rows of at most 36 floats (D <= 32 with a first-order column, 36 without)",
     "rlctr_afm_fwd": "AFM: D <= 32, F <= 23",
     "rlctr_afm_bwd": "AFM: D <= 32, F <= 23",
     "rlctr_cross_fwd": "DCN: F*D <= 512, at most 8 cross layers",
     "rlctr_cross_bwd": "DCN: F*D <= 512, at most 6 cross layers",
     "rlctr_rows_adam": "fused rows of at most 512 floats (FFM: F*D + 1 <= 512)",
-    "rlctr_group_fwd": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats",
+    "rlctr_group_fwd": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats; "
+                       "one-line records: tower-member tiles of 48 KB per 8 samples (sum of F*D over tower members <= 1496)",
     "rlctr_group_rows_adam": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats",
     "rlctr_rows_catchup": "records with an in-record stamp: rows of at most 128 floats",
     "rlctr_adam_flush": "records with an in-record stamp: rows of at most 128 floats",

@@ -602,15 +602,17 @@ featemb_fwd_kernel(const int64_t* __restrict__ ids, const float* __restrict__ ta
 // Pairwise inner products over already-gathered rows (InnerPNN, p_model.py:178-198): the tower input
 // [E (F*D) | ip (P)] (or [ip | E], the Feature_Embedding order) and its backward
 //     d E[i] = g_E[i] + sum_{j != i} g_ip[pair(i,j)] * E[j]
-// Warp per sample; E and g_ip are staged in shared memory; pair index by a byte table.
+// Warp per sample; E and g_ip are staged in shared memory; pair index by a table of PIDX entries: bytes up to F = 23
+// (P <= 253), 16-bit entries past that (F <= 64: P <= 2016).
 // ------------------------------------------------------------------------------------------
-__device__ __forceinline__ void pair_tables(unsigned char* pi, unsigned char* pj, unsigned char* pidx, int fields) {
+template <typename PIDX>
+__device__ __forceinline__ void pair_tables(unsigned char* pi, unsigned char* pj, PIDX* pidx, int fields) {
     for (int i = threadIdx.x; i < fields; i += blockDim.x) {
         const int base = i * fields - i * (i + 1) / 2;       // pairs (i, i+1..F-1) in the reference's order
         for (int j = i + 1; j < fields; ++j) {
             const int p = base + j - i - 1;
             if (pi) { pi[p] = (unsigned char)i; pj[p] = (unsigned char)j; }
-            if (pidx) { pidx[i * fields + j] = (unsigned char)p; pidx[j * fields + i] = (unsigned char)p; }
+            if (pidx) { pidx[i * fields + j] = (PIDX)p; pidx[j * fields + i] = (PIDX)p; }
         }
     }
 }
@@ -623,7 +625,7 @@ pairdots_fwd_kernel(const float* __restrict__ rows, int64_t ld_rows, float* __re
     float* stage = smem + wib * fd;
     unsigned char* pi = reinterpret_cast<unsigned char*>(smem + nw * fd);
     unsigned char* pj = pi + npair;
-    pair_tables(pi, pj, nullptr, fields);
+    pair_tables<unsigned char>(pi, pj, nullptr, fields);
     __syncthreads();
     const int e_off = ip_first ? npair : 0, ip_off = ip_first ? 0 : fd;
     for (int64_t b = (int64_t)blockIdx.x * nw + wib; b < batch; b += (int64_t)gridDim.x * nw) {
@@ -641,6 +643,7 @@ pairdots_fwd_kernel(const float* __restrict__ rows, int64_t ld_rows, float* __re
         __syncwarp();
     }
 }
+template <typename PIDX>
 __global__ void __launch_bounds__(128)
 pairdots_bwd_kernel(const float* __restrict__ rows, int64_t ld_rows, const float* __restrict__ gout, int64_t ld_g,
                     float* __restrict__ grows, int64_t ld_grows, int64_t batch, int fields, int dim, int ip_first) {
@@ -649,8 +652,8 @@ pairdots_bwd_kernel(const float* __restrict__ rows, int64_t ld_rows, const float
     const int fd = fields * dim, npair = fields * (fields - 1) / 2;
     float* stage = smem + wib * (fd + npair);
     float* gip = stage + fd;
-    unsigned char* pidx = reinterpret_cast<unsigned char*>(smem + nw * (fd + npair));
-    pair_tables(nullptr, nullptr, pidx, fields);
+    PIDX* pidx = reinterpret_cast<PIDX*>(smem + nw * (fd + npair));
+    pair_tables<PIDX>(nullptr, nullptr, pidx, fields);
     __syncthreads();
     const int e_off = ip_first ? npair : 0, ip_off = ip_first ? 0 : fd;
     for (int64_t b = (int64_t)blockIdx.x * nw + wib; b < batch; b += (int64_t)gridDim.x * nw) {
@@ -661,7 +664,7 @@ pairdots_bwd_kernel(const float* __restrict__ rows, int64_t ld_rows, const float
         __syncwarp();
         for (int t = lane; t < fd; t += 32) {
             const int i = t / dim, d = t - i * dim;
-            const unsigned char* prow = pidx + i * fields;
+            const PIDX* prow = pidx + i * fields;
             float a0 = __ldg(g + e_off + t), a1 = 0.f;                  // two chains: a string of dependent LDS -> FMA otherwise
             int j = 0;
             for (; j + 1 < fields; j += 2) {
@@ -897,7 +900,7 @@ extern "C" int rlctr_featemb_fwd(const int64_t* ids, const rlctr_table* table, f
 extern "C" int rlctr_pairdots_fwd(const float* rows, int64_t ld_rows, float* out, int64_t ld_out, int64_t batch,
                                   int32_t fields, int32_t dim, int32_t ip_first, rlctr_stream_t stream) {
     if (!rows || !out || batch < 0 || fields < 2 || dim <= 0) return RLCTR_EINVAL;
-    if (fields > 23) return RLCTR_EUNSUPPORTED;                         // pair indices are bytes: F <= 23 (P <= 253)
+    if (fields > 64) return RLCTR_EUNSUPPORTED;
     const int fd = fields * dim, npair = fields * (fields - 1) / 2;
     if (ld_rows < fd || ld_out < fd + npair) return RLCTR_EINVAL;
     if (batch == 0) return RLCTR_OK;
@@ -914,16 +917,32 @@ extern "C" int rlctr_pairdots_bwd(const float* rows, int64_t ld_rows, const floa
                                   int64_t ld_grows, int64_t batch, int32_t fields, int32_t dim, int32_t ip_first,
                                   rlctr_stream_t stream) {
     if (!rows || !gout || !grows || batch < 0 || fields < 2 || dim <= 0) return RLCTR_EINVAL;
-    if (fields > 23) return RLCTR_EUNSUPPORTED;
+    if (fields > 64) return RLCTR_EUNSUPPORTED;
     const int fd = fields * dim, npair = fields * (fields - 1) / 2;
     if (ld_rows < fd || ld_g < fd + npair || ld_grows < fd) return RLCTR_EINVAL;
     if (batch == 0) return RLCTR_OK;
     const int nw = 4;
-    const size_t smem = (size_t)nw * (fd + npair) * sizeof(float) + (size_t)fields * fields;
-    if (smem > 48 * 1024) return RLCTR_EUNSUPPORTED;
-    pairdots_bwd_kernel<<<grid_for_warps(batch, nw, 16), nw * 32, smem, (cudaStream_t)stream>>>(rows, ld_rows, gout, ld_g, grows,
-                                                                                               ld_grows, batch, fields, dim,
-                                                                                               ip_first ? 1 : 0);
+    const int grid = grid_for_warps(batch, nw, 16);
+    const size_t stage = (size_t)nw * (fd + npair) * sizeof(float);
+    if (fields <= 23) {                                                 // byte pair indices (P <= 253)
+        const size_t smem = stage + (size_t)fields * fields;
+        if (smem > 48 * 1024) return RLCTR_EUNSUPPORTED;
+        pairdots_bwd_kernel<unsigned char><<<grid, nw * 32, smem, (cudaStream_t)stream>>>(rows, ld_rows, gout, ld_g, grows, ld_grows,
+                                                                                         batch, fields, dim, ip_first ? 1 : 0);
+    } else {                                                            // 16-bit pair indices (P <= 2016)
+        const size_t smem = stage + (size_t)fields * fields * sizeof(unsigned short);
+        if (smem > 227 * 1024) return RLCTR_EUNSUPPORTED;
+        // past 48 KB (F = 64 at D = 32 takes 72 KB): the opt-in is set once per device, not per launch, which may be captured
+        int dev = 0;
+        RLCTR_CUDA(cudaGetDevice(&dev));
+        static bool opted[64] = {};
+        if (smem > 48 * 1024 && !opted[dev & 63]) {
+            RLCTR_CUDA(cudaFuncSetAttribute(pairdots_bwd_kernel<unsigned short>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+            opted[dev & 63] = true;
+        }
+        pairdots_bwd_kernel<unsigned short><<<grid, nw * 32, smem, (cudaStream_t)stream>>>(rows, ld_rows, gout, ld_g, grows, ld_grows,
+                                                                                          batch, fields, dim, ip_first ? 1 : 0);
+    }
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
 }

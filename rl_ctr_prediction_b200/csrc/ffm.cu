@@ -15,7 +15,6 @@
 
 namespace rlctr {
 
-constexpr int FFM_WARPS = 2;
 constexpr unsigned short FFM_ZERO = 0xffffu, FFM_ONE = 0xfffeu;
 
 // 16-byte asynchronous copy global -> shared; src_bytes = 0 writes zeros (an id outside the table is an all-zero row)
@@ -25,12 +24,16 @@ __device__ __forceinline__ void ffm_cp16(float* smem_dst, const float* gsrc, int
 }
 __device__ __forceinline__ void ffm_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void ffm_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-// the F rows of one sample into `dst` [F][rs]: lane f holds the id of field f (fields <= 32), the lanes take chunks lane, lane + 32 ...
-__device__ __forceinline__ void ffm_issue_rows(float* dst, int64_t my_id, const float* __restrict__ tab, const ShardView& sv,
-                                               int64_t n_rows, int pitch, int rs, int fields, int lane) {
+// the F rows of one sample into `dst` [F][rs]: lane f holds the id of field f in `my_id` and, when F64, that of field f + 32 in
+// `my_id_hi` (fields <= 32, or <= 64 with F64); the lanes take chunks lane, lane + 32 ...
+template <bool F64>
+__device__ __forceinline__ void ffm_issue_rows(float* dst, int64_t my_id, int64_t my_id_hi, const float* __restrict__ tab,
+                                               const ShardView& sv, int64_t n_rows, int pitch, int rs, int fields, int lane) {
     const int chunks = rs >> 2;
     for (int f = 0; f < fields; ++f) {
-        const int64_t id = __shfl_sync(RLCTR_FULL, my_id, f);
+        int64_t id;
+        if constexpr (F64) id = __shfl_sync(RLCTR_FULL, f < 32 ? my_id : my_id_hi, f & 31);
+        else id = __shfl_sync(RLCTR_FULL, my_id, f);
         const bool ok = (uint64_t)id < (uint64_t)n_rows;
         const float* src = row_ptr(tab, sv, ok ? id : 0, pitch);
         for (int c = lane; c < chunks; c += 32) ffm_cp16(dst + f * rs + 4 * c, src + 4 * c, ok ? 16 : 0);
@@ -38,10 +41,19 @@ __device__ __forceinline__ void ffm_issue_rows(float* dst, int64_t my_id, const 
     ffm_commit();
 }
 
+// smem bytes of a CTA of `warps` warps with `nbuf` [F][rs] stage buffers each, the pair tables and the partner table
+static inline size_t ffm_smem_bytes(int warps, int nbuf, int fields, int rs) {
+    const size_t npair = (size_t)fields * (fields - 1) / 2;
+    return (size_t)warps * nbuf * fields * rs * sizeof(float) + 2 * npair + 2 + (size_t)fields * rs;
+}
+
 // VEC: latent, emb_col and lin_col even -- a float2 of a partner row never straddles two column blocks, so the partner rows are
 // written as coalesced 8-byte stores driven by a per-block table (built once: no divisions in the per-sample loop).
-template <bool VEC>
-__global__ void __launch_bounds__(FFM_WARPS * 32)
+// WARPS samples per CTA, each warp with NBUF stage buffers; F64: fields up to 64 (two ids per lane).  <VEC, 2, 2, false> serves
+// F <= 32 at up to 200 KB; the others (one warp, double- or single-buffered) serve the shapes it cannot hold.  A sample's
+// arithmetic (lane-strided pair loop, butterfly) is the same in every variant, so its logit has the same bits in each.
+template <bool VEC, int WARPS, int NBUF, bool F64>
+__global__ void __launch_bounds__(WARPS * 32)
 ffm_fwd_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tab, const __grid_constant__ ShardView sv,
                int64_t n_rows, int pitch, int rs,
                int lin_col, int emb_col, const float* __restrict__ bias, float* __restrict__ logit,
@@ -50,11 +62,10 @@ ffm_fwd_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tab, c
     extern __shared__ __align__(16) float smem[];
     const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int npair = fields * (fields - 1) / 2;
-    const int chunks = rs >> 2;
-    // two [F][rs] buffers per warp: the rows of the warp's NEXT sample arrive (cp.async) while the current one is reduced and its
-    // partner rows are written -- the gather never waits for the arithmetic and the stores
-    float* buf0 = smem + (size_t)wib * 2 * fields * rs;
-    unsigned char* pi = reinterpret_cast<unsigned char*>(smem + (size_t)FFM_WARPS * 2 * fields * rs);
+    // NBUF = 2: two [F][rs] buffers per warp, the rows of the warp's NEXT sample arrive (cp.async) while the current one is reduced
+    // and its partner rows are written -- the gather never waits for the arithmetic and the stores
+    float* buf0 = smem + (size_t)wib * NBUF * fields * rs;
+    unsigned char* pi = reinterpret_cast<unsigned char*>(smem + (size_t)WARPS * NBUF * fields * rs);
     unsigned char* pj = pi + npair;
     // partner table: for destination float2 e = i * (rs / 2) + q of a sample's partner rows, the source float offset in `stage`
     unsigned short* ptab = reinterpret_cast<unsigned short*>(pj + npair + ((2 * npair) & 1));
@@ -81,23 +92,39 @@ ffm_fwd_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tab, c
     }
     __syncthreads();
     const float b0 = bias ? __ldg(bias) : 0.f;
-    const int64_t warp0 = (int64_t)blockIdx.x * FFM_WARPS + wib;
-    const int64_t nwarps = (int64_t)gridDim.x * FFM_WARPS;
-    // prologue: ids of the first two samples, rows of the first in flight
-    int64_t id_next = -1;
+    const int64_t warp0 = (int64_t)blockIdx.x * WARPS + wib;
+    const int64_t nwarps = (int64_t)gridDim.x * WARPS;
+    // ids of a sample: field `lane` (and `lane + 32` when F64); -1 past the last field
+    auto load_ids = [&](int64_t b, int64_t& lo, int64_t& hi) {
+        lo = (lane < fields) ? __ldg(ids + b * fields + lane) : -1;
+        if constexpr (F64) hi = (lane + 32 < fields) ? __ldg(ids + b * fields + lane + 32) : -1;
+    };
+    int64_t id_next = -1, id_next_hi = -1;
     int cur = 0;
-    if (warp0 < batch) {
-        int64_t id0 = (lane < fields) ? __ldg(ids + warp0 * fields + lane) : -1;
-        ffm_issue_rows(buf0, id0, tab, sv, n_rows, pitch, rs, fields, lane);
-        if (warp0 + nwarps < batch && lane < fields) id_next = __ldg(ids + (warp0 + nwarps) * fields + lane);
+    if constexpr (NBUF == 2) {
+        // prologue: ids of the first two samples, rows of the first in flight
+        if (warp0 < batch) {
+            int64_t id0 = -1, id0_hi = -1;
+            load_ids(warp0, id0, id0_hi);
+            ffm_issue_rows<F64>(buf0, id0, id0_hi, tab, sv, n_rows, pitch, rs, fields, lane);
+            if (warp0 + nwarps < batch) load_ids(warp0 + nwarps, id_next, id_next_hi);
+        }
     }
-    for (int64_t b = warp0; b < batch; b += nwarps, cur ^= 1) {
+    for (int64_t b = warp0; b < batch; b += nwarps, cur ^= (NBUF - 1)) {
         float* stage = buf0 + cur * fields * rs;
-        const bool more = b + nwarps < batch;                              // warp-uniform
-        if (more) ffm_issue_rows(buf0 + (cur ^ 1) * fields * rs, id_next, tab, sv, n_rows, pitch, rs, fields, lane);
-        id_next = -1;
-        if (b + 2 * nwarps < batch && lane < fields) id_next = __ldg(ids + (b + 2 * nwarps) * fields + lane);
-        if (more) ffm_wait<1>(); else ffm_wait<0>();
+        if constexpr (NBUF == 2) {
+            const bool more = b + nwarps < batch;                          // warp-uniform
+            if (more) ffm_issue_rows<F64>(buf0 + (cur ^ 1) * fields * rs, id_next, id_next_hi, tab, sv, n_rows, pitch, rs, fields, lane);
+            id_next = -1;
+            id_next_hi = -1;
+            if (b + 2 * nwarps < batch) load_ids(b + 2 * nwarps, id_next, id_next_hi);
+            if (more) ffm_wait<1>(); else ffm_wait<0>();
+        } else {                                                           // one buffer: this sample's rows, then its arithmetic
+            int64_t id = -1, id_hi = -1;
+            load_ids(b, id, id_hi);
+            ffm_issue_rows<F64>(stage, id, id_hi, tab, sv, n_rows, pitch, rs, fields, lane);
+            ffm_wait<0>();
+        }
         __syncwarp();
         // ---- first order + pair dots
         float acc = 0.f;
@@ -158,7 +185,7 @@ extern "C" int rlctr_ffm_fwd(const int64_t* ids, const rlctr_table* table, const
                              float* pctr, int64_t pctr_stride, float* partners, int64_t batch, int32_t fields,
                              int32_t latent, rlctr_stream_t stream) {
     if (!ids || !table || !table->data || table->n_rows <= 0 || batch < 0) return RLCTR_EINVAL;
-    if (fields < 2 || fields > 255 || latent <= 0) return RLCTR_EUNSUPPORTED;
+    if (fields < 2 || fields > 64 || latent <= 0) return RLCTR_EUNSUPPORTED;   // a lane holds the ids of fields lane, lane + 32
     const int rs = table->row_stride;
     if (rs % 4 != 0 || table->dim != fields * latent || table->emb_col < 0 ||
         table->emb_col + table->dim > rs || table->lin_col >= rs)
@@ -168,28 +195,64 @@ extern "C" int rlctr_ffm_fwd(const int64_t* ids, const rlctr_table* table, const
     if (batch == 0) return RLCTR_OK;
     ShardView sv;
     if (!shard_view_of(table, &sv)) return RLCTR_EUNSUPPORTED;
-    const int npair = fields * (fields - 1) / 2;
     const bool vec = (latent % 2 == 0) && (table->emb_col % 2 == 0) && (table->lin_col < 0 || table->lin_col % 2 == 0) &&
                      (size_t)fields * rs < 0xfff0u;
-    if (fields > 32) return RLCTR_EUNSUPPORTED;                          // one lane per field holds the sample's ids
-    const size_t smem = (size_t)FFM_WARPS * 2 * fields * rs * sizeof(float) + 2 * (size_t)npair + 2 + (size_t)fields * rs;
-    if (smem > 200 * 1024) return RLCTR_EUNSUPPORTED;
-    RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    int64_t want = (batch + FFM_WARPS - 1) / FFM_WARPS;
-    int per_sm = (int)((size_t)(220 * 1024) / (smem + 1024));
+    const int pitch = table->row_pitch > 0 ? table->row_pitch : rs;
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t smem = ffm_smem_bytes(2, 2, fields, rs);
+    if (fields <= 32 && smem <= 200 * 1024) {
+        RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<true, 2, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<false, 2, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        int64_t want = (batch + 1) / 2;
+        int per_sm = (int)((size_t)(220 * 1024) / (smem + 1024));
+        if (per_sm < 1) per_sm = 1;
+        if (per_sm > 16) per_sm = 16;
+        const int64_t cap = (int64_t)RLCTR_SMS * per_sm;
+        const int grid = (int)(want < cap ? want : cap);
+        if (vec)
+            ffm_fwd_kernel<true, 2, 2, false><<<grid, 64, smem, st>>>(ids, table->data, sv, table->n_rows, pitch, rs, table->lin_col,
+                                                                     table->emb_col, bias, logit, pctr, pctr_stride, partners, batch,
+                                                                     fields, latent);
+        else
+            ffm_fwd_kernel<false, 2, 2, false><<<grid, 64, smem, st>>>(ids, table->data, sv, table->n_rows, pitch, rs, table->lin_col,
+                                                                      table->emb_col, bias, logit, pctr, pctr_stride, partners, batch,
+                                                                      fields, latent);
+        RLCTR_LAUNCH_CHECK();
+        return RLCTR_OK;
+    }
+    // Shapes the two-warp kernel cannot hold: F = 33..64, or stage buffers past 200 KB.  One warp per CTA, so a CTA takes the least
+    // shared memory one sample needs; double-buffered where two buffers fit in 227 KB, else single-buffered (one [F][rs] buffer of
+    // a row of at most 512 floats is 128 KB at F = 64).  The opt-in is set once per device (not per launch, which may be captured).
+    const int nbuf = ffm_smem_bytes(1, 2, fields, rs) <= 227 * 1024 ? 2 : 1;
+    const size_t smem1 = ffm_smem_bytes(1, nbuf, fields, rs);
+    if (smem1 > 227 * 1024) return RLCTR_EUNSUPPORTED;
+    int dev = 0;
+    RLCTR_CUDA(cudaGetDevice(&dev));
+    static bool opted[2][2][64] = {};
+    bool& done = opted[vec][nbuf - 1][dev & 63];
+    if (!done) {
+        if (vec && nbuf == 2)
+            RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<true, 1, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        else if (vec)
+            RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<true, 1, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        else if (nbuf == 2)
+            RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<false, 1, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        else
+            RLCTR_CUDA(cudaFuncSetAttribute(ffm_fwd_kernel<false, 1, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+        done = true;
+    }
+    int per_sm = (int)((size_t)(228 * 1024) / (smem1 + 1024));     // 228 KB of shared memory per SM, 1 KB reserved per CTA
     if (per_sm < 1) per_sm = 1;
-    if (per_sm > 16) per_sm = 16;
+    if (per_sm > 32) per_sm = 32;
     const int64_t cap = (int64_t)RLCTR_SMS * per_sm;
-    const int grid = (int)(want < cap ? want : cap);
-    if (vec)
-        ffm_fwd_kernel<true><<<grid, FFM_WARPS * 32, smem, (cudaStream_t)stream>>>(
-            ids, table->data, sv, table->n_rows, table->row_pitch > 0 ? table->row_pitch : rs, rs, table->lin_col, table->emb_col,
-            bias, logit, pctr, pctr_stride, partners, batch, fields, latent);
-    else
-        ffm_fwd_kernel<false><<<grid, FFM_WARPS * 32, smem, (cudaStream_t)stream>>>(
-            ids, table->data, sv, table->n_rows, table->row_pitch > 0 ? table->row_pitch : rs, rs, table->lin_col, table->emb_col,
-            bias, logit, pctr, pctr_stride, partners, batch, fields, latent);
+    const int grid = (int)(batch < cap ? batch : cap);
+#define LAUNCH_FFM1(V, NB)                                                                                                     \
+    ffm_fwd_kernel<V, 1, NB, true><<<grid, 32, smem1, st>>>(ids, table->data, sv, table->n_rows, pitch, rs, table->lin_col,    \
+                                                            table->emb_col, bias, logit, pctr, pctr_stride, partners, batch,   \
+                                                            fields, latent)
+    if (vec) { if (nbuf == 2) LAUNCH_FFM1(true, 2); else LAUNCH_FFM1(true, 1); }
+    else { if (nbuf == 2) LAUNCH_FFM1(false, 2); else LAUNCH_FFM1(false, 1); }
+#undef LAUNCH_FFM1
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
 }
