@@ -455,6 +455,43 @@ int rlctr_steps_advance(int32_t* steps, const int32_t* step_index, int32_t count
 int rlctr_step_advance(int32_t* step, int32_t delta, rlctr_stream_t stream);
 
 /* ------------------------------------------------------------------------------------
+ * torch.optim.Adagrad (torch/optim/adagrad.py, _single_tensor_adagrad) over the same tables, records and gradient side as the
+ * Adam calls above.  Per element, at step t:
+ *     clr = lr / (1 + (t - 1) * lr_decay);  g += weight_decay * p;  s += g * g;  p += -clr * g / (sqrt(s) + eps)
+ * The state sum s lives where rlctr_adam.exp_avg would (the second block of a [p | exp_avg | exp_avg_sq] record); the third block
+ * is never read or written.  `clr[t]` is torch's Python-double clr of step t cast to fp32 (entry 0 unused).  With
+ * weight_decay == 0 a row no sample touched is exactly unchanged by a dense step, so no stamp is needed (stamp == NULL and
+ * stamp_col < 0): the update then replays nothing, and rlctr_adagrad_catchup / rlctr_adagrad_flush are not called.  With
+ * weight_decay > 0 the stamps work as for Adam: catch-up and flush replay the missed L2-only steps g = weight_decay * p.
+ * Each call has the argument checks and shape limits of the Adam call it mirrors.
+ * ------------------------------------------------------------------------------------ */
+typedef struct rlctr_adagrad {
+    float*         state_sum;    /* [n_rows, row_stride] at the table's row_pitch */
+    int32_t*       stamp;        /* as rlctr_adam.stamp; NULL with stamp_col < 0: no lazy bookkeeping */
+    const float*   clr;          /* [sched_len], index = step (entry 0 unused) */
+    const int32_t* step;         /* device scalar: completed steps t; update kernels apply step t+1 */
+    int32_t        sched_len;
+    int32_t        stamp_col;    /* as rlctr_adam.stamp_col */
+    double         eps, weight_decay;
+} rlctr_adagrad;
+int rlctr_rows_adagrad(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n,
+                       const rlctr_rowgrad* grad, const rlctr_table* table, const rlctr_adagrad* opt,
+                       void* ws, size_t ws_bytes, rlctr_stream_t stream);
+int rlctr_group_rows_adagrad(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_table* table,
+                             const rlctr_adagrad* opt, const rlctr_member* members, int32_t n_members, const float* sums,
+                             int32_t sums_pitch, int32_t fields, int32_t world, const uint32_t* slot_of, void* ws, size_t ws_bytes,
+                             rlctr_stream_t stream);
+int rlctr_adagrad_catchup(const uint32_t* sorted_ids, int64_t n, const rlctr_table* table, const rlctr_adagrad* opt,
+                          rlctr_stream_t stream);
+int rlctr_adagrad_flush(const rlctr_table* table, const rlctr_adagrad* opt, int64_t row_begin, int64_t row_end,
+                        rlctr_stream_t stream);
+/* Dense Adagrad for up to RLCTR_DENSE_MAX replicated tensors in one launch, per-tensor step counters as rlctr_dense_adam_multi;
+ * IEEE sqrt and division (torch's numbers element for element). */
+int rlctr_dense_adagrad_multi(float* const* params, const float* const* grads, float* const* state_sums, const int64_t* sizes,
+                              int32_t count, const float* clr, const int32_t* steps, const int32_t* step_index, double eps,
+                              double weight_decay, rlctr_stream_t stream);
+
+/* ------------------------------------------------------------------------------------
  * K6  ensemble scoring + reward: generate_preds.
  *   variant 0: src/all_main/main.py:183-271 (action in 2..M, reward +1/-1)
  *   variant 1: src/all_main/hybrid_td3_main_per.py:56-133 (action in 1..M, reward 1/0)

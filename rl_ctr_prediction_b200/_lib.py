@@ -46,6 +46,12 @@ class Adam(C.Structure):
                 ("stage", C.c_void_p)]
 
 
+class Adagrad(C.Structure):
+    """struct rlctr_adagrad"""
+    _fields_ = [("state_sum", C.c_void_p), ("stamp", C.c_void_p), ("clr", C.c_void_p), ("step", C.c_void_p),
+                ("sched_len", C.c_int32), ("stamp_col", C.c_int32), ("eps", C.c_double), ("weight_decay", C.c_double)]
+
+
 class Lookup(C.Structure):
     """struct rlctr_lookup"""
     _fields_ = [("stage", C.c_void_p), ("world", C.c_int32), ("n_per_rank", C.c_uint32), ("gathered", C.c_void_p * 8)]
@@ -72,6 +78,7 @@ RLCTR_GROUP_MAX = 4
 _P, _I64, _I32, _SZ, _F = C.c_void_p, C.c_int64, C.c_int32, C.c_size_t, C.c_double
 _TP, _AP, _GP, _LP = C.POINTER(Table), C.POINTER(Adam), C.POINTER(RowGrad), C.POINTER(Lookup)
 _MP = C.POINTER(Member)
+_AGP = C.POINTER(Adagrad)
 
 # name -> (restype, argtypes); must list every symbol include/rlctr.h declares
 SIGNATURES = {
@@ -129,6 +136,11 @@ SIGNATURES = {
     "rlctr_dense_adam_multi": (C.c_int, [_P, _P, _P, _P, _P, _I32, _P, _P, _P, _F, _F, _F, _F, _P]),
     "rlctr_steps_advance": (C.c_int, [_P, _P, _I32, _P]),
     "rlctr_step_advance": (C.c_int, [_P, _I32, _P]),
+    "rlctr_rows_adagrad": (C.c_int, [_P, _P, _I64, _GP, _TP, _AGP, _P, _SZ, _P]),
+    "rlctr_group_rows_adagrad": (C.c_int, [_P, _P, _I64, _TP, _AGP, _MP, _I32, _P, _I32, _I32, _I32, _P, _P, _SZ, _P]),
+    "rlctr_adagrad_catchup": (C.c_int, [_P, _I64, _TP, _AGP, _P]),
+    "rlctr_adagrad_flush": (C.c_int, [_TP, _AGP, _I64, _I64, _P]),
+    "rlctr_dense_adagrad_multi": (C.c_int, [_P, _P, _P, _P, _I32, _P, _P, _P, _F, _F, _P]),
     "rlctr_generate_preds": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _I64, _I32, _I32, _P]),
     "rlctr_generate_preds_v10_ws_bytes": (_SZ, [_I64]),
     "rlctr_generate_preds_v10": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I64, _I32, _P, _SZ, _P]),
@@ -181,6 +193,11 @@ SHAPE_LIMITS = {
     "rlctr_group_rows_adam": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats",
     "rlctr_rows_catchup": "records with an in-record stamp: rows of at most 128 floats",
     "rlctr_adam_flush": "records with an in-record stamp: rows of at most 128 floats",
+    "rlctr_rows_adagrad": "fused rows of at most 512 floats (FFM: F*D + 1 <= 512)",
+    "rlctr_group_rows_adagrad": "joint rows of at most 128 floats (four 128-byte lines), members' stand-alone rows of at most 36 floats",
+    "rlctr_adagrad_catchup": "records with an in-record stamp: rows of at most 128 floats",
+    "rlctr_adagrad_flush": "records with an in-record stamp: rows of at most 128 floats",
+    "rlctr_dense_adagrad_multi": "at most RLCTR_DENSE_MAX (24) tensors per call",
 }
 
 

@@ -189,7 +189,7 @@ def _member_view(m, rec, col, wide):
 class _GroupStep:
     """The parts of a group step that do not depend on where the joint table lives, shared by ColocatedCTR (one device) and
     sharded.ShardedGroup (row-sharded).  The class provides ``members``, ``_cols``, ``_geom``, ``table``, ``_meta``,
-    ``_reduce_ws``, ``_rows_ws``, ``_global_struct()`` (the table as the gathers read it) and ``_UPDATE_KEY``."""
+    ``_reduce_ws``, ``_rows_ws``, ``_global_struct()`` (the table as the gathers read it) and ``_UPDATE_TAG``."""
 
     def _member_structs(self, B, F, dev, train, pctr=None):
         """The members' views for rlctr_group_fwd.  logits[i]: the table part of member i's logit (bias + first order + FM
@@ -249,7 +249,7 @@ class _GroupStep:
         return losses, dlogits, extras
 
     def _group_update(self, stash, opt_state, st):
-        """optim.Adam.step() for the joint table: rlctr_group_rows_adam."""
+        """The optimizer step for the joint table: rlctr_group_rows_adam / rlctr_group_rows_adagrad."""
         lib = _lib.load()
         M = len(self.members)
         arr = (_lib.Member * M)()
@@ -261,13 +261,11 @@ class _GroupStep:
             s.dlogit = _lib.ptr(stash.dlogit[i])
             s.extra = _lib.ptr(stash.extra[i])
             s.extra_pitch = pitches[i]
-        t, a = table_struct(self.table.data, self._geom), opt_state.struct()
         ws_bytes = lib.rlctr_rows_ws_bytes(stash.n)
         ws = self._rows_ws(ws_bytes)
-        _lib.call("rlctr_group_rows_adam", lib.rlctr_group_rows_adam, _lib.ptr(stash.sorted_ids), _lib.ptr(stash.sorted_slots),
-                  stash.n, C.byref(t), C.byref(a), arr, M, _lib.ptr(stash.sums), stash.sums_pitch, stash.fields, stash.world,
-                  _lib.ptr(stash.slot_of), _lib.ptr(ws), ws_bytes, st, key=self._UPDATE_KEY,
-                  meta=self._meta(stash.n // stash.fields, stash.fields))
+        opt_state.group_update(stash.sorted_ids, stash.sorted_slots, stash.n, table_struct(self.table.data, self._geom), arr, M,
+                               stash.sums, stash.sums_pitch, stash.fields, stash.world, stash.slot_of, ws, ws_bytes, st,
+                               self._UPDATE_TAG, self._meta(stash.n // stash.fields, stash.fields))
 
 
 class ColocatedCTR(_GroupStep, Model._TableModel):
@@ -276,7 +274,7 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
     ``load_state_dict`` (reference keys) and their dense parameters."""
 
     _kind = "group"
-    _UPDATE_KEY = "rlctr_group_rows_adam"
+    _UPDATE_TAG = None
 
     def __init__(self, models, max_lines=1):
         super().__init__()
@@ -359,7 +357,8 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
         lib = _lib.load()
         opt = self._opt
         if opt is None:
-            raise _lib.RlctrError("build rl_ctr_prediction_b200.optim.Adam(group.parameters(), ...) before training the group")
+            raise _lib.RlctrError("build rl_ctr_prediction_b200.optim.Adam(group.parameters(), ...) (or optim.Adagrad) before "
+                                  "training the group")
         x = Model._check_ids(x)
         B, F = x.shape
         dev, st, g = x.device, _lib.stream(), self._geom
@@ -369,7 +368,7 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
         # order (rlctr_rows_catchup_ids: a claim bit per row tells the occurrences of an id apart) the sort runs on its own
         # stream -- a parallel branch of a captured step -- beside catch-up, gather and tower instead of in front of them.
         side = None
-        if UNSORTED_CATCHUP and opt.lazy and opt.stamp_col >= 0 and 5 <= (g.used + 3) // 4 <= 8:    # joint records of 5..8 chunks
+        if UNSORTED_CATCHUP and opt.catchup_ids_ok and opt.lazy and opt.stamp_col >= 0 and 5 <= (g.used + 3) // 4 <= 8:
             cur = torch.cuda.current_stream(dev)
             side = self._sort_stream
             if side is None or side.device != dev:
@@ -386,10 +385,7 @@ class ColocatedCTR(_GroupStep, Model._TableModel):
                           _lib.ptr(self._claim), cb, st, key="rlctr_rows_catchup[group]", meta=self._meta(B, F))
         else:
             sid, sslot = Model.sort_ids(x, g.n_rows)
-            if opt.lazy and opt.dirty:
-                a = opt.struct()
-                _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(sid), x.numel(), C.byref(t), C.byref(a), st,
-                          key="rlctr_rows_catchup[group]", meta=self._meta(B, F))
+            opt.catchup(t, sid, x.numel(), "group", self._meta(B, F))
         M = len(self.members)
         arr, logits, rows = self._member_structs(B, F, dev, True)
         sums = torch.empty(B, g.row_stride, dtype=torch.float32, device=dev)

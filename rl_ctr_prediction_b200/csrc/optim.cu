@@ -276,8 +276,68 @@ __device__ __forceinline__ void adam_apply4(float4& p, float4& m, float4& v, con
     adam_elem_fast(p.w, m.w, v.w, g.w, h, s.x, ib);
 }
 
+// The per-record update of the row kernels is a policy: the gradient side (run walk, long-run tree, co-located roles, peer reads,
+// routed slots) is shared, the step applied to the reduced gradient is AdamStep or AdagradStep.  Both see the record through an
+// AdamView: for Adagrad `m` is the state sum, `v` is never touched (TWO == false), `sched` points at the fp32 clr table and
+// `h` carries only eps and weight_decay.  coef(t) is the per-step scalar pair the step needs.
+struct AdamStep {
+    static constexpr bool TWO = true;                    // the record's third block (exp_avg_sq) is read and written
+    __device__ static __forceinline__ float2 coef(const float2* __restrict__ sched, int t) { return __ldg(&sched[t]); }
+    __device__ static __forceinline__ void apply4(float4& p, float4& m, float4& v, const float4& g, float2 s, const AdamHyper& h) {
+        adam_apply4(p, m, v, g, s, h);
+    }
+    __device__ static __forceinline__ void l2_step4(float4& p, float4& m, float4& v, float2 s, const AdamHyper& h) {
+        adam_l2_step4(p, m, v, s, h);
+    }
+    __device__ static __forceinline__ void replay4(float4& p, float4& m, float4& v, int from, int to, const float2* __restrict__ sched,
+                                                   const AdamHyper& h) {
+        adam_replay4(p, m, v, from, to, sched, h);
+    }
+    __device__ static __forceinline__ void apply1(float& p, float& m, float& v, float g, float2 s, const AdamHyper& h) {
+        adam_elem_fast(p, m, v, g, h, s.x, rcp_approx(s.y));
+    }
+    __device__ static __forceinline__ void replay1(float& p, float& m, float& v, int from, int to, const float2* __restrict__ sched,
+                                                   const AdamHyper& h) {
+        adam_replay1(p, m, v, from, to, sched, h);
+    }
+};
+// torch.optim.Adagrad on a table element: sqrt(s) and the division by (sqrt(s) + eps) on the SFU (MUFU.SQRT, MUFU.RCP), the form
+// of adam_elem_fast; the L2-only step is this step with g = 0 (fmaf(wd, p, 0) == wd * p), so the lazy replay and a dense step give
+// the same bits.  Dense parameters keep IEEE sqrt and division (dense_adagrad_multi_kernel).
+__device__ __forceinline__ void adagrad_elem_fast(float& p, float& s, float g, float clr, const AdamHyper& h) {
+    g = fmaf(h.wd, p, g);
+    s = fmaf(g, g, s);
+    p = fmaf(-clr * g, rcp_approx(sqrt_approx(s) + h.eps), p);
+}
+struct AdagradStep {
+    static constexpr bool TWO = false;
+    __device__ static __forceinline__ float2 coef(const float2* __restrict__ sched, int t) {
+        return make_float2(__ldg(reinterpret_cast<const float*>(sched) + t), 0.f);
+    }
+    __device__ static __forceinline__ void apply4(float4& p, float4& s, float4&, const float4& g, float2 c, const AdamHyper& h) {
+        adagrad_elem_fast(p.x, s.x, g.x, c.x, h);
+        adagrad_elem_fast(p.y, s.y, g.y, c.x, h);
+        adagrad_elem_fast(p.z, s.z, g.z, c.x, h);
+        adagrad_elem_fast(p.w, s.w, g.w, c.x, h);
+    }
+    __device__ static __forceinline__ void l2_step4(float4& p, float4& s, float4& v, float2 c, const AdamHyper& h) {
+        apply4(p, s, v, f4zero(), c, h);
+    }
+    __device__ static __forceinline__ void replay4(float4& p, float4& s, float4& v, int from, int to, const float2* __restrict__ sched,
+                                                   const AdamHyper& h) {
+        for (int t = from + 1; t <= to; ++t) l2_step4(p, s, v, coef(sched, t), h);
+    }
+    __device__ static __forceinline__ void apply1(float& p, float& s, float&, float g, float2 c, const AdamHyper& h) {
+        adagrad_elem_fast(p, s, g, c.x, h);
+    }
+    __device__ static __forceinline__ void replay1(float& p, float& s, float& v, int from, int to, const float2* __restrict__ sched,
+                                                   const AdamHyper& h) {
+        for (int t = from + 1; t <= to; ++t) apply1(p, s, v, 0.f, coef(sched, t), h);
+    }
+};
+
 // finish one distinct row: Adam (APPLY==0) or store into the dense gradient (APPLY==1)
-template <int APPLY>
+template <int APPLY, class P = AdamStep>
 __device__ __forceinline__ void finish_row(int64_t id, int col0, float4 p, const float4& acc, const TableView& t,
                                            const AdamView& a, float* dense_grad, int step, int stamp_in,
                                            const float4* m_pre = nullptr, const float4* v_pre = nullptr) {
@@ -286,17 +346,18 @@ __device__ __forceinline__ void finish_row(int64_t id, int col0, float4 p, const
         return;
     }
     const int64_t off = id * t.pitch + col0;
-    float4 m = m_pre ? *m_pre : ld4(a.m + off), v = v_pre ? *v_pre : ld4(a.v + off);
-    if (is_lazy(a) && !a.stage && stamp_in < step - 1) adam_replay4(p, m, v, stamp_in, step - 1, a.sched, a.h);
-    adam_apply4(p, m, v, acc, __ldg(&a.sched[step]), a.h);
+    float4 m = m_pre ? *m_pre : ld4(a.m + off), v = f4zero();
+    if (P::TWO) v = v_pre ? *v_pre : ld4(a.v + off);
+    if (is_lazy(a) && !a.stage && stamp_in < step - 1) P::replay4(p, m, v, stamp_in, step - 1, a.sched, a.h);
+    P::apply4(p, m, v, acc, P::coef(a.sched, step), a.h);
     embed_stamp(p, col0, a, step);
     st4(t.data + off, p);
     st4(a.m + off, m);
-    st4(a.v + off, v);
+    if (P::TWO) st4(a.v + off, v);
 }
 
 // one lane-group (LPR lanes, a float4 chunk each) per sorted position; only run heads work
-template <int LPR, int APPLY, bool GROUP = false>
+template <int LPR, int APPLY, bool GROUP = false, class P = AdamStep>
 __global__ void __launch_bounds__(256, (LPR > 8 ? 4 : 5))      // 16 / 32 lanes: wide co-located records, 64 registers: no spills
 rows_short_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                   const __grid_constant__ GradView g, TableView t, AdamView a, float* __restrict__ dense_grad,
@@ -345,7 +406,7 @@ rows_short_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __res
             p = ldg4(sp); m0 = ldg4(sp + blk); v0 = ldg4(sp + 2 * blk);
         } else {
             p = ld4(t.data + off);                       // issued with m, v: one contiguous record when pitch = 3*rs
-            if (APPLY == 0) { m0 = ld4(a.m + off); v0 = ld4(a.v + off); }
+            if (APPLY == 0) { m0 = ld4(a.m + off); if (P::TWO) v0 = ld4(a.v + off); }
         }
         float4 acc = rowgrad_any<GROUP>(g, gl, slot0, col0, p, t);
         int64_t kk = k + 1;
@@ -357,8 +418,8 @@ rows_short_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __res
             acc = f4add(acc, rowgrad_any<GROUP>(g, gl, slot, col0, p, t));
         }
         if (APPLY == 0 && a.stamp_col >= 0 && !staged) __syncwarp(__activemask());   // every chunk lane has read the in-record stamp
-        finish_row<APPLY>(id, col0, p, acc, t, a, dense_grad, step, stamp_in, &m0, &v0);
-    } else if (APPLY == 0 && a.stage != nullptr && head && col0 < t.rs) {
+        finish_row<APPLY, P>(id, col0, p, acc, t, a, dense_grad, step, stamp_in, &m0, &v0);
+    } else if (P::TWO && APPLY == 0 && a.stage != nullptr && head && col0 < t.rs) {      // (the staging array is Adam's)
         // staged update: the record was NOT read by this kernel, so its lines are not in L2.  Writing only the active chunks
         // would leave half-written 32-byte sectors that L2 has to fill from DRAM first (ncu: +94 MB of reads per launch);
         // the padding chunks are zero by construction (p = m = v = 0 stays 0 under Adam), so write them too: whole 64 B blocks.
@@ -580,7 +641,7 @@ rows_staged_tile_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t*
 // (, h+6), so each load instruction of the pair covers one whole 32-byte sector of each block -- and does the bookkeeping once
 // for 12-16 columns: 16 records per warp instead of 4, no idle lanes, ~2x the records in flight per register.  Same arithmetic
 // as the eight-lane kernel, column by column (group_col_grad, adam_apply4): bit-identical results.
-template <int CH>
+template <int CH, class P = AdamStep>
 __global__ void __launch_bounds__(256, 2)
 group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                    const __grid_constant__ GradView g, const __grid_constant__ TableView t, const __grid_constant__ AdamView a,
@@ -611,7 +672,7 @@ group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
     const int sc5 = a.stamp_col >= 0 ? (a.stamp_col >> 2) : 0;         // chunk that holds the in-record stamp
     const int stamp_src = (lane & ~1) + (sc5 & 1), stamp_j = sc5 >> 1;
     const int step = __ldg(a.step) + 1;
-    const float2 sc = __ldg(&a.sched[step]);
+    const float2 sc = P::coef(a.sched, step);
     const int64_t G = ((int64_t)gridDim.x * blockDim.x) >> 1;
     for (int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1; k < n; k += G) {
         const uint32_t id = __ldg(sorted_ids + k);
@@ -630,7 +691,7 @@ group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
 #pragma unroll
         for (int j = 0; j < CH; ++j) {
             p[j] = f4zero(); m[j] = f4zero(); v[j] = f4zero(); acc[j] = f4zero();
-            if (live[j]) { p[j] = ld4(t.data + off + 8 * j); m[j] = ld4(a.m + off + 8 * j); v[j] = ld4(a.v + off + 8 * j); }
+            if (live[j]) { p[j] = ld4(t.data + off + 8 * j); m[j] = ld4(a.m + off + 8 * j); if (P::TWO) v[j] = ld4(a.v + off + 8 * j); }
         }
         int64_t kk = k;
         bool first = true;
@@ -678,18 +739,18 @@ group_rows2_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
 #pragma unroll
         for (int j = 0; j < CH; ++j) {
             if (!live[j]) continue;
-            if (a.stamp_col >= 0 && stamp_in < step - 1) adam_replay4(p[j], m[j], v[j], stamp_in, step - 1, a.sched, a.h);
-            adam_apply4(p[j], m[j], v[j], acc[j], sc, a.h);
+            if (a.stamp_col >= 0 && stamp_in < step - 1) P::replay4(p[j], m[j], v[j], stamp_in, step - 1, a.sched, a.h);
+            P::apply4(p[j], m[j], v[j], acc[j], sc, a.h);
             embed_stamp(p[j], 4 * (h + 2 * j), a, step);
             st4(t.data + off + 8 * j, p[j]);
             st4(a.m + off + 8 * j, m[j]);
-            st4(a.v + off + 8 * j, v[j]);
+            if (P::TWO) st4(a.v + off + 8 * j, v[j]);
         }
     }
 }
 
 // block per long run: NSUB lane-groups stride the run, fixed-shape tree in shared memory
-template <int LPR, int APPLY, bool GROUP = false, int NT = 256>
+template <int LPR, int APPLY, bool GROUP = false, int NT = 256, class P = AdamStep>
 __global__ void __launch_bounds__(NT)
 rows_long_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                  const __grid_constant__ GradView g, TableView t, AdamView a, float* __restrict__ dense_grad,
@@ -735,17 +796,17 @@ rows_long_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __rest
             __syncthreads();
         }
         if (sub == 0 && chunk_on) {
-            if (staged) {
+            if (P::TWO && staged) {                      // (the staging array is Adam's)
                 if (col0 < a.stage_pitch / 3) {          // padding chunks carry no parameters: they are never touched
                     const int blk = a.stage_pitch / 3;
                     const float4 m0 = ldg4(sp + blk), v0 = ldg4(sp + 2 * blk);
-                    finish_row<APPLY>(id, col0, p, red[threadIdx.x], t, a, dense_grad, step, stamp_in, &m0, &v0);
+                    finish_row<APPLY, P>(id, col0, p, red[threadIdx.x], t, a, dense_grad, step, stamp_in, &m0, &v0);
                 } else {                                  // whole 64 B blocks (see rows_short_kernel)
                     const int64_t off = (int64_t)id * t.pitch + col0;
                     st4(t.data + off, f4zero()); st4(a.m + off, f4zero()); st4(a.v + off, f4zero());
                 }
             } else {
-                finish_row<APPLY>(id, col0, p, red[threadIdx.x], t, a, dense_grad, step, stamp_in);
+                finish_row<APPLY, P>(id, col0, p, red[threadIdx.x], t, a, dense_grad, step, stamp_in);
             }
         }
         __syncthreads();
@@ -758,6 +819,7 @@ rows_long_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __rest
 // stand-alone update and pairs them in that kernel's tree: 64 sub-groups for a 16-float row (rows_long_kernel<4>), 32 for 20..32
 // floats (rows_long_kernel<8>), one walked in slot order for 36 floats (rows_wide_kernel).  Same per-column arithmetic
 // (group_col_grad) and the same Adam step: bit-identical to each member's stand-alone update.
+template <class P = AdamStep>
 __global__ void __launch_bounds__(256)
 group_long_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                        const __grid_constant__ GradView g, const __grid_constant__ TableView t, const __grid_constant__ AdamView a,
@@ -808,7 +870,7 @@ group_long_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* 
             }
             __syncthreads();
         }
-        if (s0 == 0 && chunk_on) finish_row<0>(id, col0, p, red[c], t, a, nullptr, step, stamp_in);
+        if (s0 == 0 && chunk_on) finish_row<0, P>(id, col0, p, red[c], t, a, nullptr, step, stamp_in);
         __syncthreads();
         if (a.stamp && threadIdx.x == 0) a.stamp[id] = step;      // a separate stamp array (the in-record stamp rides in p)
     }
@@ -819,7 +881,7 @@ group_long_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* 
 // in slot order so the sum is bit-identical from run to run.  WCH = 2: rows up to 256 floats; WCH = 4: up to 512
 // (FFM at F = 15, D = 18..33).
 constexpr int WCH_MAX = 4;
-template <int APPLY, int WCH>
+template <int APPLY, int WCH, class P = AdamStep>
 __global__ void __launch_bounds__(256)
 rows_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                  GradView g, TableView t, AdamView a, float* __restrict__ dense_grad) {
@@ -857,7 +919,7 @@ rows_wide_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __rest
 #pragma unroll
     for (int u = 0; u < WCH; ++u) {
         const int c = lane + 32 * u;
-        if (c < chunks) finish_row<APPLY>(id, 4 * c, p[u], acc[u], t, a, dense_grad, step, stamp_in);
+        if (c < chunks) finish_row<APPLY, P>(id, 4 * c, p[u], acc[u], t, a, dense_grad, step, stamp_in);
     }
     if (APPLY == 0 && a.stamp) {
         __syncwarp();
@@ -876,7 +938,7 @@ struct ReplayItem {
     int t;               // steps already applied
 };
 // FLUSH: items are all chunks of rows [r0, r1).  CATCHUP: items are (sorted position, chunk); only run heads count.
-template <bool CATCHUP>
+template <bool CATCHUP, class P = AdamStep>
 __device__ __forceinline__ void replay_fetch(ReplayItem& it, int64_t k, int c, int64_t n_items, const TableView& t,
                                              const AdamView& a, int64_t r0, const uint32_t* __restrict__ sorted_ids,
                                              int upto) {
@@ -897,9 +959,9 @@ __device__ __forceinline__ void replay_fetch(ReplayItem& it, int64_t k, int c, i
     it.off = row * t.pitch + 4 * c;
     it.p = ld4(t.data + it.off);
     it.m = ld4(a.m + it.off);
-    it.v = ld4(a.v + it.off);
+    it.v = P::TWO ? ld4(a.v + it.off) : f4zero();
 }
-template <bool CATCHUP>
+template <bool CATCHUP, class P = AdamStep>
 __global__ void __launch_bounds__(256)
 replay_kernel(TableView t, AdamView a, int64_t r0, int64_t n_items, const uint32_t* __restrict__ sorted_ids) {
     const int chunks = (t.used + 3) >> 2;                 // trailing all-padding chunks are never touched
@@ -910,26 +972,26 @@ replay_kernel(TableView t, AdamView a, int64_t r0, int64_t n_items, const uint32
     int64_t k = i0 / chunks;                              // (k, c) = item index / chunks, % chunks, advanced incrementally
     int c = (int)(i0 % chunks);
     ReplayItem cur, nxt;
-    replay_fetch<CATCHUP>(cur, k, c, n_items, t, a, r0, sorted_ids, upto);
+    replay_fetch<CATCHUP, P>(cur, k, c, n_items, t, a, r0, sorted_ids, upto);
     bool cur_real = k < n_items;
     k += dk; c += dc; if (c >= chunks) { c -= chunks; ++k; }
-    replay_fetch<CATCHUP>(nxt, k, c, n_items, t, a, r0, sorted_ids, upto);
+    replay_fetch<CATCHUP, P>(nxt, k, c, n_items, t, a, r0, sorted_ids, upto);
     while (true) {
         if (cur.t >= upto) {                             // current item finished (or was nothing to do): switch
             if (cur.off >= 0) {
                 st4(t.data + cur.off, cur.p);
                 st4(a.m + cur.off, cur.m);
-                st4(a.v + cur.off, cur.v);
+                if (P::TWO) st4(a.v + cur.off, cur.v);
             }
             if (!cur_real) break;                        // ran past the end of the queue: this lane is done
             cur = nxt;
             cur_real = k < n_items;
             k += dk; c += dc; if (c >= chunks) { c -= chunks; ++k; }
-            replay_fetch<CATCHUP>(nxt, k, c, n_items, t, a, r0, sorted_ids, upto);
+            replay_fetch<CATCHUP, P>(nxt, k, c, n_items, t, a, r0, sorted_ids, upto);
             continue;
         }
         ++cur.t;
-        adam_l2_step4(cur.p, cur.m, cur.v, __ldg(&a.sched[cur.t]), a.h);
+        P::l2_step4(cur.p, cur.m, cur.v, P::coef(a.sched, cur.t), a.h);
     }
 }
 // In-record stamps (stamp_col >= 0): the stamp is part of the record, so ONE lane owns a whole row (all of its
@@ -969,7 +1031,7 @@ __device__ __forceinline__ int64_t replay_row_of(int64_t k, int64_t n_items, int
 // nothing in the caller depends on the data until the item becomes current (a full replay of another row later).
 // LPRR lanes share a row (co-located records of 5..32 chunks): lane slice h owns chunks h*CH .. h*CH+CH-1, `live` of them active
 // (none for the last slices of a record that does not fill them).
-template <int CH, bool UNSORTED = false>
+template <int CH, bool UNSORTED = false, class P = AdamStep>
 __device__ __forceinline__ void replay_row_issue(ReplayRow<CH>& it, int64_t row, const TableView& t, const AdamView& a, int first_col,
                                                  int live, uint32_t* __restrict__ claim = nullptr, bool claimer = false) {
     it.off = row < 0 ? row : row * t.pitch + first_col;
@@ -984,7 +1046,7 @@ __device__ __forceinline__ void replay_row_issue(ReplayRow<CH>& it, int64_t row,
             if (c < live) {
                 it.p[c] = ld4(t.data + it.off + 4 * c);
                 it.m[c] = ld4(a.m + it.off + 4 * c);
-                it.v[c] = ld4(a.v + it.off + 4 * c);
+                it.v[c] = P::TWO ? ld4(a.v + it.off + 4 * c) : f4zero();
             } else {
                 it.p[c] = f4zero(); it.m[c] = f4zero(); it.v[c] = f4zero();
             }
@@ -1024,7 +1086,7 @@ __device__ __forceinline__ void replay_row_arm(ReplayRow<CH>& it, const AdamView
     }
     if (st >= upto) it.off = -1; else it.t = st;
 }
-template <int CH, int LPRR, bool CATCHUP, bool UNSORTED = false>
+template <int CH, int LPRR, bool CATCHUP, bool UNSORTED = false, class P = AdamStep>
 __global__ void __launch_bounds__(128, (LPRR > 2 ? (CH == 3 ? 3 : 2) : (CH == 3 ? 4 : 3)))   // wide records (LPRR 4, 8): no spills
 replay_rows_kernel(TableView t, AdamView a, int64_t r0, int64_t n_items, const uint32_t* __restrict__ sorted_ids,
                    const int64_t* __restrict__ ids64 = nullptr, uint32_t* __restrict__ claim = nullptr) {
@@ -1041,8 +1103,8 @@ replay_rows_kernel(TableView t, AdamView a, int64_t r0, int64_t n_items, const u
     auto row_of = [&](int64_t k) -> int64_t {
         return UNSORTED ? replay_row_unsorted(k, n_items, ids64, t.n_rows) : replay_row_of<CATCHUP>(k, n_items, r0, sorted_ids, t.n_rows);
     };
-    replay_row_issue<CH, UNSORTED>(cur, row_of(kc), t, a, first_col, live, claim, h == 0);
-    replay_row_issue<CH, UNSORTED>(nxt, row_of(kc + stride), t, a, first_col, live, claim, h == 0);
+    replay_row_issue<CH, UNSORTED, P>(cur, row_of(kc), t, a, first_col, live, claim, h == 0);
+    replay_row_issue<CH, UNSORTED, P>(nxt, row_of(kc + stride), t, a, first_col, live, claim, h == 0);
     int64_t row2 = row_of(kc + 2 * stride);
     if (cur.off == -2) return;
     replay_row_arm<CH, LPRR, UNSORTED>(cur, a, upto, h);
@@ -1055,25 +1117,25 @@ replay_rows_kernel(TableView t, AdamView a, int64_t r0, int64_t n_items, const u
                         embed_stamp(cur.p[c], first_col + 4 * c, a, upto);
                         st4(t.data + cur.off + 4 * c, cur.p[c]);
                         st4(a.m + cur.off + 4 * c, cur.m[c]);
-                        st4(a.v + cur.off + 4 * c, cur.v[c]);
+                        if (P::TWO) st4(a.v + cur.off + 4 * c, cur.v[c]);
                     }
                 }
             }
             kc += stride;
             if (kc >= n_items || nxt.off == -2) break;   // end of the queue, or of the ids this table owns
             cur = nxt;                                   // its loads were issued one whole item ago
-            replay_row_issue<CH, UNSORTED>(nxt, row2, t, a, first_col, live, claim, h == 0);   // row2's id was fetched one item ago: no dependent wait here
+            replay_row_issue<CH, UNSORTED, P>(nxt, row2, t, a, first_col, live, claim, h == 0);   // row2's id was fetched one item ago: no dependent wait here
             row2 = row_of(kc + 2 * stride);
             replay_row_arm<CH, LPRR, UNSORTED>(cur, a, upto, h);
             continue;
         }
         ++cur.t;
-        const float2 sc = __ldg(&a.sched[cur.t]);
+        const float2 sc = P::coef(a.sched, cur.t);
 #pragma unroll
-        for (int c = 0; c < CH; ++c) adam_l2_step4(cur.p[c], cur.m[c], cur.v[c], sc, a.h);
+        for (int c = 0; c < CH; ++c) P::l2_step4(cur.p[c], cur.m[c], cur.v[c], sc, a.h);
     }
 }
-template <bool CATCHUP>
+template <bool CATCHUP, class P = AdamStep>
 static int launch_replay_rows(const TableView& t, const AdamView& a, int64_t r0, int64_t n_items,
                               const uint32_t* sorted_ids, cudaStream_t st, const int64_t* ids64 = nullptr, uint32_t* claim = nullptr) {
     const int ch = (t.used + 3) >> 2;
@@ -1094,18 +1156,18 @@ static int launch_replay_rows(const TableView& t, const AdamView& a, int64_t r0,
         return RLCTR_OK;
     }
     switch (ch) {
-        case 1: replay_rows_kernel<1, 1, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 2: replay_rows_kernel<2, 1, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 3: replay_rows_kernel<3, 1, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 4: replay_rows_kernel<4, 1, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 5: case 6: replay_rows_kernel<3, 2, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 7: case 8: replay_rows_kernel<4, 2, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 9: case 10: case 11: case 12: replay_rows_kernel<3, 4, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
-        case 13: case 14: case 15: case 16: replay_rows_kernel<4, 4, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 1: replay_rows_kernel<1, 1, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 2: replay_rows_kernel<2, 1, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 3: replay_rows_kernel<3, 1, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 4: replay_rows_kernel<4, 1, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 5: case 6: replay_rows_kernel<3, 2, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 7: case 8: replay_rows_kernel<4, 2, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 9: case 10: case 11: case 12: replay_rows_kernel<3, 4, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
+        case 13: case 14: case 15: case 16: replay_rows_kernel<4, 4, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids); break;
         default:
             if (ch > 32) return RLCTR_EUNSUPPORTED;      // wider than four lines
-            if (ch <= 24) replay_rows_kernel<3, 8, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids);
-            else replay_rows_kernel<4, 8, CATCHUP><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids);
+            if (ch <= 24) replay_rows_kernel<3, 8, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids);
+            else replay_rows_kernel<4, 8, CATCHUP, false, P><<<grid, 128, 0, st>>>(t, a, r0, n_items, sorted_ids);
             break;
     }
     RLCTR_LAUNCH_CHECK();
@@ -1324,6 +1386,7 @@ catchup_stamp_kernel(const uint32_t* __restrict__ sorted_ids, int64_t n, int64_t
         if (id < (uint64_t)n_rows && (k == 0 || __ldg(sorted_ids + k - 1) != id)) stamp[id] = upto;
     }
 }
+template <class P = AdamStep>
 __global__ void __launch_bounds__(256)
 adam_flush_scalar_kernel(TableView t, AdamView a, int64_t r0, int64_t r1) {   // row_stride == 1 (LR)
     const int upto = __ldg(a.step);
@@ -1331,9 +1394,9 @@ adam_flush_scalar_kernel(TableView t, AdamView a, int64_t r0, int64_t r1) {   //
         const int st = load_stamp(t, a, row);
         if (st >= upto) continue;
         const int64_t o = row * t.pitch;
-        float p = t.data[o], m = a.m[o], v = a.v[o];
-        adam_replay1(p, m, v, st, upto, a.sched, a.h);
-        t.data[o] = p; a.m[o] = m; a.v[o] = v;
+        float p = t.data[o], m = a.m[o], v = P::TWO ? a.v[o] : 0.f;
+        P::replay1(p, m, v, st, upto, a.sched, a.h);
+        t.data[o] = p; a.m[o] = m; if (P::TWO) a.v[o] = v;
         if (a.stamp_col >= 0) t.data[o + a.stamp_col] = __int_as_float(upto); else a.stamp[row] = upto;
     }
 }
@@ -1345,7 +1408,7 @@ stamp_fill_kernel(int32_t* __restrict__ stamp, const int32_t* __restrict__ step,
 }
 
 // row_stride == 1 (the LR table): one lane per sorted position
-template <int APPLY>
+template <int APPLY, class P = AdamStep>
 __global__ void __launch_bounds__(256)
 rows_scalar_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __restrict__ sorted_slots, int64_t n,
                    GradView g, TableView t, AdamView a, float* __restrict__ dense_grad) {
@@ -1368,22 +1431,22 @@ rows_scalar_kernel(const uint32_t* __restrict__ sorted_ids, const uint32_t* __re
     if (APPLY == 1) { dense_grad[id] = acc; continue; }
     const int step = __ldg(a.step) + 1;
     const int64_t o = (int64_t)id * t.pitch;
-    float p, m, v;
-    if (a.stage) {                                         // [w, m, v, 0] of this position, replayed by rlctr_rows_lookup
+    float p, m, v = 0.f;
+    if (P::TWO && a.stage) {                               // [w, m, v, 0] of this position, replayed by rlctr_rows_lookup
         const float4 r = ldg4(a.stage + 4 * k);
         p = r.x; m = r.y; v = r.z;
     } else {
-        p = t.data[o]; m = a.m[o]; v = a.v[o];
+        p = t.data[o]; m = a.m[o]; if (P::TWO) v = a.v[o];
     }
     if (is_lazy(a)) {
-        if (!a.stage) adam_replay1(p, m, v, load_stamp(t, a, id), step - 1, a.sched, a.h);
+        if (!a.stage) P::replay1(p, m, v, load_stamp(t, a, id), step - 1, a.sched, a.h);
         if (a.stamp_col >= 0) t.data[o + a.stamp_col] = __int_as_float(step); else a.stamp[id] = step;
     }
-    const float2 sc = __ldg(&a.sched[step]);
-    adam_elem_fast(p, m, v, acc, a.h, sc.x, rcp_approx(sc.y));
-    t.data[o] = p; a.m[o] = m; a.v[o] = v;
+    P::apply1(p, m, v, acc, P::coef(a.sched, step), a.h);
+    t.data[o] = p; a.m[o] = m; if (P::TWO) a.v[o] = v;
     }
 }
+template <class P = AdamStep>
 __global__ void __launch_bounds__(256)
 rows_catchup_scalar_kernel(const uint32_t* __restrict__ sorted_ids, int64_t n, TableView t, AdamView a) {
     const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1394,9 +1457,9 @@ rows_catchup_scalar_kernel(const uint32_t* __restrict__ sorted_ids, int64_t n, T
     const int st = load_stamp(t, a, id);
     if (st >= upto) return;
     const int64_t o = (int64_t)id * t.pitch;
-    float p = t.data[o], m = a.m[o], v = a.v[o];
-    adam_replay1(p, m, v, st, upto, a.sched, a.h);
-    t.data[o] = p; a.m[o] = m; a.v[o] = v;
+    float p = t.data[o], m = a.m[o], v = P::TWO ? a.v[o] : 0.f;
+    P::replay1(p, m, v, st, upto, a.sched, a.h);
+    t.data[o] = p; a.m[o] = m; if (P::TWO) a.v[o] = v;
     if (a.stamp_col >= 0) t.data[o + a.stamp_col] = __int_as_float(upto); else a.stamp[id] = upto;
 }
 
@@ -1445,6 +1508,27 @@ dense_adam_multi_kernel(const __grid_constant__ DenseGroup grp, const float2* __
         p[i] = pp; m[i] = mm; v[i] = vv;
     }
 }
+// torch.optim.Adagrad for the replicated dense parameters (DenseGroup.m = state sums, .v unused), IEEE sqrt and division:
+// grad.add(param, alpha=wd); state_sum.addcmul_(grad, grad); param.addcdiv_(grad, state_sum.sqrt().add_(eps), value=-clr)
+__global__ void __launch_bounds__(256)
+dense_adagrad_multi_kernel(const __grid_constant__ DenseGroup grp, const float* __restrict__ clr_tab, const int32_t* __restrict__ steps,
+                           float eps, float wd) {
+    int t = 0;
+    while (t + 1 < grp.count && (int)blockIdx.x >= grp.first_block[t + 1]) ++t;
+    const float clr = __ldg(&clr_tab[__ldg(steps + grp.step_index[t]) + 1]);
+    const int nb = grp.first_block[t + 1] - grp.first_block[t];
+    float* __restrict__ p = grp.p[t];
+    const float* __restrict__ g = grp.g[t];
+    float* __restrict__ s = grp.m[t];
+    for (int64_t i = (int64_t)(blockIdx.x - grp.first_block[t]) * blockDim.x + threadIdx.x; i < grp.n[t]; i += (int64_t)nb * blockDim.x) {
+        float pp = p[i], gg = g[i];
+        if (wd != 0.f) gg = __fadd_rn(gg, __fmul_rn(wd, pp));
+        const float ss = __fadd_rn(s[i], __fmul_rn(gg, gg));
+        const float std = __fadd_rn(__fsqrt_rn(ss), eps);
+        p[i] = __fadd_rn(pp, __fdiv_rn(__fmul_rn(-clr, gg), std));
+        s[i] = ss;
+    }
+}
 
 static inline int grid_1d(int64_t threads, int cap_blocks) {
     int64_t blocks = (threads + 255) / 256;
@@ -1479,12 +1563,21 @@ static inline int rows_grid_env() {
     return v;
 }
 
-template <int APPLY>
+// the optimizer structs of the C ABI: the pointers every update needs, and the AdamView the kernels take (see AdamStep / AdagradStep)
+static inline bool opt_ok(const rlctr_adam* o) { return o && o->exp_avg && o->exp_avg_sq && o->sched && o->step; }
+static inline bool opt_ok(const rlctr_adagrad* o) { return o && o->state_sum && o->clr && o->step; }
+static inline AdamView view_of(const rlctr_adagrad* o, const TableView& t) {
+    return AdamView{o->state_sum, nullptr, o->stamp_col >= 0 ? nullptr : o->stamp, o->stamp_col >= 0 ? o->stamp_col : -1,
+                    reinterpret_cast<const float2*>(o->clr), o->step, AdamHyper{0.f, 0.f, 0.f, (float)o->eps, (float)o->weight_decay},
+                    nullptr, stage_pitch_of(t)};
+}
+
+template <int APPLY, class P = AdamStep, class O = rlctr_adam>
 static int launch_rows(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_rowgrad* grad,
-                       const rlctr_table* table, const rlctr_adam* opt, float* dense_grad, void* ws, size_t ws_bytes,
+                       const rlctr_table* table, const O* opt, float* dense_grad, void* ws, size_t ws_bytes,
                        cudaStream_t st) {
     if (!sorted_ids || !sorted_slots || !grad || !table || !table->data || n < 0) return RLCTR_EINVAL;
-    if (APPLY == 0 && (!opt || !opt->exp_avg || !opt->exp_avg_sq || !opt->sched || !opt->step)) return RLCTR_EINVAL;
+    if (APPLY == 0 && !opt_ok(opt)) return RLCTR_EINVAL;
     if (APPLY == 0 && opt->stamp_col >= (table->row_pitch > 0 ? table->row_pitch : table->row_stride)) return RLCTR_EINVAL;
     if (APPLY == 0 && opt->stamp_col >= 0 && table->row_stride > 32) return RLCTR_EUNSUPPORTED;   // wide rows: separate stamps
     if (APPLY == 1 && !dense_grad) return RLCTR_EINVAL;
@@ -1498,7 +1591,7 @@ static int launch_rows(const uint32_t* sorted_ids, const uint32_t* sorted_slots,
     if ((g.flags & RLCTR_DZ_IN_SUMS) && (t.rs <= t.used || !g.sums)) return RLCTR_EINVAL;
     if (t.rs == 1) {
         if (grad->extra || grad->sums) return RLCTR_EUNSUPPORTED;
-        rows_scalar_kernel<APPLY><<<capped_blocks((n + 255) / 256, grad->world), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a,
+        rows_scalar_kernel<APPLY, P><<<capped_blocks((n + 255) / 256, grad->world), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a,
                                                                                               dense_grad);
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
@@ -1506,9 +1599,9 @@ static int launch_rows(const uint32_t* sorted_ids, const uint32_t* sorted_slots,
     if (t.rs % 4 != 0 || t.rs > 128 * WCH_MAX) return RLCTR_EUNSUPPORTED;
     if (t.rs > 32) {
         if (t.rs <= 256)
-            rows_wide_kernel<APPLY, 2><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
+            rows_wide_kernel<APPLY, 2, P><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
         else
-            rows_wide_kernel<APPLY, 4><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
+            rows_wide_kernel<APPLY, 4, P><<<(unsigned)((n + 7) / 8), 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad);
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
     }
@@ -1519,11 +1612,11 @@ static int launch_rows(const uint32_t* sorted_ids, const uint32_t* sorted_slots,
     unsigned blocks = capped_blocks((n * lpr + 255) / 256, grad->world);
     if (rows_grid_env() > 0 && blocks > (unsigned)(RLCTR_SMS * 5 * rows_grid_env())) blocks = RLCTR_SMS * 5 * rows_grid_env();
 #define LAUNCH_ROWS(L)                                                                                              \
-    rows_short_kernel<L, APPLY><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad,           \
+    rows_short_kernel<L, APPLY, false, P><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad, \
                                                         w.long_count, w.long_list);                                \
-    rows_long_kernel<L, APPLY><<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad,         \
+    rows_long_kernel<L, APPLY, false, 256, P><<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, dense_grad, \
                                                           w.long_count, w.long_list)
-    if (APPLY == 0 && a.stage && a.stamp == nullptr && lpr <= 4) {
+    if (P::TWO && APPLY == 0 && a.stage && a.stamp == nullptr && lpr <= 4) {
         // the lookup's staging array feeds the update: phased kernel (R rows per lane group in flight), then the heavy hitters
         static int r_env = -1;
         if (r_env < 0) { const char* e = getenv("RLCTR_ROWS_R"); r_env = e ? atoi(e) : 0; }
@@ -1649,15 +1742,16 @@ extern "C" int rlctr_rows_adam(const uint32_t* sorted_ids, const uint32_t* sorte
     return launch_rows<0>(sorted_ids, sorted_slots, n, grad, table, opt, nullptr, ws, ws_bytes, (cudaStream_t)stream);
 }
 
-extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_table* table,
-                                     const rlctr_adam* opt, const rlctr_member* members, int32_t n_members, const float* sums,
-                                     int32_t sums_pitch, int32_t fields, int32_t world, const uint32_t* slot_of, void* ws,
-                                     size_t ws_bytes, rlctr_stream_t stream) {
-    if (!sorted_ids || !sorted_slots || !table || !table->data || !opt || !opt->exp_avg || !opt->exp_avg_sq || !opt->sched ||
-        !opt->step || !members || !sums || n < 0 || fields <= 0)
+static inline const float* stage_of(const rlctr_adam* o) { return o->stage; }
+static inline const float* stage_of(const rlctr_adagrad*) { return nullptr; }
+template <class P, class O>
+static int group_rows(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_table* table, const O* opt,
+                      const rlctr_member* members, int32_t n_members, const float* sums, int32_t sums_pitch, int32_t fields,
+                      int32_t world, const uint32_t* slot_of, void* ws, size_t ws_bytes, rlctr_stream_t stream) {
+    if (!sorted_ids || !sorted_slots || !table || !table->data || !opt_ok(opt) || !members || !sums || n < 0 || fields <= 0)
         return RLCTR_EINVAL;
     if (n_members < 1 || n_members > RLCTR_GROUP_MAX) return RLCTR_EINVAL;
-    if (table->world > 1 || opt->stage) return RLCTR_EUNSUPPORTED;
+    if (table->world > 1 || stage_of(opt)) return RLCTR_EUNSUPPORTED;
     if (n == 0) return RLCTR_OK;
     cudaStream_t st = (cudaStream_t)stream;
     TableView t = view_of(table);
@@ -1707,9 +1801,9 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
         const int lanes = t.rs <= 64 ? 16 : 32;
         unsigned blocks = capped_blocks((n * lanes + 255) / 256, world);
         if (rows_grid_env() > 0 && blocks > (unsigned)(RLCTR_SMS * 5 * rows_grid_env())) blocks = RLCTR_SMS * 5 * rows_grid_env();
-        if (lanes == 16) rows_short_kernel<16, 0, true><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
-        else rows_short_kernel<32, 0, true><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
-        group_long_wide_kernel<<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
+        if (lanes == 16) rows_short_kernel<16, 0, true, P><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        else rows_short_kernel<32, 0, true, P><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        group_long_wide_kernel<P><<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
         RLCTR_COUNT_LAUNCH(1);                          // two kernels, one check
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
@@ -1736,9 +1830,9 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
         int64_t want = capped_blocks((2 * n + 255) / 256, world);
         const int64_t cap = (int64_t)RLCTR_SMS * 2 * (rows_grid_env() > 0 ? rows_grid_env() : 64);
         const unsigned b2 = (unsigned)(want < cap ? want : cap);
-        if ((t.used + 3) / 4 <= 6) group_rows2_kernel<3><<<b2, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
-        else group_rows2_kernel<4><<<b2, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
-        rows_long_kernel<8, 0, true, 512><<<RLCTR_SMS, 512, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        if ((t.used + 3) / 4 <= 6) group_rows2_kernel<3, P><<<b2, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
+        else group_rows2_kernel<4, P><<<b2, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, w.long_count, w.long_list);
+        rows_long_kernel<8, 0, true, 512, P><<<RLCTR_SMS, 512, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
         RLCTR_COUNT_LAUNCH(1);
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
@@ -1746,21 +1840,29 @@ extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t*
     unsigned blocks = capped_blocks((n * lpr + 255) / 256, world);
     if (rows_grid_env() > 0 && blocks > (unsigned)(RLCTR_SMS * 5 * rows_grid_env())) blocks = RLCTR_SMS * 5 * rows_grid_env();
     if (lpr == 4) {
-        rows_short_kernel<4, 0, true><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
-        rows_long_kernel<4, 0, true><<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        rows_short_kernel<4, 0, true, P><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        rows_long_kernel<4, 0, true, 256, P><<<RLCTR_SMS, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
     } else {
-        rows_short_kernel<8, 0, true><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
-        rows_long_kernel<8, 0, true, 512><<<RLCTR_SMS, 512, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        rows_short_kernel<8, 0, true, P><<<blocks, 256, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
+        rows_long_kernel<8, 0, true, 512, P><<<RLCTR_SMS, 512, 0, st>>>(sorted_ids, sorted_slots, n, g, t, a, nullptr, w.long_count, w.long_list);
     }
     RLCTR_COUNT_LAUNCH(1);                              // two kernels, one check
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
 }
 
+extern "C" int rlctr_group_rows_adam(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_table* table,
+                                     const rlctr_adam* opt, const rlctr_member* members, int32_t n_members, const float* sums,
+                                     int32_t sums_pitch, int32_t fields, int32_t world, const uint32_t* slot_of, void* ws,
+                                     size_t ws_bytes, rlctr_stream_t stream) {
+    return group_rows<AdamStep>(sorted_ids, sorted_slots, n, table, opt, members, n_members, sums, sums_pitch, fields, world, slot_of,
+                                ws, ws_bytes, stream);
+}
+
 extern "C" int rlctr_rows_grad_dense(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n,
                                      const rlctr_rowgrad* grad, const rlctr_table* table, float* dense_grad, void* ws,
                                      size_t ws_bytes, rlctr_stream_t stream) {
-    return launch_rows<1>(sorted_ids, sorted_slots, n, grad, table, nullptr, dense_grad, ws, ws_bytes,
+    return launch_rows<1>(sorted_ids, sorted_slots, n, grad, table, (const rlctr_adam*)nullptr, dense_grad, ws, ws_bytes,
                           (cudaStream_t)stream);
 }
 
@@ -1822,9 +1924,11 @@ extern "C" int rlctr_rows_lookup(const uint32_t* sorted_ids, const uint32_t* sor
     return RLCTR_OK;
 }
 
-extern "C" int rlctr_rows_catchup(const uint32_t* sorted_ids, int64_t n, const rlctr_table* table,
-                                  const rlctr_adam* opt, rlctr_stream_t stream) {
-    if (!sorted_ids || !table || !table->data || !opt || (!opt->stamp && opt->stamp_col < 0) || !opt->sched || !opt->step ||
+static inline const void* sched_of(const rlctr_adam* o) { return o->sched; }
+static inline const void* sched_of(const rlctr_adagrad* o) { return o->clr; }
+template <class P, class O>
+static int rows_catchup(const uint32_t* sorted_ids, int64_t n, const rlctr_table* table, const O* opt, rlctr_stream_t stream) {
+    if (!sorted_ids || !table || !table->data || !opt || (!opt->stamp && opt->stamp_col < 0) || !sched_of(opt) || !opt->step ||
         n < 0)
         return RLCTR_EINVAL;
     if (n == 0) return RLCTR_OK;
@@ -1832,17 +1936,21 @@ extern "C" int rlctr_rows_catchup(const uint32_t* sorted_ids, int64_t n, const r
     TableView t = view_of(table);
     AdamView a = view_of(opt, t);
     if (t.rs == 1) {
-        rows_catchup_scalar_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sorted_ids, n, t, a);
+        rows_catchup_scalar_kernel<P><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(sorted_ids, n, t, a);
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
     }
     if (t.rs % 4 != 0) return RLCTR_EUNSUPPORTED;
-    if (a.stamp_col >= 0) return launch_replay_rows<true>(t, a, 0, n, sorted_ids, st);
-    replay_kernel<true><<<grid_1d(n * ((t.used + 3) / 4), RLCTR_SMS * 8), 256, 0, st>>>(t, a, 0, n, sorted_ids);
+    if (a.stamp_col >= 0) return launch_replay_rows<true, P>(t, a, 0, n, sorted_ids, st);
+    replay_kernel<true, P><<<grid_1d(n * ((t.used + 3) / 4), RLCTR_SMS * 8), 256, 0, st>>>(t, a, 0, n, sorted_ids);
     RLCTR_LAUNCH_CHECK();
     catchup_stamp_kernel<<<grid_1d(n, RLCTR_SMS * 8), 256, 0, st>>>(sorted_ids, n, t.n_rows, a.stamp, a.step);
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
+}
+extern "C" int rlctr_rows_catchup(const uint32_t* sorted_ids, int64_t n, const rlctr_table* table,
+                                  const rlctr_adam* opt, rlctr_stream_t stream) {
+    return rows_catchup<AdamStep>(sorted_ids, n, table, opt, stream);
 }
 
 extern "C" size_t rlctr_rows_claim_bytes(int64_t n_rows) {
@@ -1862,27 +1970,31 @@ extern "C" int rlctr_rows_catchup_ids(const int64_t* ids, int64_t n, const rlctr
     return launch_replay_rows<true>(t, a, 0, n, nullptr, st, ids, reinterpret_cast<uint32_t*>(claim));
 }
 
-extern "C" int rlctr_adam_flush(const rlctr_table* table, const rlctr_adam* opt, int64_t row_begin, int64_t row_end,
-                                rlctr_stream_t stream) {
-    if (!table || !table->data || !opt || (!opt->stamp && opt->stamp_col < 0) || !opt->sched || !opt->step) return RLCTR_EINVAL;
+template <class P, class O>
+static int rows_flush(const rlctr_table* table, const O* opt, int64_t row_begin, int64_t row_end, rlctr_stream_t stream) {
+    if (!table || !table->data || !opt || (!opt->stamp && opt->stamp_col < 0) || !sched_of(opt) || !opt->step) return RLCTR_EINVAL;
     if (row_begin < 0 || row_end > table->n_rows || row_begin > row_end) return RLCTR_EINVAL;
     if (row_begin == row_end) return RLCTR_OK;
     cudaStream_t st = (cudaStream_t)stream;
     TableView t = view_of(table);
     AdamView a = view_of(opt, t);
     if (t.rs == 1) {
-        adam_flush_scalar_kernel<<<grid_1d(row_end - row_begin, RLCTR_SMS * 8), 256, 0, st>>>(t, a, row_begin, row_end);
+        adam_flush_scalar_kernel<P><<<grid_1d(row_end - row_begin, RLCTR_SMS * 8), 256, 0, st>>>(t, a, row_begin, row_end);
         RLCTR_LAUNCH_CHECK();
         return RLCTR_OK;
     }
     if (t.rs % 4 != 0) return RLCTR_EUNSUPPORTED;
-    if (a.stamp_col >= 0) return launch_replay_rows<false>(t, a, row_begin, row_end - row_begin, nullptr, st);
-    replay_kernel<false><<<grid_1d((row_end - row_begin) * ((t.used + 3) / 4), RLCTR_SMS * 8), 256, 0, st>>>(
+    if (a.stamp_col >= 0) return launch_replay_rows<false, P>(t, a, row_begin, row_end - row_begin, nullptr, st);
+    replay_kernel<false, P><<<grid_1d((row_end - row_begin) * ((t.used + 3) / 4), RLCTR_SMS * 8), 256, 0, st>>>(
         t, a, row_begin, row_end - row_begin, nullptr);
     RLCTR_LAUNCH_CHECK();
     stamp_fill_kernel<<<grid_1d(row_end - row_begin, RLCTR_SMS * 8), 256, 0, st>>>(a.stamp, a.step, row_begin, row_end);
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
+}
+extern "C" int rlctr_adam_flush(const rlctr_table* table, const rlctr_adam* opt, int64_t row_begin, int64_t row_end,
+                                rlctr_stream_t stream) {
+    return rows_flush<AdamStep>(table, opt, row_begin, row_end, stream);
 }
 
 extern "C" int rlctr_dense_adam(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,
@@ -1940,6 +2052,54 @@ extern "C" int rlctr_steps_advance(int32_t* steps, const int32_t* step_index, in
 extern "C" int rlctr_step_advance(int32_t* step, int32_t delta, rlctr_stream_t stream) {
     if (!step) return RLCTR_EINVAL;
     step_advance_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(step, delta);
+    RLCTR_LAUNCH_CHECK();
+    return RLCTR_OK;
+}
+
+// ---- torch.optim.Adagrad (include/rlctr.h): the Adam calls' gradient side and launch shapes with AdagradStep ------------------
+extern "C" int rlctr_rows_adagrad(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_rowgrad* grad,
+                                  const rlctr_table* table, const rlctr_adagrad* opt, void* ws, size_t ws_bytes,
+                                  rlctr_stream_t stream) {
+    return launch_rows<0, AdagradStep>(sorted_ids, sorted_slots, n, grad, table, opt, nullptr, ws, ws_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int rlctr_group_rows_adagrad(const uint32_t* sorted_ids, const uint32_t* sorted_slots, int64_t n, const rlctr_table* table,
+                                        const rlctr_adagrad* opt, const rlctr_member* members, int32_t n_members, const float* sums,
+                                        int32_t sums_pitch, int32_t fields, int32_t world, const uint32_t* slot_of, void* ws,
+                                        size_t ws_bytes, rlctr_stream_t stream) {
+    return group_rows<AdagradStep>(sorted_ids, sorted_slots, n, table, opt, members, n_members, sums, sums_pitch, fields, world,
+                                   slot_of, ws, ws_bytes, stream);
+}
+
+extern "C" int rlctr_adagrad_catchup(const uint32_t* sorted_ids, int64_t n, const rlctr_table* table, const rlctr_adagrad* opt,
+                                     rlctr_stream_t stream) {
+    return rows_catchup<AdagradStep>(sorted_ids, n, table, opt, stream);
+}
+
+extern "C" int rlctr_adagrad_flush(const rlctr_table* table, const rlctr_adagrad* opt, int64_t row_begin, int64_t row_end,
+                                   rlctr_stream_t stream) {
+    return rows_flush<AdagradStep>(table, opt, row_begin, row_end, stream);
+}
+
+extern "C" int rlctr_dense_adagrad_multi(float* const* params, const float* const* grads, float* const* state_sums,
+                                         const int64_t* sizes, int32_t count, const float* clr, const int32_t* steps,
+                                         const int32_t* step_index, double eps, double weight_decay, rlctr_stream_t stream) {
+    if (!params || !grads || !state_sums || !sizes || !clr || !steps || count < 0) return RLCTR_EINVAL;
+    if (count > RLCTR_DENSE_MAX) return RLCTR_EUNSUPPORTED;
+    if (count == 0) return RLCTR_OK;
+    DenseGroup grp;
+    grp.count = count;
+    int blocks = 0;
+    for (int t = 0; t < count; ++t) {
+        if (!params[t] || !grads[t] || !state_sums[t] || sizes[t] < 0) return RLCTR_EINVAL;
+        grp.p[t] = params[t]; grp.g[t] = grads[t]; grp.m[t] = state_sums[t]; grp.v[t] = nullptr; grp.n[t] = sizes[t];
+        grp.step_index[t] = step_index ? step_index[t] : 0;
+        if (grp.step_index[t] < 0) return RLCTR_EINVAL;
+        grp.first_block[t] = blocks;
+        blocks += grid_1d(sizes[t], RLCTR_SMS * 2);
+    }
+    grp.first_block[count] = blocks;
+    dense_adagrad_multi_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(grp, clr, steps, (float)eps, (float)weight_decay);
     RLCTR_LAUNCH_CHECK();
     return RLCTR_OK;
 }

@@ -168,9 +168,9 @@ class _GatherInteract(torch.autograd.Function):
         if module._opt is None and not getattr(module, "rows_grad_only", False):
             # (set ``model.rows_grad_only = True`` to inspect the row-form gradient -- module._stash -- without an optimizer)
             raise _lib.RlctrError("the embedding table's gradient exists only in row form (sorted ids + per-sample terms) and is "
-                                  "consumed by rl_ctr_prediction_b200.optim.Adam(model.parameters(), ...): build that optimizer "
-                                  "before calling backward -- a torch.optim optimizer would silently skip the table (its "
-                                  ".grad is never materialised)")
+                                  "consumed by rl_ctr_prediction_b200.optim.Adam(model.parameters(), ...) or optim.Adagrad: build "
+                                  "that optimizer before calling backward -- a torch.optim optimizer would silently skip the table "
+                                  "(its .grad is never materialised)")
         B, F = ctx.shape
         dev = gout.device
         gout = gout.contiguous()
@@ -338,12 +338,9 @@ class _TableModel(nn.Module):
             opt = self._opt
             if opt is not None and opt.lookup_on:
                 lookup = lookup_rows(self, sorted_pair, x.numel(), x.shape[1])
-            elif opt is not None and opt.lazy and opt.dirty:
-                lib = _lib.load()
-                t, a = table_struct(self.table.data, self._geom), opt.struct()
-                _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(sorted_pair[0]), x.numel(), C.byref(t),
-                          C.byref(a), _lib.stream(), key=f"rlctr_rows_catchup[{type(self).__name__}]",
-                          meta=self._meta(*x.shape))
+            elif opt is not None:
+                opt.catchup(table_struct(self.table.data, self._geom), sorted_pair[0], x.numel(), type(self).__name__,
+                            self._meta(*x.shape))
         else:
             self.flush()
         bias = getattr(self, "bias", None)

@@ -147,10 +147,8 @@ def fused_train_step(model, optimizer, features, labels):
     if opt is not None and opt.lookup_on:
         stage, gathered = Model.lookup_rows(model, (sid, sslot), x.numel(), F)
         t, ids_ptr = Model.gathered_struct(gathered, x.numel(), g), None
-    elif opt is not None and opt.lazy and opt.dirty:
-        a = opt.struct()
-        _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(sid), x.numel(), C.byref(t), C.byref(a), st,
-                  key=f"rlctr_rows_catchup[{type(model).__name__}]", meta=model._meta(B, F))
+    elif opt is not None:
+        opt.catchup(t, sid, x.numel(), type(model).__name__, model._meta(B, F))
     logit = torch.empty(B, dtype=torch.float32, device=dev)
     sums = partners = None
     if model._kind == "ffm":

@@ -329,14 +329,10 @@ class _ShardedTable(nn.Module):
         return t
 
     # ---- pieces of the step -------------------------------------------------------------------------------------------
-    def _catchup(self, srows, n_all, F, key):
-        """Lazy Adam: bring the owned rows of the sorted view up to date before any rank reads them."""
-        opt = self._opt
-        if opt is not None and opt.lazy and opt.dirty:
-            lib = _lib.load()
-            t, a = self._local_struct(), opt.struct()
-            _lib.call("rlctr_rows_catchup", lib.rlctr_rows_catchup, _lib.ptr(srows), n_all, C.byref(t), C.byref(a), _lib.stream(),
-                      key=key, meta=self._meta(n_all // F, F))
+    def _catchup(self, srows, n_all, F, tag):
+        """Lazy optimizer state: bring the owned rows of the sorted view up to date before any rank reads them."""
+        if self._opt is not None:
+            self._opt.catchup(self._local_struct(), srows, n_all, tag, self._meta(n_all // F, F))
 
     def _allreduce_dense(self):
         """Sum every dense gradient over the ranks: one all_reduce of them all, flattened."""
@@ -519,7 +515,7 @@ class ShardedCTR(_ShardedTable):
         y = _co.labels(labels)
         buf = self._grad_buffers(B, F)
         srows, sslots, n_all = shared_sorted_view(x, self.feature_nums, self.group)
-        self._catchup(srows, n_all, F, f"rlctr_rows_catchup[Sharded{self.kind}]")
+        self._catchup(srows, n_all, F, f"Sharded{self.kind}")
         self.barrier()                                        # B1: all owners caught their rows up | forward reads
         logit, trows = self._interact(x, buf, train=True)
         hook, self._after_gather = self._after_gather, None     # graphs.GraphedTrainStep: fork point of the captured step
@@ -575,7 +571,7 @@ class ShardedGroup(_co._GroupStep, _ShardedTable):
     SUMS_PITCH = 32                    # floats per sample of the exchange row: S | dL/dlogit of members 0..3 in the last four columns.
                                        # One line (S <= 28 floats); with max_lines > 1 the instance widens it to the whole lines
                                        # that hold rs + 4 floats
-    _UPDATE_KEY = "rlctr_group_rows_adam[ShardedGroup]"
+    _UPDATE_TAG = "ShardedGroup"
 
     def __init__(self, kinds, feature_nums, field_nums, latent_dims, group=None, device=None, max_lines=1):
         kinds = tuple(_ALIASES.get(k, k) for k in kinds)
@@ -678,7 +674,8 @@ class ShardedGroup(_co._GroupStep, _ShardedTable):
         """One step of every member on the local batch; returns the local mean BCE losses, float32 [M]."""
         lib = _lib.load()
         if self._opt is None:
-            raise _lib.RlctrError("build rl_ctr_prediction_b200.optim.Adam(group.parameters(), ...) before training the group")
+            raise _lib.RlctrError("build rl_ctr_prediction_b200.optim.Adam(group.parameters(), ...) (or optim.Adagrad) before "
+                                  "training the group")
         x = Model._check_ids(features)
         B, F = x.shape
         st, G, M = _lib.stream(), self.world, len(self.members)
@@ -690,7 +687,7 @@ class ShardedGroup(_co._GroupStep, _ShardedTable):
             srows, sslots, n_all = view["rows"], view["pos"], view["n_all"]
         else:
             srows, sslots, n_all = shared_sorted_view(x, self.feature_nums, self.group)
-        self._catchup(srows, n_all, F, "rlctr_rows_catchup[ShardedGroup]")
+        self._catchup(srows, n_all, F, "ShardedGroup")
         self.barrier()                                        # B1: all owners caught their rows up | forward reads
         arr, logits, rows = self._member_structs(B, F, x.device, True)
         t = self._global_struct()

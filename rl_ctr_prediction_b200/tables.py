@@ -153,7 +153,50 @@ class AdamSchedule:
             self._upload(lo, self.length)
 
 
-class TableAdamState:
+def _key(entry, tag):
+    return entry if tag is None else f"{entry}[{tag}]"
+
+
+class _TableState:
+    """What the training step asks of a table's optimizer state, whatever the optimizer: bring the batch's rows up to date
+    (``catchup``), apply the step to the rows the batch touched (``rows_update`` / ``group_update``) and settle every row
+    (``flush``).  A subclass names its C entry points and provides ``struct()``, ``lazy`` and ``lookup_on``."""
+
+    _CATCHUP = _ROWS = _GROUP = _FLUSH = None
+    catchup_ids_ok = False            # rlctr_rows_catchup_ids (batch-order catch-up of co-located records) serves this state
+
+    def catchup(self, t, sorted_ids, n, tag, meta):
+        """Replay the L2-only steps the rows of the sorted view missed (lazy state with rows behind ``step``)."""
+        if not (self.lazy and self.dirty):
+            return
+        lib = _lib.load()
+        _lib.call(self._CATCHUP, getattr(lib, self._CATCHUP), _lib.ptr(sorted_ids), n, C.byref(t), C.byref(self.struct()),
+                  _lib.stream(), key=_key(self._CATCHUP, tag), meta=meta)
+
+    def rows_update(self, sorted_ids, sorted_slots, n, grad, t, ws, ws_bytes, st, tag, meta, stage=None):
+        lib = _lib.load()
+        _lib.call(self._ROWS, getattr(lib, self._ROWS), _lib.ptr(sorted_ids), _lib.ptr(sorted_slots), n, C.byref(grad),
+                  C.byref(t), C.byref(self.struct(stage)), _lib.ptr(ws), ws_bytes, st, key=_key(self._ROWS, tag), meta=meta)
+
+    def group_update(self, sorted_ids, sorted_slots, n, t, members, n_members, sums, sums_pitch, fields, world, slot_of, ws,
+                     ws_bytes, st, tag, meta):
+        lib = _lib.load()
+        _lib.call(self._GROUP, getattr(lib, self._GROUP), _lib.ptr(sorted_ids), _lib.ptr(sorted_slots), n, C.byref(t),
+                  C.byref(self.struct()), members, n_members, _lib.ptr(sums), sums_pitch, fields, world, _lib.ptr(slot_of),
+                  _lib.ptr(ws), ws_bytes, st, key=_key(self._GROUP, tag), meta=meta)
+
+    def flush(self, data: torch.Tensor):
+        """Replay the L2-only steps every row missed."""
+        if not self.lazy or not self.dirty:
+            return
+        lib = _lib.load()
+        t = table_struct(data, self.geom)
+        _lib.call(self._FLUSH, getattr(lib, self._FLUSH), C.byref(t), C.byref(self.struct()), 0, self.geom.n_rows, _lib.stream(),
+                  meta={"rs": self.geom.row_stride, "n_rows": self.geom.n_rows})
+        self.dirty = False
+
+
+class TableAdamState(_TableState):
     """exp_avg / exp_avg_sq / per-row stamp for one fused table, plus the lazy-exact bookkeeping.
 
     mode 'lazy'   (default): rows are brought up to date when touched (rlctr_rows_catchup) and by
@@ -162,6 +205,9 @@ class TableAdamState:
     mode 'dense'  : every step also streams the whole table (the literal reference work).
     mode 'sparse' : untouched rows are left alone (numerically NOT the reference; SURVEY H1 mode C).
     """
+
+    _CATCHUP, _ROWS, _GROUP, _FLUSH = "rlctr_rows_catchup", "rlctr_rows_adam", "rlctr_group_rows_adam", "rlctr_adam_flush"
+    catchup_ids_ok = True
 
     def __init__(self, param: torch.Tensor, geom: Geometry, lr, betas, eps, weight_decay, mode):
         assert mode in ("lazy", "dense", "sparse")
@@ -217,12 +263,86 @@ class TableAdamState:
         RLCTR_LOOKUP=1.  Kept because it is the owner-pushes-rows form of the sharded lookup."""
         return self.lookup_ok and os.environ.get("RLCTR_LOOKUP", "0") == "1"
 
-    def flush(self, data: torch.Tensor):
-        """Replay the L2-only steps every row missed (rlctr_adam_flush)."""
-        if not self.lazy or not self.dirty:
+
+
+class AdagradSchedule:
+    """torch.optim.Adagrad's per-step scalar ``clr = lr / (1 + (t - 1) * lr_decay)`` (torch/optim/adagrad.py
+    ``_single_tensor_adagrad``), a Python double cast to fp32, tabulated for t = 0..len-1 on ``device`` (entry 0 unused).
+    ``ensure`` / ``set_lr`` behave as :class:`AdamSchedule`'s: an lr edit re-tabulates t >= from_step in place."""
+
+    def __init__(self, lr, lr_decay, device, length=8192):
+        self.lr, self.lr_decay, self.device = float(lr), float(lr_decay), device
+        self.length = 0
+        self.tensor = None
+        self.rows = [0.0]
+        self.ensure(length)
+
+    def _row(self, t):
+        return self.lr / (1 + (t - 1) * self.lr_decay)
+
+    def ensure(self, steps: int):
+        if steps < self.length:
+            return False
+        n = max(steps + 1, 2 * self.length, 1024)
+        self.rows.extend(self._row(t) for t in range(len(self.rows), n))
+        self.tensor = torch.tensor(self.rows, dtype=torch.float64).to(torch.float32).to(self.device).contiguous()
+        self.length = n
+        return True
+
+    def set_lr(self, lr, from_step: int):
+        if float(lr) == self.lr:
             return
-        lib = _lib.load()
-        t, a = table_struct(data, self.geom), self.struct()
-        _lib.call("rlctr_adam_flush", lib.rlctr_adam_flush, C.byref(t), C.byref(a), 0, self.geom.n_rows, _lib.stream(),
-                  meta={"rs": self.geom.row_stride, "n_rows": self.geom.n_rows})
+        self.lr = float(lr)
+        lo = max(int(from_step), 1)
+        for t in range(lo, self.length):
+            self.rows[t] = self._row(t)
+        if lo < self.length:
+            self.tensor[lo:self.length].copy_(torch.tensor(self.rows[lo:self.length], dtype=torch.float64).to(torch.float32))
+
+
+class TableAdagradState(_TableState):
+    """torch.optim.Adagrad's state_sum for one fused table: it lives in the record's exp_avg block; the exp_avg_sq block is
+    never read or written.
+
+    With ``weight_decay == 0`` a dense Adagrad step leaves every row no sample touched exactly as it was, so mode 'lazy' keeps
+    no stamps and never launches a catch-up or a flush: it is the reference's numbers with O(touched rows) traffic as it stands.
+    With ``weight_decay > 0`` (and in mode 'dense') the rows carry stamps like :class:`TableAdamState`'s and the missed L2-only
+    steps g = wd * p are replayed (rlctr_adagrad_catchup / rlctr_adagrad_flush); mode 'dense' flushes after every step."""
+
+    _CATCHUP, _ROWS, _GROUP, _FLUSH = "rlctr_adagrad_catchup", "rlctr_rows_adagrad", "rlctr_group_rows_adagrad", "rlctr_adagrad_flush"
+    lookup_on = False                 # the lookup path (RLCTR_LOOKUP) is Adam's
+
+    def __init__(self, param: torch.Tensor, geom: Geometry, lr, lr_decay, weight_decay, initial_accumulator_value, eps, mode):
+        assert mode in ("lazy", "dense")
+        self.geom, self.mode = geom, mode
+        dev = param.device
+        rs = geom.row_stride
+        if geom.has_state:
+            blk = geom.block_floats
+            self.state_sum = param[:, blk:blk + rs]
+        else:
+            self.state_sum = torch.empty_like(param)
+        self.state_sum.fill_(float(initial_accumulator_value))
+        self.stamp, self.stamp_col = None, -1
+        if geom.stamp_col >= 0:
+            param[:, geom.stamp_col].zero_()          # a previous optimizer's stamp: a padding column of p again
+        if weight_decay != 0 or mode == "dense":
+            if geom.stamp_col >= 0:
+                self.stamp_col = geom.stamp_col
+            else:
+                self.stamp = torch.zeros(geom.n_rows, dtype=torch.int32, device=dev)
+        self.step = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.host_step = 0
+        self.sched = AdagradSchedule(lr, lr_decay, dev)
+        self.eps, self.weight_decay = float(eps), float(weight_decay)
         self.dirty = False
+
+    @property
+    def lazy(self):
+        """True when untouched rows are owed their L2-only steps (weight_decay > 0, or mode 'dense')."""
+        return self.stamp is not None or self.stamp_col >= 0
+
+    def struct(self, stage=None) -> _lib.Adagrad:
+        assert stage is None
+        return _lib.Adagrad(self.state_sum.data_ptr(), _lib.ptr(self.stamp), _lib.ptr(self.sched.tensor), _lib.ptr(self.step),
+                            self.sched.length, self.stamp_col, self.eps, self.weight_decay)
