@@ -191,6 +191,11 @@ class _GroupStep:
     sharded.ShardedGroup (row-sharded).  The class provides ``members``, ``_cols``, ``_geom``, ``table``, ``_meta``,
     ``_reduce_ws``, ``_rows_ws``, ``_global_struct()`` (the table as the gathers read it) and ``_UPDATE_TAG``."""
 
+    @property
+    def _record_kind(self):
+        """The members and their columns: two groups of the same width but other members are different records."""
+        return "group:" + "+".join(f"{type(m).__name__}{list(c)}" for m, c in zip(self.members, self._cols))
+
     def _member_structs(self, B, F, dev, train, pctr=None):
         """The members' views for rlctr_group_fwd.  logits[i]: the table part of member i's logit (bias + first order + FM
         term), None for a member that has none (FNN, InnerPNN, OuterPNN, DCN: no linear column, no bias); rows[i]: the tower

@@ -109,7 +109,10 @@ class GraphedTrainStep:
 
     def _room(self):
         """Adam's per-step scalars are tabulated on the device; a captured graph holds the table's address, so
-        the table must already cover the steps the graph will be replayed for."""
+        the table must already cover the steps the graph will be replayed for, at the address it was captured with (an
+        optimizer's load_state_dict may have grown it)."""
+        if [opt._captured() for opt in self._optimizers()] != self._captured:
+            return False
         for opt in self._optimizers():
             for owner in opt._tables:
                 if owner._opt.host_step + 4 >= owner._opt.sched.length:
@@ -124,6 +127,9 @@ class GraphedTrainStep:
         for opt in self._optimizers():
             for owner in opt._tables:
                 owner._opt.sched.ensure(owner._opt.host_step + self.steps_ahead)
+                if owner._opt.lazy:
+                    owner._opt.dirty = True     # the replays leave rows behind: the captured step must hold the catch-up (a
+                                                # table just loaded or flushed is settled, and its eager step would skip it)
             if opt._dense_sched is not None:
                 opt._dense_sched.ensure(opt._dense_done + self.steps_ahead)
 
@@ -227,6 +233,7 @@ class GraphedTrainStep:
             self.losses = self._forked(self.x, self.y)
         self.launches_per_step = int(lib.rlctr_launch_count() - l0)
         self.graph = g
+        self._captured = [opt._captured() for opt in self._optimizers()]
         # the capture ran the Python side of one step (host counters advanced) but no kernel: replay it now
         g.replay()
 
@@ -327,6 +334,8 @@ class GraphedCallable:
         for opt in self.optimizers:
             for owner in opt._tables:
                 owner._opt.sched.ensure(owner._opt.host_step + self.steps_ahead)
+                if owner._opt.lazy:
+                    owner._opt.dirty = True     # the captured step must hold the catch-up (GraphedTrainStep._reserve)
             if opt._dense_sched is not None:
                 opt._dense_sched.ensure(opt._dense_done + self.steps_ahead)
 
@@ -334,6 +343,8 @@ class GraphedCallable:
         dev = tensors[0].device
         if self.stream is None:
             self.stream = torch.cuda.Stream(device=dev)
+        if self.graph is not None and [opt._captured() for opt in self.optimizers] != self._captured:
+            self.graph = None              # an optimizer's load_state_dict replaced a tensor the graph reads: capture again
         if self.graph is not None:
             for buf, t in zip(self.inputs, tensors):
                 buf.copy_(t, non_blocking=True)
@@ -362,5 +373,6 @@ class GraphedCallable:
             self.outputs = self.fn(*self.inputs)
         self.launches_per_step = int(lib.rlctr_launch_count() - l0)
         self.graph = g
+        self._captured = [opt._captured() for opt in self.optimizers]
         g.replay()                      # the capture ran the host side of one step but no kernel: replay it now
         return self.outputs

@@ -273,6 +273,20 @@ class _TableModel(nn.Module):
         if self._opt is not None:
             self._opt.flush(self.table.data)
 
+    # ---- optimizer checkpoints (optim._RowOptimizer.state_dict / load_state_dict) --------------------------------------
+    @property
+    def _record_kind(self):
+        """What a checkpointed optimizer state of this table is laid out for, beside its geometry."""
+        return self._kind
+
+    def _opt_export(self):
+        """The optimizer state of the whole table ({name: float32 [feature_nums, used]}), settled first."""
+        self.flush()
+        return self._opt.export()
+
+    def _opt_load(self, state, step):
+        self._opt.load(self.table.data, state, step)
+
     def _save_to_state_dict(self, destination, prefix, keep_vars):
         self.flush()
         for name, p in self._parameters.items():

@@ -295,6 +295,12 @@ class _ShardedTable(nn.Module):
         self._stash = None
         return super().zero_grad(set_to_none)
 
+    def _save_to_state_dict(self, destination, prefix, keep_vars):
+        # the raw shard carries the optimizer state and stamps: settled, they are what optim's load_state_dict writes, so the
+        # model and the optimizer checkpoints load in either order
+        self.flush()
+        super()._save_to_state_dict(destination, prefix, keep_vars)
+
     def barrier(self):
         self._pm.barrier()
 
@@ -304,15 +310,35 @@ class _ShardedTable(nn.Module):
     def gather_table(self):
         """The full table [N, row_pitch], rebuilt on every rank (tests / checkpointing)."""
         self.flush()
-        mine = self.table.data.contiguous()
+        return self._gather_rows(self.table.data)
+
+    def _gather_rows(self, mine):
+        """Every rank's [n_alloc, w] rows of a per-row tensor into the global [N, w] (row id = local row * G + rank)."""
+        mine = mine.contiguous()
         if self.world == 1:
             return mine[:self.feature_nums].clone()
         parts = [torch.empty_like(mine) for _ in range(self.world)]
         dist.all_gather(parts, mine, group=self.group)
-        full = torch.empty(self.feature_nums, self._geom.row_pitch, dtype=torch.float32, device=mine.device)
+        full = torch.empty(self.feature_nums, mine.shape[1], dtype=mine.dtype, device=mine.device)
         for r in range(self.world):
             full[r::self.world] = parts[r][:shard_rows(self.feature_nums, self.world, r)]
         return full
+
+    # ---- optimizer checkpoints: the world-independent [feature_nums, used] layout ---------------------------------------
+    @property
+    def _record_kind(self):
+        return self._kind
+
+    def _opt_export(self):
+        """The optimizer state of the whole table, gathered on every rank (every rank must call it)."""
+        self.flush()
+        return {k: self._gather_rows(v) for k, v in self._opt.export().items()}
+
+    def _opt_load(self, state, step):
+        """This rank's rows (ids rank, rank + G, ...) of the global state into the shard."""
+        if state is not None:
+            state = {k: v[self.rank::self.world] for k, v in state.items()}
+        self._opt.load(self.table.data, state, step)
 
     def _local_struct(self):
         """The shard as the optimizer kernels see it: n_local rows, local row ids."""

@@ -116,7 +116,9 @@ class AdamSchedule:
 
     ``set_lr(lr, from_step)`` re-tabulates the entries t >= from_step IN PLACE (same device address: a captured CUDA graph
     keeps working): an ``lr`` edited through ``param_groups`` -- an LR scheduler, or the reference's ``learning_rate += 1e-4``
-    per epoch -- takes effect from that step on, while the lazy replay of earlier steps still sees the lr they ran with."""
+    per epoch -- takes effect from that step on, while the lazy replay of earlier steps still sees the lr they ran with.  An
+    unchanged lr returns at once: the entries past the last step taken already hold it.  A checkpoint load moves the step back,
+    so the entries after the saved step may hold lrs edited later; ``force=True`` re-tabulates them whatever ``lr`` is."""
 
     def __init__(self, lr, betas, device, length=8192):
         self.lr, self.betas, self.device = float(lr), (float(betas[0]), float(betas[1])), device
@@ -142,8 +144,8 @@ class AdamSchedule:
         self.length = n
         return True
 
-    def set_lr(self, lr, from_step: int):
-        if float(lr) == self.lr:
+    def set_lr(self, lr, from_step: int, force: bool = False):
+        if float(lr) == self.lr and not force:
             return
         self.lr = float(lr)
         lo = max(int(from_step), 1)
@@ -160,7 +162,9 @@ def _key(entry, tag):
 class _TableState:
     """What the training step asks of a table's optimizer state, whatever the optimizer: bring the batch's rows up to date
     (``catchup``), apply the step to the rows the batch touched (``rows_update`` / ``group_update``) and settle every row
-    (``flush``).  A subclass names its C entry points and provides ``struct()``, ``lazy`` and ``lookup_on``."""
+    (``flush``); and save and restore the state (``export`` / ``load``).  A subclass names its C entry points and provides
+    ``struct()``, ``lazy``, ``lookup_on``, ``_blocks()`` (its state tensors by torch's names) and ``_fresh()`` (their initial
+    value)."""
 
     _CATCHUP = _ROWS = _GROUP = _FLUSH = None
     catchup_ids_ok = False            # rlctr_rows_catchup_ids (batch-order catch-up of co-located records) serves this state
@@ -194,6 +198,35 @@ class _TableState:
         _lib.call(self._FLUSH, getattr(lib, self._FLUSH), C.byref(t), C.byref(self.struct()), 0, self.geom.n_rows, _lib.stream(),
                   meta={"rs": self.geom.row_stride, "n_rows": self.geom.n_rows})
         self.dirty = False
+
+    # ---- checkpoints (optim._RowOptimizer.state_dict / load_state_dict) ---------------------------------------------------
+    def export(self):
+        """{name: float32 [rows, used]} copies of the state over the row's used columns, for every row of the allocation (a
+        shard's padding rows too).  The caller flushes first: a settled lazy table holds what a dense step would, so no stamp
+        is part of the state."""
+        u = self.geom.used
+        return {k: t[:, :u].clone() for k, t in self._blocks().items()}
+
+    def load(self, data: torch.Tensor, state, step: int):
+        """Resume at ``step`` completed steps: ``state`` ({name: [k, used]}, k <= rows; None: a fresh state) goes into the
+        first k rows in place, every row the optimizer steps is stamped settled at ``step``, the schedule covers the next
+        step.  Nothing is reallocated but the schedule, whose growth a captured graph notices (graphs.py)."""
+        u = self.geom.used
+        for k, t in self._blocks().items():
+            if state is None:
+                t.fill_(self._fresh(k))
+            else:
+                src = state[k]
+                t[:src.shape[0], :u].copy_(src)
+        if self.stamp is not None:
+            self.stamp.fill_(step)
+        elif self.stamp_col >= 0:
+            # rows past geom.n_rows (a shard's padding) are never stepped: they keep the stamp of a fresh optimizer
+            data.view(torch.int32)[:self.geom.n_rows, self.geom.offset + self.stamp_col].fill_(step)
+        self.step.fill_(step)
+        self.host_step = int(step)
+        self.dirty = False
+        self.sched.ensure(self.host_step + 2)
 
 
 class TableAdamState(_TableState):
@@ -242,6 +275,12 @@ class TableAdamState(_TableState):
         """True when untouched rows are owed their L2-only steps (modes 'lazy' and 'dense')."""
         return self.stamp is not None or self.stamp_col >= 0
 
+    def _blocks(self):
+        return {"exp_avg": self.exp_avg, "exp_avg_sq": self.exp_avg_sq}
+
+    def _fresh(self, key):
+        return 0.0
+
     def struct(self, stage=None) -> _lib.Adam:
         return _lib.Adam(self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), _lib.ptr(self.stamp),
                          _lib.ptr(self.sched.tensor), _lib.ptr(self.step), self.sched.length, self.stamp_col,
@@ -289,8 +328,8 @@ class AdagradSchedule:
         self.length = n
         return True
 
-    def set_lr(self, lr, from_step: int):
-        if float(lr) == self.lr:
+    def set_lr(self, lr, from_step: int, force: bool = False):
+        if float(lr) == self.lr and not force:
             return
         self.lr = float(lr)
         lo = max(int(from_step), 1)
@@ -335,12 +374,19 @@ class TableAdagradState(_TableState):
         self.host_step = 0
         self.sched = AdagradSchedule(lr, lr_decay, dev)
         self.eps, self.weight_decay = float(eps), float(weight_decay)
+        self.initial_accumulator_value = float(initial_accumulator_value)
         self.dirty = False
 
     @property
     def lazy(self):
         """True when untouched rows are owed their L2-only steps (weight_decay > 0, or mode 'dense')."""
         return self.stamp is not None or self.stamp_col >= 0
+
+    def _blocks(self):
+        return {"sum": self.state_sum}                  # torch.optim.Adagrad's name for it
+
+    def _fresh(self, key):
+        return self.initial_accumulator_value
 
     def struct(self, stage=None) -> _lib.Adagrad:
         assert stage is None
